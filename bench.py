@@ -6,6 +6,7 @@ GMW aggregate).
     python bench.py --impl reference [...]                       # the reference algorithm on the host CPU
     python bench.py --config sweep1m   [--gpus N]                # BASELINE configs[3]: 2^20 objects, STRONG scaling, all-gather
     python bench.py --config stress256 [--gpus N]                # BASELINE configs[4]: 256 keypoints, forward + backward
+    python bench.py [...] --dump-outputs DIR                     # also save the outputs of the last timed step as DIR/*.npy
 
 Default (`--config kitti_val`): a *step* is one forward pass of the GMW pipeline (compute_z -> edge-weight MLP ->
 softmax-weighted depth, GMW/main.py:524-533) over one KITTI-val-shaped synthetic batch (BASELINE configs[1]:
@@ -85,7 +86,30 @@ def parse():
     ap.add_argument("--objects", type=int, default=1 << 20, help="sweep1m: total objects")
     ap.add_argument("--quick", action="store_true", help="skip the per-stage breakdown (multi-rank scaling runs)")
     ap.add_argument("--graph-collective", action="store_true", help="sweep1m: also time solve + all-gather replayed from a CUDA graph")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the timed path returned in its last step as DIR/<name>.npy "
+                         "(inputs are seeded, so two builds can be compared output for output)")
     return ap.parse_args()
+
+
+DUMP_BYTES = 64 * 10**6
+
+
+def dump_outputs(args, arrays):
+    """--dump-outputs: every (float32) array as DIR/<name>.npy, at most DUMP_BYTES in all.  An array larger than its
+    share of the budget is stored as a fixed seeded sample of its flattened elements, in order; the sampled positions
+    depend only on the array's size, so the dumps of two builds stay comparable element for element."""
+    if not args.dump_outputs:
+        return
+    import numpy as np
+    os.makedirs(args.dump_outputs, exist_ok=True)
+    for name, t in arrays.items():
+        a = t.detach().float().cpu()
+        cap = DUMP_BYTES // len(arrays) // 4
+        if a.numel() > cap:
+            g = torch.Generator().manual_seed(WEIGHT_SEED)
+            a = a.reshape(-1)[torch.randperm(a.numel(), generator=g)[:cap].sort().values]
+        np.save(os.path.join(args.dump_outputs, name + ".npy"), a.numpy())
 
 
 def measured_peaks():
@@ -178,14 +202,16 @@ class CpuReference:
         self.sd = O.random_state_dict(WEIGHT_SEED)
 
     def run(self, objects: int, seed: int) -> float:
-        """Process `objects` synthetic objects; returns seconds."""
+        """Process `objects` synthetic objects; returns seconds and keeps their depths in `self.depth`."""
         from dcd_b200 import synth
         ob = synth.make_objects(N=objects, n=self.n, seed=seed)
         t0 = time.perf_counter()
         with torch.no_grad():
-            for lo in range(0, objects, 8):
-                self.O.gmw_pipeline(ob.kps_norm[lo:lo + 8], ob.kps_3d[lo:lo + 8], ob.rot_y[lo:lo + 8], self.sd, faithful=True)
-        return time.perf_counter() - t0
+            depths = [self.O.gmw_pipeline(ob.kps_norm[lo:lo + 8], ob.kps_3d[lo:lo + 8], ob.rot_y[lo:lo + 8], self.sd, faithful=True)
+                      for lo in range(0, objects, 8)]
+        secs = time.perf_counter() - t0
+        self.depth = torch.cat(depths)
+        return secs
 
 
 def cpu_reference_rate(sample_objects: int, seed: int):
@@ -215,6 +241,7 @@ def run_reference(args):
     for w in range(args.warmup):
         ref.run(8, 1 + w)
     secs = sum(ref.run(sample, 100 + s) for s in range(args.steps))
+    dump_outputs(args, {"depth": ref.depth})
     rate = sample * args.steps / secs
     line = {
         "metric": METRIC, "value": rate, "unit": UNIT, "impl": "reference", "n_gpus": args.gpus, "steps": args.steps,
@@ -442,6 +469,8 @@ def run_kitti_val(args):
     mlp_objs = sum(nc for _, _, nc in fw.mlp_events)
     assert full.numel() == N_total
     full = full.clone()
+    if rank == 0:
+        dump_outputs(args, {"depth": full})
 
     def recompute(other):
         ob2 = synth.make_objects(n=N_KPTS, seed=seed + 1000 * other,
@@ -848,6 +877,8 @@ def run_sweep1m(args):
     mlp_objs = sum(nc for _, _, nc in fw.mlp_events)
     assert full.numel() == N_total
     full = full.clone()
+    if rank == 0:
+        dump_outputs(args, {"depth": full})
 
     def recompute(other):
         ob2 = shard(other)
@@ -978,14 +1009,14 @@ def run_stress256(args):
         wt, _ = model(t_k2, t_k3, t_rot, None)
         if record:
             e1.record()
-        loss, _ = dcd_b200.compute_reg_loss(Zt, wt, t_gt, idxt)
+        loss, depth = dcd_b200.compute_reg_loss(Zt, wt, t_gt, idxt)
         loss.backward()
         if record:
             e2.record()
             fwd_ev.append((e0, e1, e2))
         if world > 1:
             ddist.allreduce_gradients(model)
-        return loss
+        return loss, depth
     for _ in range(max(args.warmup, 3)):
         train_step()
     sampler = ClockSampler(ctx.local_rank)
@@ -995,7 +1026,7 @@ def run_stress256(args):
     t_beg, t_end = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     t_beg.record()
     for _ in range(args.steps):
-        loss = train_step(True)
+        loss, depth = train_step(True)
     t_end.record()
     ctx.barrier()
     clocks = sampler.stop() if rank == 0 else None
@@ -1003,6 +1034,8 @@ def run_stress256(args):
     fwd_ms = sum(a.elapsed_time(b) for a, b, _ in fwd_ev)
     bwd_ms = sum(b.elapsed_time(c) for _, b, c in fwd_ev)
     assert torch.isfinite(loss).all() and torch.isfinite(model.params4.grad).all()
+    if rank == 0:
+        dump_outputs(args, {"loss": loss, "depth": depth, "grad_params4": model.params4.grad, "grad_params6": model.params6.grad})
 
     # e2e: host inputs, host loss, through the public API
     h_k2, h_k3, h_rot, h_gt = t_k2.cpu().pin_memory(), t_k3.cpu().pin_memory(), t_rot.cpu().pin_memory(), t_gt.cpu().pin_memory()

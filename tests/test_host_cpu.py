@@ -175,27 +175,42 @@ def test_patch_install_and_uninstall():
     assert FakeEncoder().decode_pairs_kpts_depth() == "reference" and main.compute_z() == "ref_z"
 
 
-def test_bench_reference_arm_runs_on_cpu():
+def test_bench_reference_arm_runs_on_cpu(tmp_path):
     import json
     import subprocess
     import sys
-    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1",
-                          "--warmup", "0", "--cpu-sample", "16"], capture_output=True, text=True, timeout=600)
+    import numpy as np
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "2",
+                          "--warmup", "0", "--cpu-sample", "16", "--dump-outputs", str(tmp_path)],
+                         capture_output=True, text=True, timeout=600)
     assert out.returncode == 0, out.stderr[-2000:]
     line = json.loads(out.stdout.strip().splitlines()[-1])
     assert line["impl"] == "reference" and line["value"] > 0 and line["unit"] == "objects/s"
     assert line["cpu_baseline"]["kind"] == "port" and line["e2e"]["h2d_bytes_per_step"] == 0
+    # --dump-outputs: the depths of the last timed step (8 objects of seed 101)
+    assert sorted(os.listdir(tmp_path)) == ["depth.npy"]
+    depth = np.load(tmp_path / "depth.npy")
+    assert depth.dtype == np.float32 and depth.shape == (8,)
+    ob = synth.make_objects(N=8, n=73, seed=101)
+    with torch.no_grad():
+        want = O.gmw_pipeline(ob.kps_norm, ob.kps_3d, ob.rot_y, O.random_state_dict(7))
+    assert float(((torch.from_numpy(depth) - want).abs() / want.abs()).max()) < 1e-5
 
 
-def test_patch_against_the_real_reference_objects():
-    """Only where the reference tree is mounted (the build container): install() on the real Anno_Encoder class,
-    GMW/main.py module and GMW nn.Module, weights copied bit-exactly, uninstall() restores everything."""
-    from oracle import ref_loader as rl
-    if not rl.reference_available():
-        pytest.skip("reference tree not mounted")
-    enc = rl.load_dgde_anno_encoder()
-    ref_main, _ = rl.load_gmw()
-    model = rl.new_gmw_model(3)
+def test_patch_against_reference_shaped_objects():
+    """install() on stand-ins of the reference objects: an Anno_Encoder class whose decode_pairs_kpts_depth is the oracle's,
+    a GMW/main.py module with the oracle's compute_z / compute_reg_loss, and an nn.Module with the reference GMW's
+    parameter tree; weights copied bit-exactly, uninstall() restores everything."""
+    from test_gpu_patch import reference_shaped_gmw
+
+    class Anno_Encoder:
+        def decode_pairs_kpts_depth(self, kps, kps_3d, rot_y, K, training=False, kpts_2d_mask=None, gt_depth=None, weight=None):
+            return O.decode_pairs_kpts_depth(kps, kps_3d, rot_y, K, training=training, kpts_2d_mask=kpts_2d_mask)
+
+    enc = Anno_Encoder()
+    ref_main = types.ModuleType("main")
+    ref_main.compute_z, ref_main.compute_reg_loss = O.compute_z, O.compute_reg_loss
+    model = reference_shaped_gmw(O.random_state_dict(3), 12).eval()
     orig_decode = type(enc).decode_pairs_kpts_depth
     orig_cz, orig_forward = ref_main.compute_z, model.forward
     n_keys = len(model.state_dict())
