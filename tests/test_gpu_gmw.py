@@ -19,6 +19,35 @@ from conftest import rel_err
 pytestmark = pytest.mark.gpu
 DEV = "cuda"
 
+# Slice geometries of the on-chip inference forward (mlp_fused_kernel).  An object's E = n(n-1)/2 edges are split over 24 CTAs
+# in slices of ES = 16 upo edges, upo = ceil(E / 384); inference runs the fused kernel for 3 <= upo <= 7, i.e. n = 40 .. 73.
+# upo sets the tile/object layout, the unit-stream rotation (wg - o upo) mod 3, the count tables and, at upo = 4, the hand-off:
+#   upo  n      ES   what is special
+#   3    40-48  48   one object per tile, the same unit stream for all three objects; n = 40: 7 empty ranks, ranks 16-23 hold
+#                    12 edges; n = 41: 4 edges in the last rank (only unit stream 0 live)
+#   4    49-55  64   the statistics warps do the last merge and write (mean, rstd) into all three stream slots; n = 50 / 55:
+#                    last rank of 9 / 13 edges
+#   5    56-62  80   n = 60: last rank of 10 edges
+#   6    63-68  96   stream rotation 0 like upo 3; n = 64 fills its last rank exactly, n = 67 leaves 3 edges in it
+#   7    69-73  112  n = 73: the reference's keypoint count
+# n = 39 and n = 74 take the layer-wise kernels (controls on either side of the dispatch boundary).  On a 148-SM B200 the paired
+# schedule starts between N = 18 and N = 24 depending on n (N >= 18 and N EP >= 6 groups x 3 x 24 ES): N = 17 is unpaired and
+# N = 25 paired for every n.
+# Columns: upo, the n it covers, representative n (place / schedule / poisoning; the first of them also for depth 1 and the
+# product entry), n for the correspondence branch (E % 4 == 0 takes the tensor-core K tiles, E % 4 != 0 the CUDA-core ones).
+FUSED_GEOMETRY = (
+    (3, range(40, 49), (40, 48), (40, 45)),
+    (4, range(49, 56), (50, 55), (49, 52)),
+    (5, range(56, 63), (60,), (57,)),
+    (6, range(63, 69), (64, 67), (64, 66)),
+    (7, range(69, 74), (73,), (69,)),
+)
+assert all(-(-(n * (n - 1) // 2) // 384) == upo for upo, ns, _, _ in FUSED_GEOMETRY for n in ns)
+SWEEP_N = [39] + [n for _, ns, _, _ in FUSED_GEOMETRY for n in ns] + [74]
+CLASS_N = [n for _, _, reps, _ in FUSED_GEOMETRY for n in reps]
+FIRST_CLASS_N = [reps[0] for _, _, reps, _ in FUSED_GEOMETRY]
+TRANSPORT_N = [n for _, _, _, ns in FUSED_GEOMETRY for n in ns]
+
 
 def cu(*ts):
     return [t.to(DEV) if torch.is_tensor(t) else t for t in ts]
@@ -173,15 +202,18 @@ def test_weight_gradients_full_size_vs_reference_fixture(golden):
             assert float(mine[k].abs().max()) < 1e-4 * gmax, k
 
 
-@pytest.mark.parametrize("n,depth,N", [(73, 12, 5), (60, 3, 3), (8, 2, 9), (17, 1, 1), (74, 2, 2), (73, 12, 41), (60, 2, 37), (20, 3, 19)])
+@pytest.mark.parametrize("n,depth,N", [(73, 12, 5), (60, 3, 3), (8, 2, 9), (17, 1, 1), (74, 2, 2), (73, 12, 41), (60, 2, 37), (20, 3, 19)]
+                         + [(n, 12, N) for n in SWEEP_N for N in (17, 25)])
 def test_fused_inference_forward_agrees_with_layerwise_training_forward(n, depth, N):
     """Inference (no grad) runs the whole network in one kernel with the activations on chip (n = 40 .. 73: three
     objects per group of 24 CTAs); the training forward runs layer by layer through HBM.  Same arithmetic, different
     merge order of the context-norm partials: the two must agree to FP32 rounding.  n = 74 exceeds the on-chip capacity,
     n < 40 leaves a converter warp without a unit of every object: both take the layer-wise kernels in both modes.  With
-    at least three objects per CTA group (18 on a B200) the fused kernel runs its PAIRED schedule and emits the edge
-    weights from its own epilogue (no feature round trip through HBM); below that the features go through
-    gmw_edge_weight_kernel."""
+    enough objects per CTA group (N >= 18 and N EP >= 6 x 3 x 24 ES on a 148-SM B200: N >= 18 .. 24 depending on n, see
+    FUSED_GEOMETRY) the fused kernel runs its PAIRED schedule and emits the edge weights from its own epilogue (no feature
+    round trip through HBM); below that the features go through gmw_edge_weight_kernel.  The sweep runs every n from 39 to
+    74 at N = 17 (unpaired) and N = 25 (paired), both with an incomplete last triple; the first triple and objects N - 2 and
+    N - 1 are held to an FP64 evaluation of the reference."""
     ob = synth.make_objects(N=N, n=n, seed=900 + n)
     sd = O.random_state_dict(50 + n, depth=depth)
     model = make_model(sd, depth)
@@ -195,23 +227,36 @@ def test_fused_inference_forward_agrees_with_layerwise_training_forward(n, depth
     with torch.no_grad():
         w_again, _ = model(k2, k3)
     assert torch.equal(w_inf, w_again)                    # deterministic
-    if N > 18:                                            # paired schedule vs the FP64 oracle, and vs the unpaired schedule on a slice
-        sd64 = {k: v.double().to(DEV) for k, v in sd.items()}
-        w64 = O.gmw_reg_weights(k2[:3].double(), k3[:3].double(), sd64, depth)
-        assert rel_err(w_inf[:3], w64) < 2e-4
+    sel = sorted({0, 1, 2, N - 2, N - 1} & set(range(N)))  # the first triple and the last (incomplete) one
+    sd_dev = {k: v.to(DEV) for k, v in sd.items()}
+    with torch.no_grad():
+        w32 = O.gmw_reg_weights(k2[sel], k3[sel], sd_dev, depth)
+        w64 = O.gmw_reg_weights(k2[sel].double(), k3[sel].double(), {k: v.double() for k, v in sd_dev.items()}, depth)
+    e_o, e_r = rel_err(w_inf[sel], w64), rel_err(w32, w64)
+    print("n=%d depth %d N=%d: reg_weights ours vs f64 %.3g, FP32 oracle vs f64 %.3g" % (n, depth, N, e_o, e_r))
+    assert e_o < 2e-4, (n, depth, N)
+    if N > 18:                                            # the paired schedule (N = 25) vs the unpaired one on a slice
         with torch.no_grad():
             w_few, _ = model(k2[:7].contiguous(), k3[:7].contiguous())
-        assert rel_err(w_few, w_inf[:7]) < 1e-5         # (the paired epilogue sums the squares before normalising)
+        assert torch.equal(w_few, w_inf[:7])              # (gmw_edge_weight_kernel<true> replays the epilogue's roundings)
 
 
-@pytest.mark.parametrize("n,N,step", [(73, 20, 7), (73, 23, 5), (60, 22, 4), (73, 303, 17)])
-def test_fused_forward_is_independent_of_place_and_schedule(n, N, step):
+def _place_case(n, N, step, depth=None):
+    # the depth is 12 for a short batch and 2 for a long one unless given; only depth 1 shows in the id
+    return pytest.param(n, N, step, depth or (12 if N < 100 else 2), id="%d-%d-%d" % (n, N, step) + ("-depth1" if depth == 1 else ""))
+
+
+@pytest.mark.parametrize("n,N,step,depth", [_place_case(*c) for c in [(73, 20, 7), (73, 23, 5), (60, 22, 4), (73, 303, 17)]
+                                            + [(n, N, step) for n in CLASS_N for N, step in ((25, 7), (25, 5), (301, 17))]
+                                            + [(n, 25, 7, 1) for n in FIRST_CLASS_N]])
+def test_fused_forward_is_independent_of_place_and_schedule(n, N, step, depth):
     """The on-chip forward works on three objects at a time and deals triples to the CTA groups; an object's weights must
     not depend on its place in a triple, on the incomplete last triple (N % 3 != 0 repeats the last object), on the
-    schedule (paired for N >= 18, else through the feature buffer) or on how long the kernel has been running (N = 303:
-    more than 256 statistics exchanges per group, the flagged exchange words wrap many times): bit-identical weights
-    for the whole batch and for the same objects fed in small chunks at shifted positions."""
-    depth = 12 if N < 100 else 2
+    schedule (paired for N >= 18 .. 24, else through the feature buffer) or on how long the kernel has been running
+    (N = 301, 303: more than 256 statistics exchanges per group, the flagged exchange words wrap many times; several
+    triples per group): bit-identical weights for the whole batch and for the same objects fed in small chunks at shifted
+    positions, at every slice geometry (FUSED_GEOMETRY) and at depth 1 (two layers per net: the shortest weight-reload
+    cycle)."""
     ob = synth.make_objects(N=N, n=n, seed=1000 + N)
     model = make_model(O.random_state_dict(77, depth=depth), depth)
     k2, k3 = cu(ob.kps_norm, ob.kps_3d)
@@ -224,6 +269,53 @@ def test_fused_forward_is_independent_of_place_and_schedule(n, N, step):
     sd64 = {k: v.double().to(DEV) for k, v in O.random_state_dict(77, depth=depth).items()}
     w64 = O.gmw_reg_weights(k2[-2:].double(), k3[-2:].double(), sd64, depth)      # the last (incomplete) triple against FP64
     assert rel_err(w_all[-2:], w64) < 2e-4
+
+
+@pytest.mark.parametrize("n,N", [(n, N) for n in CLASS_N for N in (17, 25)])
+def test_fused_forward_never_reads_uninitialised_workspace(n, N, monkeypatch):
+    """Every workspace NaN-filled before use, at every slice geometry and in both schedules (N = 17 unpaired, N = 25
+    paired): the padded columns of short or full last ranks, the park area of the paired schedule and the unpaired
+    feature store (columns < EP) may not leak into the edge weights."""
+    from dcd_b200 import ops
+    depth = 2
+    ob = synth.make_objects(N=N, n=n, seed=1100 + n)
+    model = make_model(O.random_state_dict(78, depth=depth), depth)
+    k2, k3 = cu(ob.kps_norm, ob.kps_3d)
+    results = []
+    for poison in (False, True):
+        monkeypatch.setattr(ops, "POISON_WORKSPACES", poison)
+        with torch.no_grad():
+            results.append(model(k2, k3)[0])
+    assert bool(torch.isfinite(results[1]).all())
+    assert torch.equal(results[0], results[1])
+
+
+@pytest.mark.parametrize("n", FIRST_CLASS_N)
+def test_fused_depth_entry_at_every_slice_geometry(n):
+    """gmw_weighted_depth (one call: edge selection, fused forward, aggregation per chunk) at one n per slice geometry, with
+    k = min(1500, E / 2) selected edges: equal to the staged pipeline (compute_z, forward, compute_reg_loss), bit-identical
+    for chunks on both sides of the paired threshold and with a short last chunk, and within 1e-5 of the aggregation fed
+    FP64 weights."""
+    depth, N = 12, 26
+    E = n * (n - 1) // 2
+    num_k = min(1500, E // 2)
+    ob = synth.make_objects(N=N, n=n, seed=1200 + n)
+    sd = O.random_state_dict(79, depth=depth)
+    model = make_model(sd, depth)
+    k2, k3, rot, gt = cu(ob.kps_norm, ob.kps_3d, ob.rot_y, ob.gt_depth)
+    fused = {chunk: dcd_b200.gmw_weighted_depth(k2, k3, rot, model, chunk=chunk, num_k=num_k) for chunk in (N, 17, 5)}
+    assert bool(torch.isfinite(fused[N]).all())
+    assert torch.equal(fused[N], fused[17]) and torch.equal(fused[N], fused[5])
+    Z, idx = dcd_b200.compute_z(k2, k3, rot, num_k=num_k)
+    with torch.no_grad():
+        w, _ = model(k2, k3)
+        _, staged = dcd_b200.compute_reg_loss(Z, w, gt, idx)
+    assert rel_err(fused[N], staged) < 1e-6
+    sel = [0, N - 2, N - 1]
+    with torch.no_grad():
+        w64 = O.gmw_reg_weights(k2[sel].double(), k3[sel].double(), {k: v.double().to(DEV) for k, v in sd.items()}, depth)
+        _, z64 = O.compute_reg_loss(Z[sel].double(), w64, gt[sel].double(), idx[sel])
+    assert rel_err(fused[N][sel], z64) < 1e-5
 
 
 def test_state_dict_round_trip():
@@ -381,8 +473,10 @@ def test_edge_transport_forward_vs_reference_fixture(golden):
 
 
 def test_edge_transport_small_shapes_vs_oracle():
-    """n != 73 (E not a multiple of the tiles), shallow nets; oracle evaluated on the GPU."""
-    for n, depth, N in ((9, 1, 3), (20, 2, 2)):
+    """n != 73 (E not a multiple of the tiles), shallow nets; oracle evaluated on the GPU.  The features always come from
+    the unpaired schedule of the on-chip forward for n = 40 .. 73: one n per slice geometry with E % 4 == 0 (tensor-core K
+    tiles of the transport kernel) and E % 4 != 0 (CUDA-core K tiles) — FUSED_GEOMETRY."""
+    for n, depth, N in [(9, 1, 3), (20, 2, 2)] + [(n, 2, 2) for n in TRANSPORT_N]:
         ob = synth.make_objects(N=N, n=n, seed=300 + n)
         sd = O.random_state_dict(n, depth=depth)
         model = make_model(sd, depth)
