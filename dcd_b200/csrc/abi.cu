@@ -30,6 +30,7 @@ size_t gmw_bwd_scratch_floats(int64_t N, int n, int depth);
 size_t tc_weight_image_bytes(int depth);
 int launch_gmw_weights_bwd(const float*, const float*, const float*, const float*, int64_t, int, int, const float*,
                            const float*, const float*, float*, float*, float*, float*, cudaStream_t);
+int launch_gmw_kpts_bwd(const float*, const float*, int64_t, int, int, float*, float*, float*, cudaStream_t);
 size_t gmw_transport_bwd_workspace_bytes(int64_t N, int E);
 int launch_gmw_transport_bwd(const float*, const float*, const float*, const float*, const float*, const float*, int64_t, int, float,
                              int, float, float*, float*, float*, void*, cudaStream_t);
@@ -232,6 +233,15 @@ int dcd_gmw_weights_bwd(const float* kpts2d, const float* kpts3d, const float* p
     return launch_gmw_weights_bwd(kpts2d, kpts3d, params4, params6, N, n, depth, grad_reg_weights, grad_nfeat4, grad_nfeat6,
                                   grad_params4, grad_params6, static_cast<float*>(workspace), static_cast<float*>(scratch),
                                   (cudaStream_t)stream);
+}
+
+int dcd_gmw_kpts_bwd(const float* params4, const float* params6, int64_t N, int n, int depth, void* scratch,
+                     size_t scratch_bytes, float* grad_kpts2d, float* grad_kpts3d, void* stream) {
+    if (N <= 0 || bad_n(n) || depth < 1) return DCD_E_INVALID;
+    if (!params4 || !params6 || !scratch || (!grad_kpts2d && !grad_kpts3d)) return DCD_E_INVALID;
+    if (misaligned(scratch, 256) || scratch_bytes < dcd_gmw_bwd_scratch_bytes(N, n, depth)) return DCD_E_WORKSPACE;
+    return launch_gmw_kpts_bwd(params4, params6, N, n, depth, static_cast<float*>(scratch), grad_kpts2d, grad_kpts3d,
+                               (cudaStream_t)stream);
 }
 
 int dcd_gmw_aggregate_fwd(const float* reg_weights, const float* depths, const int64_t* idx, int64_t N, int64_t E,

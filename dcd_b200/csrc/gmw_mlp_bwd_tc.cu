@@ -5,7 +5,8 @@
 // last to first, two launches of ONE templated kernel (plus the small sums kernel of the second norm):
 //     R2 :  dy2 = CN'(G * relu')          dW2 += dy2 . yhat1^T     d yhat1 = W2^T dy2   (+ sums for CN1')
 //     R3F:  dy1 = CN'(d yhat1)            dWf += dy1 . x^T         G       = Wf^T dy1 + G   (folded preconv.conv1, residual path)
-// followed by the chain rule through the fold (fold_wgrad_kernel: dWp, dW1 from dWf).
+// followed by the chain rule through the fold (fold_wgrad_kernel: dWp, dW1 from dWf).  What the block loop leaves in G,
+// dL/d(conv_in output), also gives the keypoint gradient (dcd_gmw_kpts_bwd: kpts_feat_bwd_kernel, kpts_gather_bwd_kernel).
 // Every launch is the same dataflow on a 128-edge tile:
 //   * the gradient operand A1 (128 channels x 128 edges) and the activation operand A2 are written ONCE into
 //     shared memory as FP16 hi/lo images in the 128B-swizzled layout of the forward; the same A1 image is the
@@ -571,6 +572,73 @@ __global__ void __launch_bounds__(128) reduce_conv_in_tc_kernel(BwdTcArgs a, flo
     else g[blob_in_w() + (int64_t)k * CH + c] = s;
 }
 
+// ---- keypoint gradient (dcd_gmw_kpts_bwd), from G = dL/dx0 left by the block loop.  conv_in and edge_expand are linear:
+//   KA: dF[e][k] = sum_c W_in^T[k][c] G[c][e]   one thread per (net, object, edge), channels in a fixed order
+//   KB: d kpt[i]  = sum_{j>i} dF_(i,j)[0:h] + sum_{h'<i} dF_(h',i)[h:2h]   one warp per (net, object, keypoint), h = cin / 2
+// dF [net][N][E][cin] lives in the D1 region of the scratch (dead after the block loop, >= 2 N E 128 floats).
+template <int CIN>
+__device__ __forceinline__ void kpts_feat_bwd_edge(const float* __restrict__ G, const float* __restrict__ w_s, int EP, int e,
+                                                   float* __restrict__ out) {
+    float acc[CIN];
+#pragma unroll
+    for (int k = 0; k < CIN; ++k) acc[k] = 0.f;
+#pragma unroll 4
+    for (int c = 0; c < CH; ++c) {
+        const float g = G[(int64_t)c * EP + e];
+#pragma unroll
+        for (int k = 0; k < CIN; ++k) acc[k] = fmaf(w_s[k * CH + c], g, acc[k]);
+    }
+#pragma unroll
+    for (int k = 0; k < CIN; ++k) out[k] = acc[k];
+}
+
+__global__ void __launch_bounds__(256) kpts_feat_bwd_kernel(const float* __restrict__ params4, const float* __restrict__ params6,
+                                                            const float* __restrict__ Gs, float* __restrict__ dF, int64_t N,
+                                                            int E, int EP, int net0) {
+    const int net = net0 + blockIdx.y, cin = net == 0 ? 4 : 6;
+    const int nb = (E + 255) / 256;
+    const int64_t obj = blockIdx.x / nb;
+    const int e = (blockIdx.x % nb) * 256 + threadIdx.x;
+    __shared__ float w_s[6 * CH];
+    const float* prm = (net == 0 ? params4 : params6) + blob_in_w();
+    for (int t = threadIdx.x; t < cin * CH; t += 256) w_s[t] = __ldg(prm + t);
+    __syncthreads();
+    if (e >= E) return;                                   // padded columns e >= E contribute nothing
+    const float* G = Gs + ((int64_t)net * N + obj) * CH * EP;
+    float* out = dF + (net == 0 ? 0 : N * (int64_t)E * 4) + (obj * E + e) * cin;
+    if (net == 0) kpts_feat_bwd_edge<4>(G, w_s, EP, e, out);
+    else kpts_feat_bwd_edge<6>(G, w_s, EP, e, out);
+}
+
+__global__ void __launch_bounds__(256) kpts_gather_bwd_kernel(const float* __restrict__ dF, int64_t N, int n, int net0,
+                                                              float* __restrict__ grad2, float* __restrict__ grad3) {
+    const int net = net0 + blockIdx.y, cin = net == 0 ? 4 : 6, h = cin / 2;
+    const int E = n * (n - 1) / 2;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int nb = (n + 7) / 8;
+    const int64_t obj = blockIdx.x / nb;
+    const int kk = (blockIdx.x % nb) * 8 + warp;
+    if (kk >= n) return;
+    const float* F = dF + (net == 0 ? 0 : N * (int64_t)E * 4) + obj * E * (int64_t)cin;
+    float s[3] = {0.f, 0.f, 0.f};
+    for (int m = lane; m < n; m += 32) {                  // the n - 1 incident edges, lane-strided in partner order
+        if (m == kk) continue;
+        const int i = min(kk, m), j = max(kk, m);
+        const float* f = F + (int64_t)(row_offset(i, n) + j - i - 1) * cin + (kk == i ? 0 : h);
+#pragma unroll
+        for (int q = 0; q < 3; ++q)
+            if (q < h) s[q] += f[q];
+    }
+#pragma unroll
+    for (int q = 0; q < 3; ++q) s[q] = warp_sum(s[q]);
+    if (lane == 0) {
+        float* o = (net == 0 ? grad2 : grad3) + (obj * n + kk) * h;
+#pragma unroll
+        for (int q = 0; q < 3; ++q)
+            if (q < h) o[q] = s[q];
+    }
+}
+
 struct BwdTcScratch {
     int64_t G, D1, bstat, wpart, inpart, gmax, dwf, total;   // float offsets
 };
@@ -648,6 +716,22 @@ int launch_gmw_weights_bwd(const float* kpts2d, const float* kpts3d, const float
     }
     conv_in_bwd_tc_kernel<<<tgrid, 256, 0, st>>>(a);
     reduce_conv_in_tc_kernel<<<dim3(7, 2), 128, 0, st>>>(a, grad4, grad6);
+    DCD_CHECK_LAUNCH();
+    return DCD_OK;
+}
+
+int launch_gmw_kpts_bwd(const float* params4, const float* params6, int64_t N, int n, int depth, float* scratch,
+                        float* grad_kpts2d, float* grad_kpts3d, cudaStream_t st) {
+    const WsLayout L = make_layout(N, n, depth, 1);
+    if ((int64_t)L.T * N > 0x7fffffffLL) return DCD_E_UNSUPPORTED;
+    const BwdTcScratch S = bwd_tc_layout(L, 1);          // the G and D1 offsets do not depend on the CTA count
+    const int net0 = grad_kpts2d != nullptr ? 0 : 1;
+    const unsigned nets = (grad_kpts2d != nullptr && grad_kpts3d != nullptr) ? 2 : 1;
+    const int64_t ga = (int64_t)((L.E + 255) / 256) * N, gb = (int64_t)((n + 7) / 8) * N;
+    if (ga > 0x7fffffffLL) return DCD_E_UNSUPPORTED;
+    kpts_feat_bwd_kernel<<<dim3((unsigned)ga, nets), 256, 0, st>>>(params4, params6, scratch + S.G, scratch + S.D1, N, L.E,
+                                                                    L.EP, net0);
+    kpts_gather_bwd_kernel<<<dim3((unsigned)gb, nets), 256, 0, st>>>(scratch + S.D1, N, n, net0, grad_kpts2d, grad_kpts3d);
     DCD_CHECK_LAUNCH();
     return DCD_OK;
 }

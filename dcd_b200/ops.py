@@ -409,7 +409,10 @@ def ray_rescale(raw_location, pred_depth, dim):
 
 
 def compute_z(kpts_2d, kpts_3d, pred_rot, num_k: int = K_SEL) -> Tuple[torch.Tensor, torch.Tensor]:
-    """Drop-in for GMW/main.py:373-416: (Z_v_raw [b,E] clamped to [0.1,80], good_idx [b,1500] int64)."""
+    """Drop-in for GMW/main.py:373-416: (Z_v_raw [b,E] clamped to [0.1,80], good_idx [b,1500] int64).
+
+    Z_v_raw is differentiable w.r.t. kpts_2d (v column; the u column's gradient is exactly 0, the solve does not read it)
+    and kpts_3d, like the reference's.  pred_rot receives no gradient (as in decode_pairs_kpts_depth)."""
     require_cuda(kpts_2d, kpts_3d, pred_rot)
     kps, kps_3d = f32c(kpts_2d), f32c(kpts_3d)
     rot = f32c(pred_rot).reshape(-1)
@@ -417,8 +420,8 @@ def compute_z(kpts_2d, kpts_3d, pred_rot, num_k: int = K_SEL) -> Tuple[torch.Ten
     if _num_edges(n) < num_k:
         raise RuntimeError("selected index k out of range")
     lo, hi = GMW_CLAMP
+    Z, _ = _EdgeSolve.apply(kps, kps_3d, rot, None, lo, hi, 0, True, False)
     with torch.no_grad():
-        Z, _ = _EdgeSolve.apply(kps, kps_3d, rot, None, lo, hi, 0, True, False)
         idx = torch.empty((N, num_k), dtype=torch.int64, device=kps.device)
         if N:
             check(_lib.lib().dcd_edge_select_fwd(ptr(kps), ptr(kps_3d), ptr(rot), 0, 0, N, n, num_k, lo, hi, 0,
@@ -437,6 +440,29 @@ def _alloc_bytes(nbytes: int, dev) -> torch.Tensor:
     if POISON_WORKSPACES:
         t.fill_(float("nan"))       # the kernels must never read what they did not write
     return t
+
+
+def _mlp_backward(ctx, kpts_2d, kpts_3d, params4, params6, depth, g_reg_w, gn4, gn6):
+    """dcd_gmw_weights_bwd over the activations the forward saved in ctx.ws, then dcd_gmw_kpts_bwd from the same scratch
+    when a keypoint tensor needs a gradient -> (d kpts_2d, d kpts_3d, d params4, d params6), None where not needed.
+    Frozen parameters still take the parameter backward (it fills the scratch the keypoint gradient is read from): its
+    blobs are thrown away."""
+    N, n = kpts_2d.shape[0], kpts_2d.shape[1]
+    need = ctx.needs_input_grad
+    g4 = torch.zeros_like(params4)
+    g6 = torch.zeros_like(params6)
+    gk2 = torch.zeros_like(kpts_2d) if need[0] else None
+    gk3 = torch.zeros_like(kpts_3d) if need[1] else None
+    if N and (g_reg_w is not None or gn4 is not None or gn6 is not None):
+        L = _lib.lib()
+        scratch = _alloc_bytes(L.dcd_gmw_bwd_scratch_bytes(N, n, depth), kpts_2d.device)
+        check(L.dcd_gmw_weights_bwd(ptr(kpts_2d), ptr(kpts_3d), ptr(params4), ptr(params6), N, n, depth,
+                                    ptr(g_reg_w), ptr(gn4), ptr(gn6), ptr(g4), ptr(g6), ptr(ctx.ws), ctx.ws.numel() * 4,
+                                    ptr(scratch), scratch.numel() * 4, stream_ptr()), "dcd_gmw_weights_bwd")
+        if gk2 is not None or gk3 is not None:
+            check(L.dcd_gmw_kpts_bwd(ptr(params4), ptr(params6), N, n, depth, ptr(scratch), scratch.numel() * 4,
+                                     ptr(gk2), ptr(gk3), stream_ptr()), "dcd_gmw_kpts_bwd")
+    return gk2, gk3, (g4 if need[2] else None), (g6 if need[3] else None)
 
 
 class _GmwWeights(torch.autograd.Function):
@@ -463,18 +489,9 @@ class _GmwWeights(torch.autograd.Function):
     @staticmethod
     def backward(ctx, g_reg_w):
         kpts_2d, kpts_3d, params4, params6 = ctx.saved_tensors
-        N, n = kpts_2d.shape[0], kpts_2d.shape[1]
-        L = _lib.lib()
-        g4 = torch.zeros_like(params4)
-        g6 = torch.zeros_like(params6)
-        if N:
-            g = f32c(g_reg_w)
-            scratch = _alloc_bytes(L.dcd_gmw_bwd_scratch_bytes(N, n, ctx.depth), g.device)
-            check(L.dcd_gmw_weights_bwd(ptr(kpts_2d), ptr(kpts_3d), ptr(params4), ptr(params6), N, n, ctx.depth,
-                                        ptr(g), 0, 0, ptr(g4), ptr(g6), ptr(ctx.ws), ctx.ws.numel() * 4,
-                                        ptr(scratch), scratch.numel() * 4, stream_ptr()), "dcd_gmw_weights_bwd")
+        grads = _mlp_backward(ctx, kpts_2d, kpts_3d, params4, params6, ctx.depth, f32c(g_reg_w), None, None)
         ctx.ws = None
-        return None, None, g4, g6, None, None
+        return grads + (None, None)
 
 
 SINKHORN_CG_ITERATIONS, SINKHORN_CG_TOLERANCE = 32, 1e-7
@@ -482,8 +499,9 @@ SINKHORN_CG_ITERATIONS, SINKHORN_CG_TOLERANCE = 32, 1e-7
 
 class _GmwWeightsTransport(torch.autograd.Function):
     """GMW.forward with both outputs like the reference (GMW/model/model.py:195-207): reg_weights [b,E] and the Sinkhorn
-    transport plan edge_P [b,E,E], both differentiable w.r.t. the parameter blobs.  Backward = implicit gradient of the
-    Sinkhorn fixed point (optimal_transport.py:75-128 as one conjugate-gradient solve) -> feature gradients -> MLP backward."""
+    transport plan edge_P [b,E,E], both differentiable w.r.t. the parameter blobs and the keypoints.  Backward = implicit
+    gradient of the Sinkhorn fixed point (optimal_transport.py:75-128 as one conjugate-gradient solve) -> feature gradients
+    -> MLP backward."""
 
     @staticmethod
     def forward(ctx, kpts_2d, kpts_3d, params4, params6, depth, need_grad, lam, tol, iters):
@@ -518,24 +536,18 @@ class _GmwWeightsTransport(torch.autograd.Function):
         depth, lam = ctx.cfg
         N, n = kpts_2d.shape[0], kpts_2d.shape[1]
         L = _lib.lib()
-        g4 = torch.zeros_like(params4)
-        g6 = torch.zeros_like(params6)
-        if N and (g_reg_w is not None or g_P is not None):
-            gn4 = gn6 = None
-            if g_P is not None:
-                gP = f32c(g_P)
-                gn4, gn6 = torch.empty_like(f4), torch.empty_like(f6)
-                tws = _alloc_bytes(L.dcd_gmw_transport_bwd_workspace_bytes(N, n), gP.device)
-                check(L.dcd_gmw_transport_bwd(ptr(f4), ptr(f6), ptr(P), ptr(u), ptr(v), ptr(gP), N, n, lam,
-                                              SINKHORN_CG_ITERATIONS, SINKHORN_CG_TOLERANCE, ptr(gn4), ptr(gn6), 0,
-                                              ptr(tws), tws.numel() * 4, stream_ptr()), "dcd_gmw_transport_bwd")
-            g = f32c(g_reg_w) if g_reg_w is not None else None
-            scratch = _alloc_bytes(L.dcd_gmw_bwd_scratch_bytes(N, n, depth), kpts_2d.device)
-            check(L.dcd_gmw_weights_bwd(ptr(kpts_2d), ptr(kpts_3d), ptr(params4), ptr(params6), N, n, depth,
-                                        ptr(g), ptr(gn4), ptr(gn6), ptr(g4), ptr(g6), ptr(ctx.ws), ctx.ws.numel() * 4,
-                                        ptr(scratch), scratch.numel() * 4, stream_ptr()), "dcd_gmw_weights_bwd")
+        gn4 = gn6 = None
+        if N and g_P is not None:
+            gP = f32c(g_P)
+            gn4, gn6 = torch.empty_like(f4), torch.empty_like(f6)
+            tws = _alloc_bytes(L.dcd_gmw_transport_bwd_workspace_bytes(N, n), gP.device)
+            check(L.dcd_gmw_transport_bwd(ptr(f4), ptr(f6), ptr(P), ptr(u), ptr(v), ptr(gP), N, n, lam,
+                                          SINKHORN_CG_ITERATIONS, SINKHORN_CG_TOLERANCE, ptr(gn4), ptr(gn6), 0,
+                                          ptr(tws), tws.numel() * 4, stream_ptr()), "dcd_gmw_transport_bwd")
+        g = f32c(g_reg_w) if g_reg_w is not None else None
+        grads = _mlp_backward(ctx, kpts_2d, kpts_3d, params4, params6, depth, g, gn4, gn6)
         ctx.ws = None
-        return None, None, g4, g6, None, None, None, None, None
+        return grads + (None, None, None, None, None)
 
 
 class _GmwAggregate(torch.autograd.Function):
@@ -571,7 +583,9 @@ class GMW(nn.Module):
     of the classification branch, SURVEY 8f row N1) is None unless the module attribute `with_edge_P`
     is set (dcd_b200.patch.install sets it: both loops of GMW/main.py consume edge_P, :456 and :526); then it
     is the [b,E,E] transport plan, differentiable like the reference's (implicit Sinkhorn gradient,
-    optimal_transport.py:75-128).  `edge_transport` gives the plan's (sum, trace) without materialising it.
+    optimal_transport.py:75-128).  Both outputs are differentiable w.r.t. kpts_2d and kpts_3d as well (frozen parameters
+    and keypoints that require grad: a trained GMW as a differentiable refiner of upstream keypoints).
+    `edge_transport` gives the plan's (sum, trace) without materialising it.
     Parameters live in two flat blobs; `load_state_dict`/`state_dict` of the *reference* format
     are available through `load_reference_state_dict` / `reference_state_dict`.
     """
@@ -643,7 +657,9 @@ class GMW(nn.Module):
         k2, k3 = f32c(kpts_2d), f32c(kpts_3d)
         if k2.dim() != 3 or k2.shape[-1] != 2 or tuple(k3.shape) != (k2.shape[0], k2.shape[1], 3):
             raise ValueError("kpts_2d must be [b,n,2] and kpts_3d [b,n,3]")
-        need_grad = torch.is_grad_enabled() and (params4.requires_grad or params6.requires_grad)
+        # the layer-wise forward that saves its activations runs whenever autograd will call the backward; otherwise
+        # (torch.no_grad(), or nothing requires grad) the on-chip inference forward
+        need_grad = torch.is_grad_enabled() and any(t.requires_grad for t in (k2, k3, params4, params6))
         if self.with_edge_P:
             return _GmwWeightsTransport.apply(k2, k3, params4, params6, self.depth, need_grad, self.SINKHORN_LAMBDA,
                                               self.SINKHORN_TOLERANCE, self.SINKHORN_ITERATIONS)

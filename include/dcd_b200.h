@@ -211,6 +211,15 @@ int dcd_gmw_weights_bwd(const float* kpts2d, const float* kpts3d, const float* p
                         void* workspace, size_t workspace_bytes, void* scratch, size_t scratch_bytes,
                         void* stream);
 
+/* Backward of dcd_gmw_weights_fwd w.r.t. the keypoints, from the scratch that dcd_gmw_weights_bwd just filled
+ * (same N, n, depth, params; same stream; nothing written to the scratch in between).  grad_kpts2d [N,n,2],
+ * grad_kpts3d [N,n,3], each may be NULL (not both), OVERWRITTEN.  Deterministic.
+ * The chain below the first residual block is linear: dF = W_in^T-contraction of dL/d(conv_in output) per edge
+ * (GMW/model/yi2018cvpr/model.py:63), then the backward of edge_expand (GMW/model/model.py:153-163) as a per-keypoint
+ * gather over the n-1 incident edges (fixed order, no atomics).  dcd_gmw_weights_bwd's own outputs do not change. */
+int dcd_gmw_kpts_bwd(const float* params4, const float* params6, int64_t N, int n, int depth,
+                     void* scratch, size_t scratch_bytes, float* grad_kpts2d, float* grad_kpts3d, void* stream);
+
 /* ------------------------------------------------------------------------------------------------
  * GMW weighted aggregation.  Replaces the forward of compute_reg_loss (GMW/main.py:364-371):
  * depth_out[N] = sum_r softmax_r(reg_weights[idx[r]]) * depths[idx[r]].  depths is [N,E] when
