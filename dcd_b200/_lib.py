@@ -38,6 +38,8 @@ SIGNATURES = {
     "dcd_gmw_bwd_scratch_bytes": (c_size_t, [c_int64, c_int, c_int]),
     "dcd_gmw_transport_bwd_workspace_bytes": (c_size_t, [c_int64, c_int]),
     "dcd_gmw_transport_bwd": (c_int, [c_void_p] * 6 + [c_int64, c_int, c_float, c_int, c_float] + [c_void_p] * 4 + [c_size_t, c_void_p]),
+    "dcd_gmw_transport_terms_bwd": (c_int, [c_void_p] * 3 + [c_size_t] + [c_void_p] * 3 + [c_int64, c_int, c_float, c_int, c_float]
+                                    + [c_void_p] * 4 + [c_size_t, c_void_p]),
     "dcd_gmw_weights_bwd": (c_int, [c_void_p] * 4 + [c_int64, c_int, c_int] + [c_void_p] * 6 + [c_size_t, c_void_p, c_size_t, c_void_p]),
     "dcd_gmw_kpts_bwd": (c_int, [c_void_p] * 2 + [c_int64, c_int, c_int, c_void_p, c_size_t, c_void_p, c_void_p, c_void_p]),
     "dcd_gmw_aggregate_fwd": (c_int, [c_void_p] * 3 + [c_int64, c_int64, c_int, c_int, c_void_p, c_void_p, c_void_p]),

@@ -34,6 +34,9 @@ int launch_gmw_kpts_bwd(const float*, const float*, int64_t, int, int, float*, f
 size_t gmw_transport_bwd_workspace_bytes(int64_t N, int E);
 int launch_gmw_transport_bwd(const float*, const float*, const float*, const float*, const float*, const float*, int64_t, int, float,
                              int, float, float*, float*, float*, void*, cudaStream_t);
+const float* gmw_transport_workspace_k(const void*);
+int launch_gmw_transport_terms_bwd(const float*, const float*, const float*, const float*, const float*, const float*, int64_t, int,
+                                   float, int, float, float*, float*, float*, void*, cudaStream_t);
 }  // namespace dcd
 
 using namespace dcd;
@@ -192,6 +195,21 @@ int dcd_gmw_transport_bwd(const float* feat4, const float* feat6, const float* P
     if (misaligned(workspace, 256) || workspace_bytes < dcd_gmw_transport_bwd_workspace_bytes(N, n)) return DCD_E_WORKSPACE;
     return launch_gmw_transport_bwd(feat4, feat6, P, u, v, grad_P, N, (int)num_edges(n), lambda, max_cg_iterations, cg_tolerance,
                                     grad_nfeat4, grad_nfeat6, cg_info, workspace, (cudaStream_t)stream);
+}
+
+int dcd_gmw_transport_terms_bwd(const float* feat4, const float* feat6, const void* fwd_workspace, size_t fwd_workspace_bytes,
+                                const float* u, const float* v, const float* grad_terms, int64_t N, int n, float lambda,
+                                int max_cg_iterations, float cg_tolerance, float* grad_nfeat4, float* grad_nfeat6, float* cg_info,
+                                void* workspace, size_t workspace_bytes, void* stream) {
+    if (N < 1 || bad_n(n) || max_cg_iterations < 1 || !(lambda > 0.f) || !(cg_tolerance >= 0.f)) return DCD_E_INVALID;
+    if (!feat4 || !feat6 || !fwd_workspace || !u || !v || !grad_terms || !grad_nfeat4 || !grad_nfeat6 || !workspace)
+        return DCD_E_INVALID;
+    if (N > 65535) return DCD_E_UNSUPPORTED;
+    if (misaligned(fwd_workspace, 256) || fwd_workspace_bytes < dcd_gmw_transport_workspace_bytes(N, n)) return DCD_E_WORKSPACE;
+    if (misaligned(workspace, 256) || workspace_bytes < dcd_gmw_transport_bwd_workspace_bytes(N, n)) return DCD_E_WORKSPACE;
+    return launch_gmw_transport_terms_bwd(feat4, feat6, gmw_transport_workspace_k(fwd_workspace), u, v, grad_terms, N,
+                                          (int)num_edges(n), lambda, max_cg_iterations, cg_tolerance, grad_nfeat4, grad_nfeat6,
+                                          cg_info, workspace, (cudaStream_t)stream);
 }
 
 size_t dcd_gmw_param_count(int cin, int depth) { return (size_t)blob_size(cin, depth); }

@@ -363,6 +363,9 @@ size_t gmw_transport_workspace_bytes(int64_t N, int E) {
            al((size_t)N * 2 * e * 4) + 256;
 }
 
+// K inside a workspace filled by launch_gmw_transport_fwd (its first block, [N][E][E]): the plan source of the terms backward
+const float* gmw_transport_workspace_k(const void* workspace) { return reinterpret_cast<const float*>(workspace); }
+
 int launch_gmw_transport_fwd(const float* feat4, const float* feat6, int64_t N, int E, float lambda, float tol, int max_iter,
                              float* P, float* u_out, float* v_out, float* sums, void* workspace, cudaStream_t st) {
     const size_t e = (size_t)E;

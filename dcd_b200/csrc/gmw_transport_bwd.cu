@@ -18,6 +18,9 @@
 //     dL/da_i = (sum_j W_ij) a_i - sum_j W_ij c_j,      dL/dc_j = (sum_i W_ij) c_j - sum_i W_ij a_i
 // (a, c the normalised features) as two tiled FP32 products that never materialise W.
 // Deterministic: fixed-order partial sums, no floating-point atomics.
+// Two instantiations of the same passes: the dense one (P and V read from [N][E][E] tensors, dcd_gmw_transport_bwd) and the
+// terms one for a loss on (sum P, trace P) only (dcd_gmw_transport_terms_bwd): P rebuilt from the forward's K, u, v and
+// V = alpha 11^T + beta I formed in registers, so that only K is E x E; same results bit for bit on the same P and V values.
 #include "gmw_mlp.cuh"
 
 namespace dcd {
@@ -42,9 +45,93 @@ struct TbWs {                           // per-object vectors of length E unless
     float* nrm;     // [4][E]: |f4|, |f6| (clamped), then unused
 };
 
+// Sources of the two E x E operands of the passes below, the plan P and V = dL/dP.  A kernel binds a source to its object
+// (`bind`) and reads row i through `row(i)`: at(j) one entry, at4(j) the four entries j..j+3 (j % 4 == 0, 16-byte aligned).
+//   PlanDense  the P that dcd_gmw_transport_fwd wrote.
+//   PlanFromK  P rebuilt from that call's K, u and v as (u_i K_ij) v_j: the two roundings of transport_p_kernel, so every
+//              entry is bit-identical to the written plan and nothing E x E but K is read.
+//   GradDense  a dense V [N][E][E] (streamed: read once per pass).
+//   GradTerms  V = alpha 11^T + beta I, the gradient of a loss on (sum P, trace P), from terms [N][2] = (alpha, beta) in
+//              registers; alpha + beta is rounded once per object.
+// With the same P and V values the two instantiations run the same loads-to-arithmetic sequence: same results, bit for bit.
+struct PlanDense {
+    const float* P;
+    struct Row {
+        const float* p;
+        __device__ __forceinline__ float at(int j) const { return __ldg(p + j); }
+        __device__ __forceinline__ float4 at4(int j) const { return __ldg(reinterpret_cast<const float4*>(p + j)); }
+    };
+    struct Obj {
+        const float* P;
+        int E;
+        __device__ __forceinline__ Row row(int i) const { return {P + (int64_t)i * E}; }
+    };
+    __device__ __forceinline__ Obj bind(int64_t obj, int E) const { return {P + obj * (int64_t)E * E, E}; }
+};
+
+struct PlanFromK {
+    const float* K;
+    const float* u;
+    const float* v;
+    struct Row {
+        const float* k;
+        float ui;
+        const float* v;
+        __device__ __forceinline__ float at(int j) const { return __fmul_rn(__fmul_rn(ui, __ldg(k + j)), __ldg(v + j)); }
+        __device__ __forceinline__ float4 at4(int j) const {
+            const float4 kk = __ldg(reinterpret_cast<const float4*>(k + j));
+            return make_float4(__fmul_rn(__fmul_rn(ui, kk.x), __ldg(v + j)), __fmul_rn(__fmul_rn(ui, kk.y), __ldg(v + j + 1)),
+                               __fmul_rn(__fmul_rn(ui, kk.z), __ldg(v + j + 2)), __fmul_rn(__fmul_rn(ui, kk.w), __ldg(v + j + 3)));
+        }
+    };
+    struct Obj {
+        const float* K;
+        const float* u;
+        const float* v;
+        int E;
+        __device__ __forceinline__ Row row(int i) const { return {K + (int64_t)i * E, __ldg(u + i), v}; }
+    };
+    __device__ __forceinline__ Obj bind(int64_t obj, int E) const {
+        return {K + obj * (int64_t)E * E, u + obj * (int64_t)E, v + obj * (int64_t)E, E};
+    }
+};
+
+struct GradDense {
+    const float* V;
+    struct Row {
+        const float* p;
+        __device__ __forceinline__ float at(int j) const { return __ldcs(p + j); }
+        __device__ __forceinline__ float4 at4(int j) const { return __ldcs(reinterpret_cast<const float4*>(p + j)); }
+    };
+    struct Obj {
+        const float* V;
+        int E;
+        __device__ __forceinline__ Row row(int i) const { return {V + (int64_t)i * E}; }
+    };
+    __device__ __forceinline__ Obj bind(int64_t obj, int E) const { return {V + obj * (int64_t)E * E, E}; }
+};
+
+struct GradTerms {
+    const float* terms;
+    struct Row {
+        float off, diag;
+        int i;
+        __device__ __forceinline__ float at(int j) const { return j == i ? diag : off; }
+        __device__ __forceinline__ float4 at4(int j) const { return make_float4(at(j), at(j + 1), at(j + 2), at(j + 3)); }
+    };
+    struct Obj {
+        float off, diag;
+        __device__ __forceinline__ Row row(int i) const { return {off, diag, i}; }
+    };
+    __device__ __forceinline__ Obj bind(int64_t obj, int) const {
+        const float alpha = __ldg(terms + 2 * obj);
+        return {alpha, __fadd_rn(alpha, __ldg(terms + 2 * obj + 1))};
+    }
+};
+
 // warp per row i of P
-template <int MODE>
-__global__ void __launch_bounds__(256) tb_row_kernel(const float* __restrict__ P, const float* __restrict__ V, int E, float lambda,
+template <int MODE, class Plan, class Grad>
+__global__ void __launch_bounds__(256) tb_row_kernel(Plan plan, Grad grad, int E, float lambda,
                                                      const float* __restrict__ vec, const float* __restrict__ r1, const float* __restrict__ u1,
                                                      const float* __restrict__ scal, float* __restrict__ out0, float* __restrict__ out1,
                                                      int64_t stride_scal) {
@@ -52,20 +139,18 @@ __global__ void __launch_bounds__(256) tb_row_kernel(const float* __restrict__ P
     if (MODE == ROW_MATVEC && scal[obj * stride_scal + 2] != 0.f) return;         // this object's CG has converged
     const int i = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
     if (i >= E) return;
-    const float* Pp = P + (obj * E + i) * (int64_t)E;
-    const float* Vp = MODE == ROW_INIT ? V + (obj * E + i) * (int64_t)E : nullptr;
+    const auto Pp = plan.bind(obj, E).row(i);
+    const auto Vp = grad.bind(obj, E).row(i);                                      // read by ROW_INIT only
     const float* xp = MODE == ROW_INIT ? nullptr : vec + obj * (int64_t)E;
     float a = 0.f, b = 0.f;
     if ((E & 3) == 0) {
-        const float4* P4 = reinterpret_cast<const float4*>(Pp);
-        const float4* V4 = reinterpret_cast<const float4*>(Vp);
         const float4* x4 = reinterpret_cast<const float4*>(xp);
         const int E4 = E >> 2;
 #pragma unroll 4
         for (int j = lane; j < E4; j += 32) {
-            const float4 p = P4[j];
-            if (MODE == ROW_INIT) {
-                const float4 v = __ldcs(V4 + j);
+            const float4 p = Pp.at4(4 * j);
+            if constexpr (MODE == ROW_INIT) {
+                const float4 v = Vp.at4(4 * j);
                 a += (p.x + p.y) + (p.z + p.w);
                 b = fmaf(p.w, v.w, fmaf(p.z, v.z, fmaf(p.y, v.y, fmaf(p.x, v.x, b))));
             } else {
@@ -75,8 +160,8 @@ __global__ void __launch_bounds__(256) tb_row_kernel(const float* __restrict__ P
         }
     } else {
         for (int j = lane; j < E; j += 32) {
-            const float p = Pp[j];
-            if (MODE == ROW_INIT) { a += p; b = fmaf(p, Vp[j], b); }
+            const float p = Pp.at(j);
+            if constexpr (MODE == ROW_INIT) { a += p; b = fmaf(p, Vp.at(j), b); }
             else a = fmaf(p, xp[j], a);
         }
     }
@@ -106,8 +191,8 @@ __global__ void __launch_bounds__(256) tb_y0_kernel(const float* __restrict__ u1
 
 // thread per column j, rows split into TB_CHUNKS chunks: part[0][chunk][j] = sum_i P_ij t_i  (INIT: t = 1 and
 // part[1] = sum_i P_ij V_ij)
-template <bool INIT>
-__global__ void __launch_bounds__(256) tb_col_kernel(const float* __restrict__ P, const float* __restrict__ V, int E,
+template <bool INIT, class Plan, class Grad>
+__global__ void __launch_bounds__(256) tb_col_kernel(Plan plan, Grad grad, int E,
                                                      const float* __restrict__ t, const float* __restrict__ scal, int64_t stride_scal,
                                                      float* __restrict__ part) {
     const int64_t obj = blockIdx.z;
@@ -116,14 +201,14 @@ __global__ void __launch_bounds__(256) tb_col_kernel(const float* __restrict__ P
     const int rows = (E + TB_CHUNKS - 1) / TB_CHUNKS;
     const int ib = blockIdx.y * rows, ie = min(E, ib + rows);
     if (j >= E) return;
-    const float* Pp = P + obj * (int64_t)E * E + j;
-    const float* Vp = INIT ? V + obj * (int64_t)E * E + j : nullptr;
+    const auto Pm = plan.bind(obj, E);
+    const auto Vm = grad.bind(obj, E);                                             // read by INIT only
     const float* tp = INIT ? nullptr : t + obj * (int64_t)E;
     float a = 0.f, b = 0.f;
 #pragma unroll 4
     for (int i = ib; i < ie; ++i) {
-        const float p = Pp[(int64_t)i * E];
-        if (INIT) { a += p; b = fmaf(p, __ldcs(Vp + (int64_t)i * E), b); }
+        const float p = Pm.row(i).at(j);
+        if constexpr (INIT) { a += p; b = fmaf(p, Vm.row(i).at(j), b); }
         else a = fmaf(p, tp[i], a);
     }
     float* o = part + (obj * 2 * TB_CHUNKS + blockIdx.y) * (int64_t)E + j;
@@ -250,9 +335,8 @@ constexpr int FT = 64;
 constexpr int FT_WS = FT + 4;           // WsT[k][own] row stride (floats; keeps 16-byte alignment)
 constexpr size_t kFeatSmem = ((size_t)FT * FT_WS + (size_t)FT * CH + 4 * FT + 2 * FT) * sizeof(float);
 
-template <bool TRANS>
-__global__ void __launch_bounds__(256) tb_feat_kernel(const float* __restrict__ P, const float* __restrict__ V,
-                                                      const float* __restrict__ feat_own, const float* __restrict__ feat_oth,
+template <bool TRANS, class Plan, class Grad>
+__global__ void __launch_bounds__(256) tb_feat_kernel(Plan plan, Grad grad, const float* __restrict__ feat_own, const float* __restrict__ feat_oth,
                                                       const float* __restrict__ nrm, int64_t stride_nrm,
                                                       const float* __restrict__ uvec, const float* __restrict__ vvec,
                                                       const float* __restrict__ u3, const float* __restrict__ x,
@@ -269,8 +353,8 @@ __global__ void __launch_bounds__(256) tb_feat_kernel(const float* __restrict__ 
     const int64_t vo = obj * (int64_t)E;
     const float* n_own = nrm + obj * stride_nrm + (TRANS ? E : 0);
     const float* n_oth = nrm + obj * stride_nrm + (TRANS ? 0 : E);
-    const float* Pm = P + obj * (int64_t)E * E;
-    const float* Vm = V + obj * (int64_t)E * E;
+    const auto Pm = plan.bind(obj, E);
+    const auto Vm = grad.bind(obj, E);
 
     // tile-load mapping: `lo` = own index inside the tile, `seg` = 16 consecutive k
     const int lo = tid & 63, seg = tid >> 6;
@@ -316,8 +400,8 @@ __global__ void __launch_bounds__(256) tb_feat_kernel(const float* __restrict__ 
                 float4 p = make_float4(0.f, 0.f, 0.f, 0.f), v = p;
                 const bool ok = own_ok && k < E;             // E % 4 == 0: the four columns are valid together
                 if (ok) {
-                    p = *reinterpret_cast<const float4*>(Pm + (int64_t)own * E + k);
-                    v = __ldcs(reinterpret_cast<const float4*>(Vm + (int64_t)own * E + k));
+                    p = Pm.row(own).at4(k);
+                    v = Vm.row(own).at4(k);
                 }
                 const float pp[4] = {p.x, p.y, p.z, p.w}, vv[4] = {v.x, v.y, v.z, v.w};
 #pragma unroll
@@ -333,8 +417,8 @@ __global__ void __launch_bounds__(256) tb_feat_kernel(const float* __restrict__ 
                 const int kk = seg * 16 + q, k = k0 + kk;
                 float wv = 0.f;
                 if (own_ok && k < E) {
-                    const int64_t off = TRANS ? (int64_t)k * E + own : (int64_t)own * E + k;
-                    const float p = Pm[off], v = __ldcs(Vm + off);
+                    const int r = TRANS ? k : own, c = TRANS ? own : k;
+                    const float p = Pm.row(r).at(c), v = Vm.row(r).at(c);
                     wv = TRANS ? w_entry(p, v, kvec_s[kk], own_a, kvec_s[FT + kk], own_ln, lambda, inv_lambda)
                                : w_entry(p, v, own_a, kvec_s[kk], own_ln, kvec_s[FT + kk], lambda, inv_lambda);
                 }
@@ -393,9 +477,12 @@ size_t gmw_transport_bwd_workspace_bytes(int64_t N, int E) {
     return 9 * al((size_t)N * e * 4) + al((size_t)N * 2 * TB_CHUNKS * e * 4) + al((size_t)N * 2 * e * 4) + al((size_t)N * 8 * 4);
 }
 
-int launch_gmw_transport_bwd(const float* feat4, const float* feat6, const float* P, const float* u, const float* v,
-                             const float* gradP, int64_t N, int E, float lambda, int max_iter, float tol,
-                             float* gn4, float* gn6, float* cg_info, void* workspace, cudaStream_t st) {
+namespace {
+
+// the whole backward on one pair of operand sources (see PlanDense ... GradTerms)
+template <class Plan, class Grad>
+int run_transport_bwd(Plan P, Grad gradP, const float* feat4, const float* feat6, const float* u, const float* v, int64_t N, int E,
+                      float lambda, int max_iter, float tol, float* gn4, float* gn6, float* cg_info, void* workspace, cudaStream_t st) {
     if (E > 256 * TB_EPT) return DCD_E_UNSUPPORTED;
     const size_t e = (size_t)E;
     unsigned char* p = reinterpret_cast<unsigned char*>(workspace);
@@ -417,28 +504,45 @@ int launch_gmw_transport_bwd(const float* feat4, const float* feat6, const float
     tb_cg_kernel<CG_INIT><<<(unsigned)N, 256, 0, st>>>(w, E, lambda, 0.f, sv);
     // rhs = u2 - B'^T (u1 / r1)
     tb_y0_kernel<<<vgrid, 256, 0, st>>>(w.u1, w.r1, E, w.y);
-    tb_col_kernel<false><<<cgrid, 256, 0, st>>>(P, nullptr, E, w.y, nullptr, 8, w.part);
+    tb_col_kernel<false><<<cgrid, 256, 0, st>>>(P, gradP, E, w.y, nullptr, 8, w.part);
     tb_cg_kernel<CG_RHS><<<(unsigned)N, 256, 0, st>>>(w, E, lambda, 0.f, sv);
     DCD_CHECK_LAUNCH();
     // conjugate gradients on S x = rhs, S p = c2 * p - B'^T ((B' p) / r1); converged objects skip their passes
     for (int it = 0; it < max_iter; ++it) {
-        tb_row_kernel<ROW_MATVEC><<<rgrid, 256, 0, st>>>(P, nullptr, E, lambda, w.p, w.r1, nullptr, w.scal, w.y, nullptr, 8);
-        tb_col_kernel<false><<<cgrid, 256, 0, st>>>(P, nullptr, E, w.y, w.scal, 8, w.part);
+        tb_row_kernel<ROW_MATVEC><<<rgrid, 256, 0, st>>>(P, gradP, E, lambda, w.p, w.r1, nullptr, w.scal, w.y, nullptr, 8);
+        tb_col_kernel<false><<<cgrid, 256, 0, st>>>(P, gradP, E, w.y, w.scal, 8, w.part);
         tb_cg_kernel<CG_UPDATE><<<(unsigned)N, 256, 0, st>>>(w, E, lambda, tol * tol, sv);
     }
     DCD_CHECK_LAUNCH();
     // u3 = (u1 - B' x) / r1
-    tb_row_kernel<ROW_U3><<<rgrid, 256, 0, st>>>(P, nullptr, E, lambda, w.x, w.r1, w.u1, nullptr, w.u3, nullptr, 8);
+    tb_row_kernel<ROW_U3><<<rgrid, 256, 0, st>>>(P, gradP, E, lambda, w.x, w.r1, w.u1, nullptr, w.u3, nullptr, 8);
     // gradients of the normalised features
     tb_norm_kernel<<<vgrid, 256, 0, st>>>(feat4, feat6, E, w.nrm, 2 * sv);
-    cudaFuncSetAttribute(tb_feat_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFeatSmem);
-    cudaFuncSetAttribute(tb_feat_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFeatSmem);
+    cudaFuncSetAttribute(tb_feat_kernel<false, Plan, Grad>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFeatSmem);
+    cudaFuncSetAttribute(tb_feat_kernel<true, Plan, Grad>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFeatSmem);
     const dim3 fgrid((unsigned)((E + FT - 1) / FT), (unsigned)N);
     tb_feat_kernel<false><<<fgrid, 256, kFeatSmem, st>>>(P, gradP, feat4, feat6, w.nrm, 2 * sv, u, v, w.u3, w.x, E, lambda, gn4);
     tb_feat_kernel<true><<<fgrid, 256, kFeatSmem, st>>>(P, gradP, feat6, feat4, w.nrm, 2 * sv, u, v, w.u3, w.x, E, lambda, gn6);
     if (cg_info != nullptr) cudaMemcpyAsync(cg_info, w.scal, (size_t)N * 8 * sizeof(float), cudaMemcpyDeviceToDevice, st);
     DCD_CHECK_LAUNCH();
     return DCD_OK;
+}
+
+}  // namespace
+
+int launch_gmw_transport_bwd(const float* feat4, const float* feat6, const float* P, const float* u, const float* v,
+                             const float* gradP, int64_t N, int E, float lambda, int max_iter, float tol,
+                             float* gn4, float* gn6, float* cg_info, void* workspace, cudaStream_t st) {
+    return run_transport_bwd(PlanDense{P}, GradDense{gradP}, feat4, feat6, u, v, N, E, lambda, max_iter, tol, gn4, gn6, cg_info,
+                             workspace, st);
+}
+
+// the plan from the forward's K (+ u, v), dL/dP = alpha 11^T + beta I from grad_terms [N][2]
+int launch_gmw_transport_terms_bwd(const float* feat4, const float* feat6, const float* K, const float* u, const float* v,
+                                   const float* grad_terms, int64_t N, int E, float lambda, int max_iter, float tol,
+                                   float* gn4, float* gn6, float* cg_info, void* workspace, cudaStream_t st) {
+    return run_transport_bwd(PlanFromK{K, u, v}, GradTerms{grad_terms}, feat4, feat6, u, v, N, E, lambda, max_iter, tol, gn4, gn6,
+                             cg_info, workspace, st);
 }
 
 }  // namespace dcd

@@ -550,6 +550,70 @@ class _GmwWeightsTransport(torch.autograd.Function):
         return grads + (None, None, None, None, None)
 
 
+class _GmwTransportTerms(torch.autograd.Function):
+    """reg_weights [b,E] and the plan's two sums, terms [b,2] = (sum P, trace P), without the plan: the forward runs the
+    Sinkhorn with P = NULL and keeps K (its workspace), u and v; the backward takes dL/dP = alpha 11^T + beta I from
+    (alpha, beta) = dL/dterms and rebuilds P from K, u, v inside the kernels (dcd_gmw_transport_terms_bwd).  The only E x E
+    tensor alive between forward and backward is K.  Same gradients as _GmwWeightsTransport with dL/dP of that form."""
+
+    @staticmethod
+    def forward(ctx, kpts_2d, kpts_3d, params4, params6, depth, need_grad, lam, tol, iters):
+        N, n = kpts_2d.shape[0], kpts_2d.shape[1]
+        E = _num_edges(n)
+        dev = kpts_2d.device
+        L = _lib.lib()
+        reg_w = torch.empty((N, E), dtype=torch.float32, device=dev)
+        terms = torch.empty((N, 2), dtype=torch.float32, device=dev)
+        ctx.set_materialize_grads(False)          # an unused output passes None: no transport backward for a reg-only loss
+        f4 = f6 = u = v = ws = tws = None
+        if N:
+            save = 1 if need_grad else 0
+            f4 = torch.empty((N, 128, E), dtype=torch.float32, device=dev)
+            f6 = torch.empty((N, 128, E), dtype=torch.float32, device=dev)
+            if need_grad:
+                u = torch.empty((N, E), dtype=torch.float32, device=dev)
+                v = torch.empty((N, E), dtype=torch.float32, device=dev)
+            ws = _alloc_bytes(L.dcd_gmw_workspace_bytes(N, n, depth, save), dev)
+            check(L.dcd_gmw_weights_fwd(ptr(kpts_2d), ptr(kpts_3d), ptr(params4), ptr(params6), N, n, depth, save,
+                                        ptr(reg_w), ptr(f4), ptr(f6), ptr(ws), ws.numel() * 4, stream_ptr()), "dcd_gmw_weights_fwd")
+            if not need_grad:
+                ws = None
+            tws = _alloc_bytes(L.dcd_gmw_transport_workspace_bytes(N, n), dev)
+            check(L.dcd_gmw_transport_fwd(ptr(f4), ptr(f6), N, n, lam, tol, iters, 0, ptr(u), ptr(v), ptr(terms),
+                                          ptr(tws), tws.numel() * 4, stream_ptr()), "dcd_gmw_transport_fwd")
+        if need_grad:
+            ctx.save_for_backward(kpts_2d, kpts_3d, params4, params6, f4, f6, u, v)
+            ctx.ws, ctx.tws = ws, tws
+            ctx.cfg = (depth, lam)
+        return reg_w, terms
+
+    @staticmethod
+    def backward(ctx, g_reg_w, g_terms):
+        kpts_2d, kpts_3d, params4, params6, f4, f6, u, v = ctx.saved_tensors
+        depth, lam = ctx.cfg
+        N, n = kpts_2d.shape[0], kpts_2d.shape[1]
+        L = _lib.lib()
+        gn4 = gn6 = None
+        if N and g_terms is not None:
+            gt = f32c(g_terms)
+            gn4, gn6 = torch.empty_like(f4), torch.empty_like(f6)
+            bws = _alloc_bytes(L.dcd_gmw_transport_bwd_workspace_bytes(N, n), gt.device)
+            check(L.dcd_gmw_transport_terms_bwd(ptr(f4), ptr(f6), ptr(ctx.tws), ctx.tws.numel() * 4, ptr(u), ptr(v), ptr(gt),
+                                                N, n, lam, SINKHORN_CG_ITERATIONS, SINKHORN_CG_TOLERANCE, ptr(gn4), ptr(gn6), 0,
+                                                ptr(bws), bws.numel() * 4, stream_ptr()), "dcd_gmw_transport_terms_bwd")
+        ctx.tws = None
+        g = f32c(g_reg_w) if g_reg_w is not None else None
+        grads = _mlp_backward(ctx, kpts_2d, kpts_3d, params4, params6, depth, g, gn4, gn6)
+        ctx.ws = None
+        return grads + (None, None, None, None, None)
+
+
+def correspondence_loss(terms: torch.Tensor) -> torch.Tensor:
+    """correspondenceLoss(edge_P, eye) of GMW/main.py:456-457 (lib/losses.py:22-26,115-119) from GMW.transport_terms's
+    terms [b,2] = (sum P, trace P): mean over objects of sum - 2 trace."""
+    return (terms[:, 0] - 2 * terms[:, 1]).mean()
+
+
 class _GmwAggregate(torch.autograd.Function):
     @staticmethod
     def forward(ctx, reg_w, depths, idx):
@@ -585,7 +649,8 @@ class GMW(nn.Module):
     is the [b,E,E] transport plan, differentiable like the reference's (implicit Sinkhorn gradient,
     optimal_transport.py:75-128).  Both outputs are differentiable w.r.t. kpts_2d and kpts_3d as well (frozen parameters
     and keypoints that require grad: a trained GMW as a differentiable refiner of upstream keypoints).
-    `edge_transport` gives the plan's (sum, trace) without materialising it.
+    `edge_transport` gives the plan's (sum, trace) without materialising it; `transport_terms` gives them differentiably
+    (with `correspondence_loss`, the correspondence loss at the memory cost of K alone).
     Parameters live in two flat blobs; `load_state_dict`/`state_dict` of the *reference* format
     are available through `load_reference_state_dict` / `reference_state_dict`.
     """
@@ -647,12 +712,23 @@ class GMW(nn.Module):
                                           ptr(tws), tws.numel() * 4, stream_ptr()), "dcd_gmw_transport_fwd")
         return reg_w, P, sums
 
+    def transport_terms(self, kpts_2d, kpts_3d, params=None):
+        """Differentiable correspondence branch without the plan: (reg_weights [b,E], terms [b,2] = (sum P, trace P)).
+        correspondenceLoss(edge_P, eye) of GMW/main.py:456-457 is `dcd_b200.correspondence_loss(terms)`.  Both outputs are
+        differentiable w.r.t. the parameter blobs and the keypoints like forward()'s; the gradient of the plan goes through
+        the same implicit Sinkhorn backward as edge_P's, rebuilding P from the forward's K (dcd_gmw_transport_terms_bwd),
+        so the E x E tensors of edge_P, of the loss and of dL/dP are never formed: K (4 E^2 bytes per object) is the only one
+        kept for the backward.  Under torch.no_grad() this is edge_transport(materialise=False) without the plan."""
+        p4, p6 = params if params is not None else (self.params4, self.params6)
+        k2, k3, need_grad = self._prepare(kpts_2d, kpts_3d, p4, p6)
+        return _GmwTransportTerms.apply(k2, k3, p4, p6, self.depth, need_grad, self.SINKHORN_LAMBDA, self.SINKHORN_TOLERANCE,
+                                        self.SINKHORN_ITERATIONS)
+
     def forward(self, kpts_2d, kpts_3d, pred_rot=None, args=None):
         return self.forward_blobs(kpts_2d, kpts_3d, self.params4, self.params6)
 
-    def forward_blobs(self, kpts_2d, kpts_3d, params4, params6):
-        """forward() on explicit parameter blobs (dcd_b200.patch passes blobs packed from the LIVE reference parameters,
-        so that their optimizer, checkpoints and DDP hooks keep working unchanged)."""
+    @staticmethod
+    def _prepare(kpts_2d, kpts_3d, params4, params6):
         require_cuda(kpts_2d, kpts_3d, params4, params6)
         k2, k3 = f32c(kpts_2d), f32c(kpts_3d)
         if k2.dim() != 3 or k2.shape[-1] != 2 or tuple(k3.shape) != (k2.shape[0], k2.shape[1], 3):
@@ -660,6 +736,12 @@ class GMW(nn.Module):
         # the layer-wise forward that saves its activations runs whenever autograd will call the backward; otherwise
         # (torch.no_grad(), or nothing requires grad) the on-chip inference forward
         need_grad = torch.is_grad_enabled() and any(t.requires_grad for t in (k2, k3, params4, params6))
+        return k2, k3, need_grad
+
+    def forward_blobs(self, kpts_2d, kpts_3d, params4, params6):
+        """forward() on explicit parameter blobs (dcd_b200.patch passes blobs packed from the LIVE reference parameters,
+        so that their optimizer, checkpoints and DDP hooks keep working unchanged)."""
+        k2, k3, need_grad = self._prepare(kpts_2d, kpts_3d, params4, params6)
         if self.with_edge_P:
             return _GmwWeightsTransport.apply(k2, k3, params4, params6, self.depth, need_grad, self.SINKHORN_LAMBDA,
                                               self.SINKHORN_TOLERANCE, self.SINKHORN_ITERATIONS)

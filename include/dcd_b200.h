@@ -196,6 +196,19 @@ int dcd_gmw_transport_bwd(const float* feat4, const float* feat6, const float* P
                           float* grad_nfeat4, float* grad_nfeat6, float* cg_info, void* workspace, size_t workspace_bytes,
                           void* stream);
 
+/* The same backward for a loss on the plan's two sums only, L(sum P, trace P) (correspondenceLoss, lib/losses.py:115-119),
+ * without any E x E tensor besides the forward's K.  dL/dP is then alpha 11^T + beta I per object, with grad_terms [N,2] =
+ * (alpha, beta) = (dL/d sum P, dL/d trace P), formed in registers; the plan is rebuilt entry by entry from K, u and v as
+ * (u_i K_ij) v_j, the forward's own two roundings.  With the same plan and the same dL/dP values this gives grad_nfeat4 /
+ * grad_nfeat6 and cg_info bit-identical to dcd_gmw_transport_bwd with a dense grad_P.
+ * fwd_workspace: the workspace of the dcd_gmw_transport_fwd call (same N, n, lambda; P may have been NULL there), which holds
+ * K; nothing may be written to it in between.  u, v: that call's u / v outputs; feat4 / feat6: its inputs.  The workspace is
+ * sized by dcd_gmw_transport_bwd_workspace_bytes.  N >= 1. */
+int dcd_gmw_transport_terms_bwd(const float* feat4, const float* feat6, const void* fwd_workspace, size_t fwd_workspace_bytes,
+                                const float* u, const float* v, const float* grad_terms, int64_t N, int n, float lambda,
+                                int max_cg_iterations, float cg_tolerance, float* grad_nfeat4, float* grad_nfeat6, float* cg_info,
+                                void* workspace, size_t workspace_bytes, void* stream);
+
 /* Backward of dcd_gmw_weights_fwd w.r.t. the parameters (autograd of GMW/main.py:465).
  * workspace: the one filled by the forward call with save=1 (same N, n, depth).  grad_reg_weights [N,E] (reg path) and/or
  * grad_nfeat4 / grad_nfeat6 [N,128,E] (gradient w.r.t. the normalised final features, from dcd_gmw_transport_bwd: cls path);
