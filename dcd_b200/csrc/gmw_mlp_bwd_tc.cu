@@ -13,10 +13,12 @@
 //     MN-major B operand of the data-gradient GEMM (A = W^T resident in tensor memory) and the K-major A operand
 //     of the weight-gradient GEMM (B = A2 image, K = edges) — only the descriptors differ;
 //   * FP32 fidelity: FP16x3 split (3 MMAs per product) as in the forward; the gradient image is scaled by a
-//     power of two derived from the running maximum of the upstream gradient (tracked with one atomicMax per
-//     warp in the producing epilogue), so hi/lo stay inside FP16's normal range;
-//   * the 128x128 weight gradient ACCUMULATES IN TENSOR MEMORY across all tiles of the CTA and is written once
-//     per CTA as a partial, reduced in a fixed order afterwards (deterministic, no float atomics);
+//     power of two derived from the running maximum of the object's upstream gradient (tracked per object with one
+//     atomicMax per warp in the producing epilogue), so hi/lo stay inside FP16's normal range whatever the other
+//     objects' gradients are (a batch-wide maximum left an object 2^-12 below it with a subnormal lo part);
+//   * the 128x128 weight gradient ACCUMULATES IN TENSOR MEMORY across the tiles of one object within the CTA; at each
+//     object change and at the end it is unscaled into the CTA's partial (written by the first object, added to by the
+//     next), reduced over the CTAs in a fixed order afterwards (deterministic, no float atomics);
 //   * block conv biases receive exact zeros: they are cancelled by the mean subtraction that follows each of
 //     them (SURVEY 7-H5; the reference's own values there are rounding noise around 1e-8).
 #include "gmw_tc_common.cuh"
@@ -37,7 +39,7 @@ struct BwdTcArgs {
     float2* bstat;          // [2][2][N][T][128] partial sums of the context-norm backward
     float* wpart;           // [3][2 * ctas][128*128] per-CTA partial weight gradients
     float* inpart;          // [2*N*T][128][8] partial conv_in gradients
-    float* gmax;            // [2][3*depth + 1] running |gradient| maxima (float bits, >= 0)
+    float* gmax;            // [2][N][3*depth + 1] running |gradient| maxima per object (float bits, >= 0)
 };
 
 size_t tc_fold_offset_bytes(int depth);
@@ -57,7 +59,9 @@ constexpr size_t SMB_RED = SMB_SB + CH * sizeof(float2);           // [4][128] f
 constexpr size_t SMB_BAR = SMB_RED + 4 * CH * sizeof(float2);
 constexpr size_t kBwdTcSmem = SMB_BAR + 64;
 
-__device__ __forceinline__ int gmax_slot(int depth, int net, int blk, int stage) { return net * (3 * depth + 1) + blk * 3 + stage; }
+__device__ __forceinline__ int64_t gmax_slot(const WsLayout& L, int net, int64_t obj, int blk, int stage) {
+    return ((int64_t)net * L.N + obj) * (3 * L.depth + 1) + blk * 3 + stage;
+}
 
 __device__ __forceinline__ void atomic_max_abs(float* slot, float v) {
     v = warp_max(v);
@@ -85,8 +89,8 @@ __device__ __forceinline__ void load_chunk(const unsigned char* hi, const unsign
     }
 }
 
-__global__ void bwd_tc_init_kernel(float* gmax, int n) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+__global__ void bwd_tc_init_kernel(float* gmax, int64_t n) {
+    const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (i < n) gmax[i] = 0.f;
 }
 
@@ -160,8 +164,8 @@ __global__ void __launch_bounds__(256) edge_weight_bwd_tc_kernel(BwdTcArgs a, co
             m6 = fmaxf(m6, fabsf(g6));
         }
     }
-    atomic_max_abs(a.gmax + gmax_slot(L.depth, 0, last, 0), m4);
-    atomic_max_abs(a.gmax + gmax_slot(L.depth, 1, last, 0), m6);
+    atomic_max_abs(a.gmax + gmax_slot(L, 0, obj, last, 0), m4);
+    atomic_max_abs(a.gmax + gmax_slot(L, 1, obj, last, 0), m6);
 }
 
 // partial sums (sum dyh, sum dyh*yh) of the second context norm's backward, dyh = G * (yh > 0)
@@ -243,12 +247,9 @@ __global__ void __launch_bounds__(BT_THREADS, 1) mlp_bwd_tc_kernel(BwdTcArgs a, 
     if (warp < 8)
         load_weight_row_to_tmem_T(MODE == MODE_R3F ? a.fold + ((int64_t)net * L.depth + blk) * FOLD_STRIDE : prm + blob_w(cin, blk, which),
                                   wsc.x, ch, tmem_base + lane_off + TMB_W_HI, tmem_base + lane_off + TMB_W_LO, cq & 1);
-    // scale of the gradient image from the running maximum of what feeds it
-    const float gin = a.gmax[gmax_slot(L.depth, net, blk, MODE == MODE_R3F ? 1 : MODE)];
-    const float gs = pow2_scale(gin, 4);                              // |dy| <= ~1700 x the tracked maximum
-    const float un_d = wsc.y / gs;                                    // data-gradient accumulator -> FP32
-    float* gout = a.gmax + (kResidual ? (blk > 0 ? gmax_slot(L.depth, net, blk - 1, 0) : gmax_slot(L.depth, net, L.depth, 0))
-                                             : gmax_slot(L.depth, net, blk, MODE + 1));
+    // the stage's slots of the per-object maxima: read (what feeds the gradient image) and written (this launch's output)
+    const int in_blk = blk, in_stage = MODE == MODE_R3F ? 1 : MODE;
+    const int out_blk = kResidual ? (blk > 0 ? blk - 1 : L.depth) : blk, out_stage = kResidual ? 0 : MODE + 1;
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
@@ -259,6 +260,25 @@ __global__ void __launch_bounds__(BT_THREADS, 1) mlp_bwd_tc_kernel(BwdTcArgs a, 
     uint32_t mma_phase = 0;
     int64_t stat_obj = -1;
     float omax = 0.f;
+    float gs = 1.f, un_d = 0.f;       // the current object's image scale and data-gradient unscale
+    float* part = a.wpart + (((int64_t)which * 2 + net) * gridDim.x + blockIdx.x) * (CH * CH) + (int64_t)ch * CH + cq * 32;
+    bool part_written = false;
+    // the weight gradient accumulated in tensor memory for one object -> (unscaled) into this CTA's partial
+    auto flush_wgrad = [&]() {
+        float v[32];
+        tmem_ld32(tmem_base + TMB_DW + lane_off + (uint32_t)(cq * 32), v);
+        const float un_w = 1.f / gs;
+#pragma unroll
+        for (int i = 0; i < 32; i += 4) {
+            float4 w = make_float4(v[i] * un_w, v[i + 1] * un_w, v[i + 2] * un_w, v[i + 3] * un_w);
+            if (part_written) {
+                const float4 p = *reinterpret_cast<const float4*>(part + i);
+                w.x += p.x; w.y += p.y; w.z += p.z; w.w += p.w;
+            }
+            *reinterpret_cast<float4*>(part + i) = w;
+        }
+        part_written = true;
+    };
 
     for (int64_t t = t_begin; t < t_end; ++t) {
         const int64_t obj = t / T;
@@ -266,8 +286,17 @@ __global__ void __launch_bounds__(BT_THREADS, 1) mlp_bwd_tc_kernel(BwdTcArgs a, 
         const int64_t obj_off = obj * (int64_t)CH * EP;
         const int valid = min(TE, E - tile * TE);
         const int64_t gobj = ((int64_t)net * L.N + obj) * CH * EP;
+        const bool new_obj = stat_obj != obj;          // CTA-uniform
 
-        if (stat_obj != obj) {
+        if (new_obj) {
+            if (stat_obj >= 0) {                       // leave the previous object: its output maximum and weight gradient
+                atomic_max_abs(a.gmax + gmax_slot(L, net, stat_obj, out_blk, out_stage), omax);
+                omax = 0.f;
+                flush_wgrad();
+            }
+            // scale of the gradient image from the running maximum of what feeds it, for this object
+            gs = pow2_scale(a.gmax[gmax_slot(L, net, obj, in_blk, in_stage)], 4);   // |dy| <= ~1700 x the tracked maximum
+            un_d = wsc.y / gs;                                                     // data-gradient accumulator -> FP32
             if (tid < CH) {
                 st1_s[tid] = merge_cn_stats(stat_ptr(a.ws, L, net, blk, 0) + obj * (int64_t)T * CH, tid, T, E);
                 if (MODE == MODE_R2)
@@ -343,8 +372,8 @@ __global__ void __launch_bounds__(BT_THREADS, 1) mlp_bwd_tc_kernel(BwdTcArgs a, 
         __syncthreads();
         if (warp == 0 && elect_one()) {
             tc_fence_after();
-            // weight gradient: D_w[o][i] += sum_e A1[o][e] A2[i][e]   (both K-major views, accumulates over tiles)
-            uint32_t acc = (t == t_begin) ? 0u : 1u;
+            // weight gradient: D_w[o][i] += sum_e A1[o][e] A2[i][e]   (both K-major views, accumulates over the object's tiles)
+            uint32_t acc = new_obj ? 0u : 1u;
 #pragma unroll
             for (int term = 0; term < 3; ++term) {
                 const uint32_t pa = smem_u32(term == 1 ? A1_lo : A1_hi);
@@ -417,17 +446,10 @@ __global__ void __launch_bounds__(BT_THREADS, 1) mlp_bwd_tc_kernel(BwdTcArgs a, 
             __syncthreads();                                 // images free for the next tile
         }
     }
-    atomic_max_abs(gout, omax);
-
-    // ---- weight gradient of this CTA's tiles: tensor memory -> one partial per CTA
-    if (t_begin < t_end) {
-        float v[32];
-        tmem_ld32(tmem_base + TMB_DW + lane_off + (uint32_t)(cq * 32), v);
-        const float un_w = 1.f / gs;
-        float* part = a.wpart + (((int64_t)which * 2 + net) * gridDim.x + blockIdx.x) * (CH * CH) + (int64_t)ch * CH + cq * 32;
-#pragma unroll
-        for (int i = 0; i < 32; i += 4)
-            *reinterpret_cast<float4*>(part + i) = make_float4(v[i] * un_w, v[i + 1] * un_w, v[i + 2] * un_w, v[i + 3] * un_w);
+    // ---- the last object of this CTA's tiles: output maximum, weight gradient -> the CTA's partial
+    if (stat_obj >= 0) {
+        atomic_max_abs(a.gmax + gmax_slot(L, net, stat_obj, out_blk, out_stage), omax);
+        flush_wgrad();
     }
     tc_fence_before();
     __syncthreads();
@@ -652,7 +674,7 @@ BwdTcScratch bwd_tc_layout(const WsLayout& L, int ctas) {
     s.bstat = take((int64_t)2 * 2 * L.stat * 2);
     s.wpart = take((int64_t)3 * 2 * ctas * CH * CH);
     s.inpart = take((int64_t)2 * L.N * L.T * CH * 8);
-    s.gmax = take((int64_t)2 * (3 * L.depth + 1));
+    s.gmax = take((int64_t)2 * L.N * (3 * L.depth + 1));
     s.dwf = take((int64_t)2 * CH * CH);
     s.total = o;
     return s;
@@ -700,8 +722,8 @@ int launch_gmw_weights_bwd(const float* kpts2d, const float* kpts3d, const float
     cudaFuncSetAttribute(mlp_bwd_tc_kernel<MODE_R2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kBwdTcSmem);
     cudaFuncSetAttribute(mlp_bwd_tc_kernel<MODE_R3F>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kBwdTcSmem);
 
-    const int ng = 2 * (3 * depth + 1);
-    bwd_tc_init_kernel<<<(ng + 127) / 128, 128, 0, st>>>(a.gmax, ng);
+    const int64_t ng = 2 * N * (3 * depth + 1);
+    bwd_tc_init_kernel<<<(unsigned)((ng + 127) / 128), 128, 0, st>>>(a.gmax, ng);
     const unsigned g0 = (unsigned)(((a.L.E + 255) / 256) * N);
     edge_weight_bwd_tc_kernel<<<g0, 256, 0, st>>>(a, grad_reg_w, grad_nfeat4, grad_nfeat6);
     const dim3 tgrid((unsigned)(a.L.T * N), 2);
