@@ -9,9 +9,10 @@ launch per step.  Gradients land in the model's parameter blobs' .grad exactly a
     loss = step(kpts_2d, kpts_3d, pred_rot, gt_depth)        # == eager: compute_z -> model -> losses -> backward
     optimizer.step()
 
-With cls_weight != 0 the step adds the correspondence loss (GMW/main.py:455-457).  plan_free=True takes it from
-GMW.transport_terms + correspondence_loss instead of the [b,E,E] plan edge_P: same gradients bit for bit, and no E x E
-tensor but the Sinkhorn kernel K is allocated (not the plan, the loss's [b,E,E] temporaries or a dense dL/dP).
+With cls_weight != 0 the step adds the correspondence loss (GMW/main.py:455-457), taken from GMW.transport_terms +
+correspondence_loss instead of the [b,E,E] plan edge_P: the same gradients bit for bit as through edge_P, and no E x E
+tensor but the Sinkhorn kernel K is allocated (not the plan, the loss's [b,E,E] temporaries or a dense dL/dP).  With
+cls_weight == 0 the Sinkhorn branch does not run, whatever the model's with_edge_P says.
 """
 from __future__ import annotations
 
@@ -22,14 +23,13 @@ from . import ops
 
 class GraphedGmwStep:
     def __init__(self, model: "ops.GMW", batch: int, n: int = 73, cls_weight: float = 0.0, reg_weight: float = 1.0,
-                 warmup: int = 3, plan_free: bool = False):
+                 warmup: int = 3):
         p = model.params4
         if not p.is_cuda:
             raise RuntimeError("GraphedGmwStep needs the model on a CUDA device")
         dev = p.device
         self.model = model
         self.cls_weight, self.reg_weight = float(cls_weight), float(reg_weight)
-        self.plan_free = bool(plan_free)
         self.k2 = torch.zeros((batch, n, 2), device=dev)
         self.k3 = torch.zeros((batch, n, 3), device=dev)
         self.rot = torch.zeros((batch, 1), device=dev)
@@ -43,23 +43,14 @@ class GraphedGmwStep:
     def _eager(self):
         model = self.model
         Z, idx = ops.compute_z(self.k2, self.k3, self.rot)
-        if self.plan_free and self.cls_weight != 0.0:
+        if self.cls_weight != 0.0:
             w, terms = model.transport_terms(self.k2, self.k3)
-            reg, zsel = ops.compute_reg_loss(Z, w, self.gt, idx)
-            loss = self.reg_weight * reg + self.cls_weight * ops.correspondence_loss(terms)
-            loss.backward()
-            return loss.detach(), zsel.detach()
-        saved = model.with_edge_P
-        model.with_edge_P = self.cls_weight != 0.0
-        try:
-            w, P = model(self.k2, self.k3, self.rot, None)
-        finally:
-            model.with_edge_P = saved
+        else:
+            w, terms = model._edge_branch(None, self.k2, self.k3, model.params4, model.params6)
         reg, zsel = ops.compute_reg_loss(Z, w, self.gt, idx)
         loss = self.reg_weight * reg
-        if P is not None:
-            eye = torch.eye(P.shape[1], device=P.device).expand_as(P)         # GMW/main.py:456-457
-            loss = loss + self.cls_weight * ((1.0 - 2.0 * eye) * P).sum(dim=(-2, -1)).mean()
+        if terms is not None:
+            loss = loss + self.cls_weight * ops.correspondence_loss(terms)
         loss.backward()
         return loss.detach(), zsel.detach()
 

@@ -24,7 +24,7 @@ from . import _lib
 from ._lib import check, f32c, ptr, require_cuda, stream_ptr
 from .weights import NET_DEPTH, NET_NAMES, blob_size, pack_state_dict, unpack_blob
 
-_CHECK_FINITE = os.environ.get("DCD_B200_CHECK_FINITE", "0") == "1"   # debug: synchronising range check of GMW.forward
+_CHECK_FINITE = os.environ.get("DCD_B200_CHECK_FINITE", "0") == "1"   # debug: synchronising range check of the GMW edge weights
 K_SEL = 1500                 # anno_encoder.py:378, GMW/main.py:413
 DGDE_CLAMP = (2.0, 80.0)     # anno_encoder.py:375
 GMW_CLAMP = (0.1, 80.0)      # GMW/main.py:410
@@ -465,147 +465,92 @@ def _mlp_backward(ctx, kpts_2d, kpts_3d, params4, params6, depth, g_reg_w, gn4, 
     return gk2, gk3, (g4 if need[2] else None), (g6 if need[3] else None)
 
 
-class _GmwWeights(torch.autograd.Function):
-    @staticmethod
-    def forward(ctx, kpts_2d, kpts_3d, params4, params6, depth, need_grad):
-        N, n = kpts_2d.shape[0], kpts_2d.shape[1]
-        E = _num_edges(n)
-        dev = kpts_2d.device
-        L = _lib.lib()
-        reg_w = torch.empty((N, E), dtype=torch.float32, device=dev)
-        save = 1 if need_grad else 0
-        ws = None
-        if N:
-            nbytes = L.dcd_gmw_workspace_bytes(N, n, depth, save)
-            ws = _alloc_bytes(nbytes, dev)
-            check(L.dcd_gmw_weights_fwd(ptr(kpts_2d), ptr(kpts_3d), ptr(params4), ptr(params6), N, n, depth, save,
-                                        ptr(reg_w), 0, 0, ptr(ws), ws.numel() * 4, stream_ptr()), "dcd_gmw_weights_fwd")
-        if need_grad:
-            ctx.save_for_backward(kpts_2d, kpts_3d, params4, params6)
-            ctx.ws = ws
-            ctx.depth = depth
-        return reg_w
-
-    @staticmethod
-    def backward(ctx, g_reg_w):
-        kpts_2d, kpts_3d, params4, params6 = ctx.saved_tensors
-        grads = _mlp_backward(ctx, kpts_2d, kpts_3d, params4, params6, ctx.depth, f32c(g_reg_w), None, None)
-        ctx.ws = None
-        return grads + (None, None)
-
-
 SINKHORN_CG_ITERATIONS, SINKHORN_CG_TOLERANCE = 32, 1e-7
 
 
-class _GmwWeightsTransport(torch.autograd.Function):
-    """GMW.forward with both outputs like the reference (GMW/model/model.py:195-207): reg_weights [b,E] and the Sinkhorn
-    transport plan edge_P [b,E,E], both differentiable w.r.t. the parameter blobs and the keypoints.  Backward = implicit
-    gradient of the Sinkhorn fixed point (optimal_transport.py:75-128 as one conjugate-gradient solve) -> feature gradients
-    -> MLP backward."""
-
-    @staticmethod
-    def forward(ctx, kpts_2d, kpts_3d, params4, params6, depth, need_grad, lam, tol, iters):
-        N, n = kpts_2d.shape[0], kpts_2d.shape[1]
-        E = _num_edges(n)
-        dev = kpts_2d.device
-        L = _lib.lib()
-        reg_w = torch.empty((N, E), dtype=torch.float32, device=dev)
-        P = torch.empty((N, E, E), dtype=torch.float32, device=dev)
-        u = torch.empty((N, E), dtype=torch.float32, device=dev)
-        v = torch.empty((N, E), dtype=torch.float32, device=dev)
-        f4 = torch.empty((N, 128, E), dtype=torch.float32, device=dev)
-        f6 = torch.empty((N, 128, E), dtype=torch.float32, device=dev)
-        save = 1 if need_grad else 0
-        ws = None
-        if N:
-            ws = _alloc_bytes(L.dcd_gmw_workspace_bytes(N, n, depth, save), dev)
-            check(L.dcd_gmw_weights_fwd(ptr(kpts_2d), ptr(kpts_3d), ptr(params4), ptr(params6), N, n, depth, save,
-                                        ptr(reg_w), ptr(f4), ptr(f6), ptr(ws), ws.numel() * 4, stream_ptr()), "dcd_gmw_weights_fwd")
-            tws = _alloc_bytes(L.dcd_gmw_transport_workspace_bytes(N, n), dev)
-            check(L.dcd_gmw_transport_fwd(ptr(f4), ptr(f6), N, n, lam, tol, iters, ptr(P), ptr(u), ptr(v), 0,
-                                          ptr(tws), tws.numel() * 4, stream_ptr()), "dcd_gmw_transport_fwd")
-        if need_grad:
-            ctx.save_for_backward(kpts_2d, kpts_3d, params4, params6, f4, f6, P, u, v)
-            ctx.ws = ws
-            ctx.cfg = (depth, lam)
-        return reg_w, P
-
-    @staticmethod
-    def backward(ctx, g_reg_w, g_P):
-        kpts_2d, kpts_3d, params4, params6, f4, f6, P, u, v = ctx.saved_tensors
-        depth, lam = ctx.cfg
-        N, n = kpts_2d.shape[0], kpts_2d.shape[1]
-        L = _lib.lib()
-        gn4 = gn6 = None
-        if N and g_P is not None:
-            gP = f32c(g_P)
-            gn4, gn6 = torch.empty_like(f4), torch.empty_like(f6)
-            tws = _alloc_bytes(L.dcd_gmw_transport_bwd_workspace_bytes(N, n), gP.device)
-            check(L.dcd_gmw_transport_bwd(ptr(f4), ptr(f6), ptr(P), ptr(u), ptr(v), ptr(gP), N, n, lam,
-                                          SINKHORN_CG_ITERATIONS, SINKHORN_CG_TOLERANCE, ptr(gn4), ptr(gn6), 0,
-                                          ptr(tws), tws.numel() * 4, stream_ptr()), "dcd_gmw_transport_bwd")
-        g = f32c(g_reg_w) if g_reg_w is not None else None
-        grads = _mlp_backward(ctx, kpts_2d, kpts_3d, params4, params6, depth, g, gn4, gn6)
-        ctx.ws = None
-        return grads + (None, None, None, None, None)
-
-
-class _GmwTransportTerms(torch.autograd.Function):
-    """reg_weights [b,E] and the plan's two sums, terms [b,2] = (sum P, trace P), without the plan: the forward runs the
-    Sinkhorn with P = NULL and keeps K (its workspace), u and v; the backward takes dL/dP = alpha 11^T + beta I from
-    (alpha, beta) = dL/dterms and rebuilds P from K, u, v inside the kernels (dcd_gmw_transport_terms_bwd).  The only E x E
-    tensor alive between forward and backward is K.  Same gradients as _GmwWeightsTransport with dL/dP of that form."""
-
-    @staticmethod
-    def forward(ctx, kpts_2d, kpts_3d, params4, params6, depth, need_grad, lam, tol, iters):
-        N, n = kpts_2d.shape[0], kpts_2d.shape[1]
-        E = _num_edges(n)
-        dev = kpts_2d.device
-        L = _lib.lib()
-        reg_w = torch.empty((N, E), dtype=torch.float32, device=dev)
-        terms = torch.empty((N, 2), dtype=torch.float32, device=dev)
-        ctx.set_materialize_grads(False)          # an unused output passes None: no transport backward for a reg-only loss
-        f4 = f6 = u = v = ws = tws = None
-        if N:
-            save = 1 if need_grad else 0
+def _gmw_forward(kpts_2d, kpts_3d, params4, params6, depth, save, plan, sums, lam, tol, iters):
+    """Edge MLP (dcd_gmw_weights_fwd), then the Sinkhorn correspondence branch (dcd_gmw_transport_fwd, GMW/model/model.py:
+    170-192) when `plan` or `sums` asks for it -> (reg_weights [N,E], edge_P [N,E,E] or None, (sum P, trace P) [N,2] or
+    None, kept).  kept = (MLP workspace, f4, f6, u, v, Sinkhorn workspace whose first block is K) holds what a backward
+    reads; with save=False (no backward will run) the MLP workspace is released before the Sinkhorn workspace is allocated
+    and u, v are not written."""
+    N, n = kpts_2d.shape[0], kpts_2d.shape[1]
+    E = _num_edges(n)
+    dev = kpts_2d.device
+    L = _lib.lib()
+    transport = plan or sums
+    reg_w = torch.empty((N, E), dtype=torch.float32, device=dev)
+    P = torch.empty((N, E, E), dtype=torch.float32, device=dev) if plan else None
+    terms = torch.empty((N, 2), dtype=torch.float32, device=dev) if sums else None
+    ws = f4 = f6 = u = v = tws = None
+    if N:
+        if transport:
             f4 = torch.empty((N, 128, E), dtype=torch.float32, device=dev)
             f6 = torch.empty((N, 128, E), dtype=torch.float32, device=dev)
-            if need_grad:
+        ws = _alloc_bytes(L.dcd_gmw_workspace_bytes(N, n, depth, int(save)), dev)
+        check(L.dcd_gmw_weights_fwd(ptr(kpts_2d), ptr(kpts_3d), ptr(params4), ptr(params6), N, n, depth, int(save),
+                                    ptr(reg_w), ptr(f4), ptr(f6), ptr(ws), ws.numel() * 4, stream_ptr()), "dcd_gmw_weights_fwd")
+        if _CHECK_FINITE and not bool(torch.isfinite(reg_w).all()):
+            # the tensor-core path carries activations as FP16 hi+lo pairs: |activation| must stay below 65504
+            raise FloatingPointError("dcd_b200.GMW: non-finite edge weights (activation outside the FP16 hi/lo range?)")
+        if not save:
+            ws = None
+        if transport:
+            if save:
                 u = torch.empty((N, E), dtype=torch.float32, device=dev)
                 v = torch.empty((N, E), dtype=torch.float32, device=dev)
-            ws = _alloc_bytes(L.dcd_gmw_workspace_bytes(N, n, depth, save), dev)
-            check(L.dcd_gmw_weights_fwd(ptr(kpts_2d), ptr(kpts_3d), ptr(params4), ptr(params6), N, n, depth, save,
-                                        ptr(reg_w), ptr(f4), ptr(f6), ptr(ws), ws.numel() * 4, stream_ptr()), "dcd_gmw_weights_fwd")
-            if not need_grad:
-                ws = None
             tws = _alloc_bytes(L.dcd_gmw_transport_workspace_bytes(N, n), dev)
-            check(L.dcd_gmw_transport_fwd(ptr(f4), ptr(f6), N, n, lam, tol, iters, 0, ptr(u), ptr(v), ptr(terms),
+            check(L.dcd_gmw_transport_fwd(ptr(f4), ptr(f6), N, n, lam, tol, iters, ptr(P), ptr(u), ptr(v), ptr(terms),
                                           ptr(tws), tws.numel() * 4, stream_ptr()), "dcd_gmw_transport_fwd")
-        if need_grad:
-            ctx.save_for_backward(kpts_2d, kpts_3d, params4, params6, f4, f6, u, v)
-            ctx.ws, ctx.tws = ws, tws
-            ctx.cfg = (depth, lam)
-        return reg_w, terms
+    return reg_w, P, terms, (ws, f4, f6, u, v, tws)
+
+
+class _GmwEdgeBranch(torch.autograd.Function):
+    """GMW.forward like the reference (GMW/model/model.py:195-207): reg_weights [b,E] and, by `branch`, no second output
+    (None), the Sinkhorn transport plan edge_P [b,E,E] ("plan") or its two sums terms [b,2] = (sum P, trace P) ("terms"),
+    all differentiable w.r.t. the parameter blobs and the keypoints.  Backward = implicit gradient of the Sinkhorn fixed
+    point (optimal_transport.py:75-128 as one conjugate-gradient solve) -> feature gradients -> MLP backward.  For "terms"
+    dL/dP = alpha 11^T + beta I with (alpha, beta) = dL/dterms: the backward rebuilds P from the forward's K, u and v inside
+    the kernels (dcd_gmw_transport_terms_bwd), so K is the only E x E tensor kept between forward and backward, and the
+    gradients equal the "plan" branch's for a dL/dP of that form.  An output the loss does not use passes no gradient
+    (set_materialize_grads(False)): a reg_weights-only loss runs no transport backward on either branch."""
 
     @staticmethod
-    def backward(ctx, g_reg_w, g_terms):
-        kpts_2d, kpts_3d, params4, params6, f4, f6, u, v = ctx.saved_tensors
-        depth, lam = ctx.cfg
+    def forward(ctx, kpts_2d, kpts_3d, params4, params6, depth, need_grad, branch, lam, tol, iters):
+        ctx.set_materialize_grads(False)
+        reg_w, P, terms, (ws, f4, f6, u, v, tws) = _gmw_forward(kpts_2d, kpts_3d, params4, params6, depth, need_grad,
+                                                                branch == "plan", branch == "terms", lam, tol, iters)
+        if need_grad:
+            ctx.save_for_backward(kpts_2d, kpts_3d, params4, params6, f4, f6, u, v, P)
+            ctx.ws, ctx.tws = ws, (tws if branch == "terms" else None)
+            ctx.cfg = (depth, branch, lam)
+        return reg_w, (P if branch == "plan" else terms)
+
+    @staticmethod
+    def backward(ctx, g_reg_w, g_second):
+        kpts_2d, kpts_3d, params4, params6, f4, f6, u, v, P = ctx.saved_tensors
+        depth, branch, lam = ctx.cfg
         N, n = kpts_2d.shape[0], kpts_2d.shape[1]
         L = _lib.lib()
         gn4 = gn6 = None
-        if N and g_terms is not None:
-            gt = f32c(g_terms)
+        if N and g_second is not None:
+            g = f32c(g_second)
             gn4, gn6 = torch.empty_like(f4), torch.empty_like(f6)
-            bws = _alloc_bytes(L.dcd_gmw_transport_bwd_workspace_bytes(N, n), gt.device)
-            check(L.dcd_gmw_transport_terms_bwd(ptr(f4), ptr(f6), ptr(ctx.tws), ctx.tws.numel() * 4, ptr(u), ptr(v), ptr(gt),
-                                                N, n, lam, SINKHORN_CG_ITERATIONS, SINKHORN_CG_TOLERANCE, ptr(gn4), ptr(gn6), 0,
-                                                ptr(bws), bws.numel() * 4, stream_ptr()), "dcd_gmw_transport_terms_bwd")
+            bws = _alloc_bytes(L.dcd_gmw_transport_bwd_workspace_bytes(N, n), g.device)
+            if branch == "plan":
+                check(L.dcd_gmw_transport_bwd(ptr(f4), ptr(f6), ptr(P), ptr(u), ptr(v), ptr(g), N, n, lam,
+                                              SINKHORN_CG_ITERATIONS, SINKHORN_CG_TOLERANCE, ptr(gn4), ptr(gn6), 0,
+                                              ptr(bws), bws.numel() * 4, stream_ptr()), "dcd_gmw_transport_bwd")
+            else:
+                check(L.dcd_gmw_transport_terms_bwd(ptr(f4), ptr(f6), ptr(ctx.tws), ctx.tws.numel() * 4, ptr(u), ptr(v),
+                                                    ptr(g), N, n, lam, SINKHORN_CG_ITERATIONS, SINKHORN_CG_TOLERANCE,
+                                                    ptr(gn4), ptr(gn6), 0, ptr(bws), bws.numel() * 4, stream_ptr()),
+                      "dcd_gmw_transport_terms_bwd")
         ctx.tws = None
         g = f32c(g_reg_w) if g_reg_w is not None else None
         grads = _mlp_backward(ctx, kpts_2d, kpts_3d, params4, params6, depth, g, gn4, gn6)
         ctx.ws = None
-        return grads + (None, None, None, None, None)
+        return grads + (None,) * 6
 
 
 def correspondence_loss(terms: torch.Tensor) -> torch.Tensor:
@@ -690,27 +635,9 @@ class GMW(nn.Module):
         correspondenceLoss(edge_P, eye) of GMW/main.py:456-457 is `(cls_terms[:, 0] - 2 * cls_terms[:, 1]).mean()`;
         with materialise=False the 4 E^2 bytes per object of edge_P are never written.  No gradient."""
         p4, p6 = params if params is not None else (self.params4, self.params6)
-        require_cuda(kpts_2d, kpts_3d, p4, p6)
-        k2, k3 = f32c(kpts_2d), f32c(kpts_3d)
-        N, n = k2.shape[0], k2.shape[1]
-        E = _num_edges(n)
-        dev = k2.device
-        L = _lib.lib()
-        reg_w = torch.empty((N, E), dtype=torch.float32, device=dev)
-        P = torch.empty((N, E, E), dtype=torch.float32, device=dev) if materialise else None
-        sums = torch.empty((N, 2), dtype=torch.float32, device=dev)
-        if N:
-            f4 = torch.empty((N, 128, E), dtype=torch.float32, device=dev)
-            f6 = torch.empty((N, 128, E), dtype=torch.float32, device=dev)
-            ws = _alloc_bytes(L.dcd_gmw_workspace_bytes(N, n, self.depth, 0), dev)
-            check(L.dcd_gmw_weights_fwd(ptr(k2), ptr(k3), ptr(p4), ptr(p6), N, n, self.depth, 0,
-                                        ptr(reg_w), ptr(f4), ptr(f6), ptr(ws), ws.numel() * 4, stream_ptr()), "dcd_gmw_weights_fwd")
-            del ws
-            tws = _alloc_bytes(L.dcd_gmw_transport_workspace_bytes(N, n), dev)
-            check(L.dcd_gmw_transport_fwd(ptr(f4), ptr(f6), N, n, self.SINKHORN_LAMBDA, self.SINKHORN_TOLERANCE,
-                                          self.SINKHORN_ITERATIONS, ptr(P) if P is not None else 0, 0, 0, ptr(sums),
-                                          ptr(tws), tws.numel() * 4, stream_ptr()), "dcd_gmw_transport_fwd")
-        return reg_w, P, sums
+        k2, k3, _ = self._prepare(kpts_2d, kpts_3d, p4, p6)
+        return _gmw_forward(k2, k3, p4, p6, self.depth, False, materialise, True, self.SINKHORN_LAMBDA,
+                            self.SINKHORN_TOLERANCE, self.SINKHORN_ITERATIONS)[:3]
 
     def transport_terms(self, kpts_2d, kpts_3d, params=None):
         """Differentiable correspondence branch without the plan: (reg_weights [b,E], terms [b,2] = (sum P, trace P)).
@@ -720,9 +647,7 @@ class GMW(nn.Module):
         so the E x E tensors of edge_P, of the loss and of dL/dP are never formed: K (4 E^2 bytes per object) is the only one
         kept for the backward.  Under torch.no_grad() this is edge_transport(materialise=False) without the plan."""
         p4, p6 = params if params is not None else (self.params4, self.params6)
-        k2, k3, need_grad = self._prepare(kpts_2d, kpts_3d, p4, p6)
-        return _GmwTransportTerms.apply(k2, k3, p4, p6, self.depth, need_grad, self.SINKHORN_LAMBDA, self.SINKHORN_TOLERANCE,
-                                        self.SINKHORN_ITERATIONS)
+        return self._edge_branch("terms", kpts_2d, kpts_3d, p4, p6)
 
     def forward(self, kpts_2d, kpts_3d, pred_rot=None, args=None):
         return self.forward_blobs(kpts_2d, kpts_3d, self.params4, self.params6)
@@ -741,15 +666,12 @@ class GMW(nn.Module):
     def forward_blobs(self, kpts_2d, kpts_3d, params4, params6):
         """forward() on explicit parameter blobs (dcd_b200.patch passes blobs packed from the LIVE reference parameters,
         so that their optimizer, checkpoints and DDP hooks keep working unchanged)."""
+        return self._edge_branch("plan" if self.with_edge_P else None, kpts_2d, kpts_3d, params4, params6)
+
+    def _edge_branch(self, branch, kpts_2d, kpts_3d, params4, params6):
         k2, k3, need_grad = self._prepare(kpts_2d, kpts_3d, params4, params6)
-        if self.with_edge_P:
-            return _GmwWeightsTransport.apply(k2, k3, params4, params6, self.depth, need_grad, self.SINKHORN_LAMBDA,
-                                              self.SINKHORN_TOLERANCE, self.SINKHORN_ITERATIONS)
-        reg_w = _GmwWeights.apply(k2, k3, params4, params6, self.depth, need_grad)
-        if _CHECK_FINITE and not bool(torch.isfinite(reg_w).all()):
-            # the tensor-core path carries activations as FP16 hi+lo pairs: |activation| must stay below 65504
-            raise FloatingPointError("dcd_b200.GMW: non-finite edge weights (activation outside the FP16 hi/lo range?)")
-        return reg_w, None
+        return _GmwEdgeBranch.apply(k2, k3, params4, params6, self.depth, need_grad, branch, self.SINKHORN_LAMBDA,
+                                    self.SINKHORN_TOLERANCE, self.SINKHORN_ITERATIONS)
 
 
 def compute_reg_loss(pre_depths, edge_weight, gt_depth, good_idx=None, validate: bool = False):

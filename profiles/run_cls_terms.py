@@ -4,10 +4,10 @@
 One training step = compute_z -> GMW (depth 12) -> w_cls * correspondence loss + w_reg * reg loss -> backward, on two paths:
     dense  GMW.forward with with_edge_P = True, correspondenceLoss((1 - 2 eye) * P) as the reference writes it
     terms  GMW.transport_terms + dcd_b200.correspondence_loss (no E x E tensor but K)
-each eager and replayed from a CUDA graph (GraphedGmwStep(plan_free=False / True)), for
+each eager, and the terms step also replayed from a CUDA graph (GraphedGmwStep), for
     cls        w_cls = 1.0, w_reg = 0.0 (GMW's first 50 epochs, GMW/main.py:313-315)
     cls+reg    w_cls = 0.1, w_reg = 1.0
-at n = 73 and b = 8, 64.  The four step kinds of a (b, weights) cell are alternated step by step in one process and timed
+at n = 73 and b = 8, 64.  The three step kinds of a (b, weights) cell are alternated step by step in one process and timed
 with CUDA events around each whole step (it ends in a device synchronise), after warm-up steps of every kind.
 Peak memory: torch.cuda.max_memory_allocated of one eager step above what was allocated before it, after empty_cache and
 reset_peak_memory_stats.  n = 256, b = 1: one cls step of each path (time and peak); the batch each path's measured
@@ -93,16 +93,12 @@ def main():
         for wname, (w_cls, w_reg) in WEIGHTS.items():
             peaks = {path: peak_bytes(lambda: eager_step(model, data, w_cls, w_reg, path == "terms"))
                      for path in ("dense", "terms")}
-            graphs = {}
-            for path in ("dense", "terms"):
-                gm = dcd_b200.GMW(depth=12).cuda().load_reference_state_dict(sd)
-                graphs[path] = dcd_b200.GraphedGmwStep(gm, batch=b, n=73, cls_weight=w_cls, reg_weight=w_reg,
-                                                       plan_free=path == "terms")
+            graph = dcd_b200.GraphedGmwStep(dcd_b200.GMW(depth=12).cuda().load_reference_state_dict(sd), batch=b, n=73,
+                                            cls_weight=w_cls, reg_weight=w_reg)
             kinds = {
                 "dense_eager": lambda: eager_step(model, data, w_cls, w_reg, False),
                 "terms_eager": lambda: eager_step(model, data, w_cls, w_reg, True),
-                "dense_graph": lambda: graphs["dense"](*data),
-                "terms_graph": lambda: graphs["terms"](*data),
+                "terms_graph": lambda: graph(*data),
             }
             for _ in range(args.warmup):
                 for fn in kinds.values():
@@ -113,15 +109,14 @@ def main():
                     times[k].append(timed(fn))
             cell = {"b": b, "loss": wname, "w_cls": w_cls, "w_reg": w_reg, "ms": {k: stats(t) for k, t in times.items()},
                     "peak_bytes": peaks}
-            for mode in ("eager", "graph"):
-                cell["ms"]["saved_%s_ms" % mode] = cell["ms"]["dense_" + mode]["median"] - cell["ms"]["terms_" + mode]["median"]
+            cell["ms"]["saved_eager_ms"] = cell["ms"]["dense_eager"]["median"] - cell["ms"]["terms_eager"]["median"]
             cell["peak_saved_bytes"] = peaks["dense"] - peaks["terms"]
             cell["peak_saved_in_bEE_tensors"] = cell["peak_saved_bytes"] / (b * 4 * 2628 * 2628)
             result["cells"].append(cell)
             print("n=73 b=%2d %-7s " % (b, wname) + "  ".join("%s %.3f ms" % (k, cell["ms"][k]["median"]) for k in kinds)
                   + "  peak dense %.0f MB terms %.0f MB (%.2f [b,E,E] tensors less)"
                   % (peaks["dense"] / 1e6, peaks["terms"] / 1e6, cell["peak_saved_in_bEE_tensors"]), flush=True)
-            del graphs, kinds
+            del graph, kinds
     # n = 256, b = 1, cls only: one step of each path (after one warm-up step each), time and peak
     ob = synth.make_objects(N=1, n=256, seed=12)
     data = (ob.kps_norm.cuda(), ob.kps_3d.cuda(), ob.rot_y.cuda().reshape(-1, 1), ob.gt_depth.cuda())

@@ -658,10 +658,12 @@ def test_large_magnitude_weights_stay_in_the_fp16_split_range(monkeypatch):
 
 def test_cuda_graph_training_step_equals_eager():
     """The whole training step (compute_z, forward with saved activations, losses, backward) captured in a CUDA graph:
-    replays on new inputs give the eager step's loss and gradients bit for bit (every kernel is deterministic)."""
+    replays on new inputs give the eager step's loss and gradients bit for bit (every kernel is deterministic).  The step
+    does not depend on the model's with_edge_P and leaves it as it was."""
     depth, b = 3, 4
     sd = O.random_state_dict(31, depth=depth)
     model = make_model(sd, depth)
+    model.with_edge_P = True
     eager = make_model(sd, depth)
     step = dcd_b200.GraphedGmwStep(model, batch=b, n=73)
     for seed in (1, 2, 3):
@@ -675,3 +677,4 @@ def test_cuda_graph_training_step_equals_eager():
         loss_e.backward()
         assert torch.equal(loss_g, loss_e.detach())
         assert torch.equal(model.params4.grad, eager.params4.grad) and torch.equal(model.params6.grad, eager.params6.grad)
+    assert model.with_edge_P

@@ -195,14 +195,15 @@ def test_transport_terms_keypoint_gradients_vs_fp64_unrolled_sinkhorn():
         assert ok, (key, e_o, e_r)
 
 
-def _partial_step(model, k2, k3, which, plan_free, R=None):
+def _partial_step(model, k2, k3, which, path, R):
+    """path: "terms" (GMW.transport_terms), "plan" (GMW.forward with with_edge_P) or "weights" (GMW.forward without it)."""
     model.zero_grad(set_to_none=True)
     a, b = _leaves(k2, k3)
-    if plan_free:
+    if path == "terms":
         w, terms = model.transport_terms(a, b)
         loss = {"trace": lambda: terms[:, 1].sum(), "sum": lambda: terms[:, 0].sum(), "reg": lambda: (w * R).sum()}[which]()
     else:
-        model.with_edge_P = which != "reg"
+        model.with_edge_P = path == "plan"
         try:
             w, P = model(a, b)
         finally:
@@ -215,25 +216,29 @@ def _partial_step(model, k2, k3, which, plan_free, R=None):
 @pytest.mark.parametrize("which", ["trace", "sum", "reg"])
 def test_partial_cotangents(which, monkeypatch):
     """A loss on trace P only (dL/dP = g I), on sum P only (g 11^T), or on reg_weights only: bit-identical to the dense path
-    (GMW.forward with with_edge_P, or without it for reg_weights).  The reg-only loss runs no transport backward."""
+    (GMW.forward with with_edge_P).  The reg-only loss runs no transport backward on either path, and equals GMW.forward
+    without with_edge_P bit for bit."""
     n, depth, N = 40, 2, 2
     model, k2, k3, _, _, _ = setup(n, depth, N, 2300)
     R = torch.randn(N, n * (n - 1) // 2, generator=torch.Generator().manual_seed(23)).to(DEV)
-    dense = _partial_step(model, k2, k3, which, False, R)
     L = _lib.lib()
-    calls = []
-    real = L.dcd_gmw_transport_terms_bwd
+    calls = {"dcd_gmw_transport_bwd": 0, "dcd_gmw_transport_terms_bwd": 0}
+    for name in calls:
+        def counted(*args, _name=name, _real=getattr(L, name)):
+            calls[_name] += 1
+            return _real(*args)
 
-    def counted(*args):
-        calls.append(1)
-        return real(*args)
-
-    monkeypatch.setattr(L, "dcd_gmw_transport_terms_bwd", counted)
-    terms = _partial_step(model, k2, k3, which, True, R)
-    assert len(calls) == (0 if which == "reg" else 1)
+        monkeypatch.setattr(L, name, counted)
+    expected = 0 if which == "reg" else 1
+    dense = _partial_step(model, k2, k3, which, "plan", R)
+    assert calls["dcd_gmw_transport_bwd"] == expected
+    terms = _partial_step(model, k2, k3, which, "terms", R)
+    assert calls["dcd_gmw_transport_terms_bwd"] == expected
+    others = [dense] + ([_partial_step(model, k2, k3, which, "weights", R)] if which == "reg" else [])
     for key in GRADS:
         assert float(terms[key].abs().max()) > 0, key
-        assert torch.equal(terms[key], dense[key]), key
+        for other in others:
+            assert torch.equal(terms[key], other[key]), key
 
 
 def test_frozen_parameters_and_frozen_keypoints():
@@ -284,42 +289,47 @@ def test_no_grad_empty_poisoned_and_rerun(monkeypatch):
 
 
 @pytest.mark.parametrize("w_cls,w_reg", [(1.0, 0.0), (0.1, 1.0)])
-def test_graphed_step_plan_free(w_cls, w_reg):
-    """GraphedGmwStep(plan_free=True): replayed gradients equal the eager terms step's and GraphedGmwStep(plan_free=False)'s
-    bit for bit; the loss matches to rel 1e-5."""
+def test_graphed_step_correspondence_loss(w_cls, w_reg):
+    """GraphedGmwStep with a correspondence loss: replayed gradients equal the eager terms step's and the eager dense step's
+    (edge_P + correspondenceLoss, GMW/main.py:456-457) bit for bit; the loss matches both to rel 1e-5."""
     n, depth, b = 73, 12, 8
     ob = synth.make_objects(N=b, n=n, seed=2600)
     model = make_model(O.random_state_dict(26, depth=depth), depth)
     k2, k3, rot, gt = cu(ob.kps_norm, ob.kps_3d, ob.rot_y, ob.gt_depth)
 
-    def eager_step():                                         # returns nothing that keeps its autograd graph alive
+    def eager_step(plan_free):                                # returns nothing that keeps its autograd graph alive
         model.zero_grad(set_to_none=True)
         Z, idx = dcd_b200.compute_z(k2, k3, rot)
-        w, terms = model.transport_terms(k2, k3)
+        if plan_free:
+            w, terms = model.transport_terms(k2, k3)
+            cls = dcd_b200.correspondence_loss(terms)
+        else:
+            model.with_edge_P = True
+            try:
+                w, P = model(k2, k3)
+            finally:
+                model.with_edge_P = False
+            cls = O.correspondence_loss(P, torch.eye(P.shape[1], device=DEV).expand_as(P))
         reg, _ = dcd_b200.compute_reg_loss(Z, w, gt, idx)
-        loss = w_reg * reg + w_cls * dcd_b200.correspondence_loss(terms)
+        loss = w_reg * reg + w_cls * cls
         loss.backward()
         return float(loss.detach()), (model.params4.grad.clone(), model.params6.grad.clone())
 
-    loss_eager, eager = eager_step()
+    loss_terms, terms = eager_step(True)
+    loss_dense, dense = eager_step(False)
     model.zero_grad(set_to_none=True)
-
-    def graphed(plan_free):
-        step = dcd_b200.GraphedGmwStep(model, batch=b, n=n, cls_weight=w_cls, reg_weight=w_reg, plan_free=plan_free)
-        step(k2, k3, rot, gt)
-        loss = float(step(k2, k3, rot, gt))                 # a second replay: nothing accumulates
-        torch.cuda.synchronize()
-        return loss, (model.params4.grad.clone(), model.params6.grad.clone())
-
-    loss_dense, dense = graphed(False)
-    loss_free, free = graphed(True)
-    print("graphed step, cls %g reg %g: loss plan-free %.7g, dense %.7g, eager %.7g"
-          % (w_cls, w_reg, loss_free, loss_dense, loss_eager))
-    for x, y, z in zip(free, eager, dense):
+    step = dcd_b200.GraphedGmwStep(model, batch=b, n=n, cls_weight=w_cls, reg_weight=w_reg)
+    step(k2, k3, rot, gt)
+    loss_graph = float(step(k2, k3, rot, gt))                 # a second replay: nothing accumulates
+    torch.cuda.synchronize()
+    graph = (model.params4.grad.clone(), model.params6.grad.clone())
+    print("graphed step, cls %g reg %g: loss graphed %.7g, eager terms %.7g, eager dense %.7g"
+          % (w_cls, w_reg, loss_graph, loss_terms, loss_dense))
+    for x, y, z in zip(graph, terms, dense):
         assert float(x.abs().max()) > 0
         assert torch.equal(x, y) and torch.equal(x, z)
-    assert abs(loss_free - loss_dense) <= 1e-5 * abs(loss_dense)
-    assert abs(loss_free - loss_eager) <= 1e-5 * abs(loss_eager)
+    assert abs(loss_graph - loss_dense) <= 1e-5 * abs(loss_dense)
+    assert abs(loss_graph - loss_terms) <= 1e-5 * abs(loss_terms)
 
 
 def _peak_bytes(fn):
