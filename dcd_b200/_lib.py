@@ -29,6 +29,9 @@ SIGNATURES = {
                            + [c_void_p] * 5),
     "dcd_dgde_depth_ensemble_fwd": (c_int, [c_void_p] * 7 + [c_int64, c_float, c_float, c_float, c_float] + [c_void_p] * 6),
     "dcd_poi_gather_fwd": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int, c_int64, c_void_p, c_void_p]),
+    "dcd_poi_gather_bwd": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int, c_int64, c_void_p, c_void_p]),
+    "dcd_dgde_locate_bwd": (c_int, [c_void_p] * 6 + [c_int64, c_float] + [c_void_p] * 4),
+    "dcd_dgde_depth_ensemble_bwd": (c_int, [c_void_p] * 7 + [c_int64, c_float, c_float, c_float, c_float] + [c_void_p] * 11),
     "dcd_gmw_ray_rescale_fwd": (c_int, [c_void_p] * 3 + [c_int64, c_void_p, c_void_p]),
     "dcd_gmw_param_count": (c_size_t, [c_int, c_int]),
     "dcd_gmw_workspace_bytes": (c_size_t, [c_int64, c_int, c_int, c_int]),

@@ -23,6 +23,12 @@ int launch_dgde_depth_ensemble(const float*, const float*, const float*, const f
                                int64_t, float, float, float, float, float*, float*, float*, int64_t*, float*, cudaStream_t);
 int launch_gmw_ray_rescale(const float*, const float*, const float*, int64_t, float*, cudaStream_t);
 int launch_poi_gather(const float*, const int64_t*, int64_t, int64_t, int, int64_t, float*, cudaStream_t);
+int launch_poi_gather_bwd(const float*, const int64_t*, int64_t, int64_t, int, int64_t, float*, cudaStream_t);
+int launch_dgde_locate_bwd(const float*, const float*, const float*, const float*, const float*, const float*, int64_t, float, float*,
+                           float*, float*, cudaStream_t);
+int launch_dgde_depth_ensemble_bwd(const float*, const float*, const float*, const float*, const float*, const float*, const float*,
+                                   int64_t, float, float, float, float, const float*, const float*, const float*, const float*, float*,
+                                   float*, float*, float*, float*, float*, cudaStream_t);
 size_t gmw_transport_workspace_bytes(int64_t N, int E);
 int launch_gmw_transport_fwd(const float*, const float*, int64_t, int, float, float, int, float*, float*, float*, float*, void*,
                              cudaStream_t);
@@ -151,6 +157,46 @@ int dcd_poi_gather_fwd(const float* feature_maps, const int64_t* index, int64_t 
     if (B == 0 || K == 0) return DCD_OK;
     if (!feature_maps || !index || !out) return DCD_E_INVALID;
     return launch_poi_gather(feature_maps, index, B, K, C, HW, out, (cudaStream_t)stream);
+}
+
+int dcd_poi_gather_bwd(const float* grad_out, const int64_t* index, int64_t B, int64_t K, int C, int64_t HW, float* grad_maps,
+                       void* stream) {
+    if (B < 0 || K < 0 || C < 1 || HW < 1) return DCD_E_INVALID;
+    if (K > DCD_POI_BWD_MAX_K) return DCD_E_UNSUPPORTED;
+    if (B == 0) return DCD_OK;
+    if (!grad_maps || (K > 0 && (!grad_out || !index))) return DCD_E_INVALID;
+    return launch_poi_gather_bwd(grad_out, index, B, K, C, HW, grad_maps, (cudaStream_t)stream);
+}
+
+int dcd_dgde_locate_bwd(const float* K, const float* points, const float* offsets, const float* pad, const float* depth,
+                        const float* grad_loc, int64_t N, float down_ratio, float* grad_offsets, float* grad_points,
+                        float* grad_depth, void* stream) {
+    if (N < 0) return DCD_E_INVALID;
+    if (N == 0) return DCD_OK;
+    if (!K || !points || !offsets || !pad || !depth || !grad_loc) return DCD_E_INVALID;
+    if (!grad_offsets && !grad_points && !grad_depth) return DCD_E_INVALID;
+    return launch_dgde_locate_bwd(K, points, offsets, pad, depth, grad_loc, N, down_ratio, grad_offsets, grad_points, grad_depth,
+                                  (cudaStream_t)stream);
+}
+
+int dcd_dgde_depth_ensemble_bwd(const float* kp10, const float* dims, const float* K, const float* direct,
+                                const float* log_unc_direct, const float* log_unc_kp, const float* scores, int64_t N,
+                                float down_ratio, float eps, float lo, float hi, const float* grad_kp_depths,
+                                const float* grad_depth, const float* grad_depth_error, const float* grad_scores_out,
+                                float* grad_kp10, float* grad_dims, float* grad_direct, float* grad_log_unc_direct,
+                                float* grad_log_unc_kp, float* grad_scores, void* stream) {
+    if (N < 0) return DCD_E_INVALID;
+    if (N == 0) return DCD_OK;
+    if (!kp10 || !dims || !K) return DCD_E_INVALID;
+    const bool ensemble = grad_depth || grad_depth_error || grad_scores_out;
+    if (!ensemble && !grad_kp_depths) return DCD_E_INVALID;
+    if (!grad_kp10 && !grad_dims && !grad_direct && !grad_log_unc_direct && !grad_log_unc_kp && !grad_scores) return DCD_E_INVALID;
+    if (ensemble && (!log_unc_kp || (direct && !log_unc_direct))) return DCD_E_INVALID;
+    if (grad_scores_out && !scores) return DCD_E_INVALID;
+    if ((grad_direct || grad_log_unc_direct) && !direct) return DCD_E_INVALID;
+    return launch_dgde_depth_ensemble_bwd(kp10, dims, K, direct, log_unc_direct, log_unc_kp, scores, N, down_ratio, eps, lo, hi,
+                                          grad_kp_depths, grad_depth, grad_depth_error, grad_scores_out, grad_kp10, grad_dims,
+                                          grad_direct, grad_log_unc_direct, grad_log_unc_kp, grad_scores, (cudaStream_t)stream);
 }
 
 int dcd_gmw_ray_rescale_fwd(const float* raw_location, const float* pred_depth, const float* dim, int64_t N,

@@ -194,6 +194,45 @@ int launch_dgde_frame(const float* fmap, const int64_t* index, const int32_t* ba
     return DCD_OK;
 }
 
+namespace {
+
+// Backward of the no-solve form of dgde_locate_warp_kernel (decode_location_flatten, anno_encoder.py:147-161), one thread per
+// object, in the order torch's autograd forms it for x = ((u - c_u) * d) / f_u + b_x, u = (p + o) * down_ratio - pad:
+//   d/du: (g_x / f_u) * d,  d/d(p + o) = that * down_ratio,  d/dd: (g_x / f_u) * (u - c_u) + (y likewise) + g_z.
+__global__ void __launch_bounds__(256)
+dgde_locate_bwd_kernel(const float* __restrict__ K, const float* __restrict__ points, const float* __restrict__ offsets,
+                       const float* __restrict__ pad, const float* __restrict__ depth, const float* __restrict__ grad_loc, int64_t N,
+                       float down_ratio, float* __restrict__ grad_offsets, float* __restrict__ grad_points,
+                       float* __restrict__ grad_depth) {
+    const int64_t o = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (o >= N) return;
+    const float* Ko = K + o * 12;
+    const float f_u = __ldg(Ko + 0), c_u = __ldg(Ko + 2), f_v = __ldg(Ko + 5), c_v = __ldg(Ko + 6);
+    const float d = __ldg(depth + o);
+    const float gx = __ldg(grad_loc + o * 3), gy = __ldg(grad_loc + o * 3 + 1), gz = __ldg(grad_loc + o * 3 + 2);
+    const float ax = __fdiv_rn(gx, f_u), ay = __fdiv_rn(gy, f_v);
+    const float g_u = __fmul_rn(__fmul_rn(ax, d), down_ratio), g_v = __fmul_rn(__fmul_rn(ay, d), down_ratio);
+    if (grad_offsets != nullptr) { grad_offsets[o * 2] = g_u; grad_offsets[o * 2 + 1] = g_v; }
+    if (grad_points != nullptr) { grad_points[o * 2] = g_u; grad_points[o * 2 + 1] = g_v; }
+    if (grad_depth != nullptr) {
+        const float u = __fsub_rn(__fmul_rn(__fadd_rn(__ldg(points + o * 2), __ldg(offsets + o * 2)), down_ratio), __ldg(pad + o * 2));
+        const float v = __fsub_rn(__fmul_rn(__fadd_rn(__ldg(points + o * 2 + 1), __ldg(offsets + o * 2 + 1)), down_ratio),
+                                  __ldg(pad + o * 2 + 1));
+        grad_depth[o] = __fadd_rn(__fadd_rn(__fmul_rn(ax, __fsub_rn(u, c_u)), __fmul_rn(ay, __fsub_rn(v, c_v))), gz);
+    }
+}
+
+}  // namespace
+
+int launch_dgde_locate_bwd(const float* K, const float* points, const float* offsets, const float* pad, const float* depth,
+                           const float* grad_loc, int64_t N, float down_ratio, float* grad_offsets, float* grad_points,
+                           float* grad_depth, cudaStream_t st) {
+    dgde_locate_bwd_kernel<<<(unsigned)((N + 255) / 256), 256, 0, st>>>(K, points, offsets, pad, depth, grad_loc, N, down_ratio,
+                                                                         grad_offsets, grad_points, grad_depth);
+    DCD_CHECK_LAUNCH();
+    return DCD_OK;
+}
+
 int launch_dgde_locate(const float* kpts_off, const float* kps3d, const float* rot, const float* K, const float* points,
                        const float* offsets, const float* pad, const float* dims, const float* depth_in, int64_t N, int n,
                        float lo, float hi, int flags, float down_ratio, float* depth_out, float* loc_out, cudaStream_t st) {
@@ -284,6 +323,171 @@ dgde_depth_ensemble_kernel(const float* __restrict__ kp10, const float* __restri
     }
 }
 
+// Backward of dgde_depth_ensemble_kernel: the forward is recomputed in its own operation order, then every backward formula is
+// torch's for the reference's op (div: g / b and -g * ((a / b) / b); 1 / u = reciprocal: -g * (r * r); exp: g * e; mean of two:
+// g / 2; relu: g where height > 0; clamp: g where lo <= x <= hi), with a term skipped (not multiplied by 0) when its upstream
+// gradient is absent, so that infinities and NaNs reach the same gradients as in the reference's autograd.  The NaN -> 0 of
+// the scores (detector_infer.py:202) zeroes their upstream gradient there.  One thread per object: nothing crosses objects.
+__global__ void __launch_bounds__(256)
+dgde_depth_ensemble_bwd_kernel(const float* __restrict__ kp10, const float* __restrict__ dims, const float* __restrict__ K,
+                               const float* __restrict__ direct, const float* __restrict__ log_unc_direct,
+                               const float* __restrict__ log_unc_kp, const float* __restrict__ scores, int64_t N, float down_ratio,
+                               float eps, float lo, float hi, const float* __restrict__ g_kp_depths, const float* __restrict__ g_depth,
+                               const float* __restrict__ g_depth_error, const float* __restrict__ g_scores_out,
+                               float* __restrict__ grad_kp10, float* __restrict__ grad_dims, float* __restrict__ grad_direct,
+                               float* __restrict__ grad_lud, float* __restrict__ grad_luk, float* __restrict__ grad_scores) {
+    const int64_t o = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (o >= N) return;
+    const float* kp = kp10 + o * 20;
+    float v[10];
+#pragma unroll
+    for (int t = 0; t < 10; ++t) v[t] = __ldg(kp + 2 * t + 1);
+    const float f_u = __ldg(K + o * 12);
+    const float fh = __fmul_rn(f_u, __ldg(dims + o * 3 + 1));
+    // heights in the forward's order: centre (8, 9), corner_02 (0, 4), (2, 6), corner_13 (1, 5), (3, 7)
+    constexpr int PA[5] = {8, 0, 2, 1, 3}, PB[5] = {9, 4, 6, 5, 7};
+    float ht[5], q[5];
+#pragma unroll
+    for (int e = 0; e < 5; ++e) {
+        ht[e] = __fsub_rn(v[PA[e]], v[PB[e]]);
+        q[e] = height_depth(fh, ht[e], down_ratio, eps);
+    }
+    float draw[4], d[4];
+    draw[1] = q[0];
+    draw[2] = __fmul_rn(__fadd_rn(q[1], q[2]), 0.5f);
+    draw[3] = __fmul_rn(__fadd_rn(q[3], q[4]), 0.5f);
+#pragma unroll
+    for (int j = 1; j < 4; ++j) d[j] = fminf(fmaxf(draw[j], lo), hi);
+
+    // gradients of the keypoint depths (after the clamp); has[j]: some upstream gradient reached d[j]
+    float gd[4] = {0.f, 0.f, 0.f, 0.f};
+    bool has[4] = {false, false, false, false};
+    if (g_kp_depths != nullptr) {
+#pragma unroll
+        for (int j = 1; j < 4; ++j) { gd[j] = __ldg(g_kp_depths + o * 3 + j - 1); has[j] = true; }
+    }
+    const bool want_depth = g_depth != nullptr;
+    const bool want_err = g_depth_error != nullptr || g_scores_out != nullptr;
+    float g_sc = 0.f;
+    if (want_depth || want_err) {
+        const int first = direct != nullptr ? 0 : 1;
+        float u[4], r[4], wn[4];
+        if (first == 0) {
+            d[0] = __ldg(direct + o);
+            u[0] = expf(__ldg(log_unc_direct + o));
+        }
+#pragma unroll
+        for (int j = 1; j < 4; ++j) u[j] = expf(__ldg(log_unc_kp + o * 3 + j - 1));
+        float S = 0.f;
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            if (j < first) continue;
+            r[j] = __fdiv_rn(1.f, u[j]);
+            S = __fadd_rn(S, r[j]);
+        }
+        float esum = 0.f;
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            if (j < first) continue;
+            wn[j] = __fdiv_rn(r[j], S);
+            esum = __fadd_rn(esum, __fmul_rn(wn[j], u[j]));
+        }
+        // depth_error's gradient: its own, plus the score path  out = scores * (1 - clamp(err, 0.01, 1)); out[isnan(out)] = 0
+        float ge = g_depth_error != nullptr ? __ldg(g_depth_error + o) : 0.f;
+        if (g_scores_out != nullptr) {
+            const float qnan = __int_as_float(0x7fc00000);
+            const float cl = esum != esum ? qnan : fminf(fmaxf(esum, 0.01f), 1.f);    // torch.clamp keeps NaN
+            const float conf = __fsub_rn(1.f, cl);
+            const float sc = __ldg(scores + o);
+            const float s = __fmul_rn(sc, conf);
+            const float go = s != s ? 0.f : __ldg(g_scores_out + o);
+            g_sc = __fmul_rn(go, conf);
+            const float gconf = __fmul_rn(go, sc);
+            const float gcl = (esum >= 0.01f && esum <= 1.f) ? -gconf : 0.f;
+            ge = g_depth_error != nullptr ? __fadd_rn(ge, gcl) : gcl;
+        }
+        const float gdep = want_depth ? __ldg(g_depth + o) : 0.f;
+        // depth = sum(d * wn), err = sum(wn * u), wn = r / S, r = 1 / u, u = exp(l)
+        float gwn[4], gu[4], gS = 0.f;
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            if (j < first) continue;
+            if (want_depth && want_err) gwn[j] = __fadd_rn(__fmul_rn(gdep, d[j]), __fmul_rn(ge, u[j]));
+            else gwn[j] = want_depth ? __fmul_rn(gdep, d[j]) : __fmul_rn(ge, u[j]);
+            gS = __fsub_rn(gS, __fmul_rn(gwn[j], __fdiv_rn(__fdiv_rn(r[j], S), S)));
+        }
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            if (j < first) continue;
+            const float gr = __fadd_rn(__fdiv_rn(gwn[j], S), gS);
+            const float grec = __fmul_rn(-gr, __fmul_rn(r[j], r[j]));
+            gu[j] = want_err ? __fadd_rn(__fmul_rn(ge, wn[j]), grec) : grec;
+            if (want_depth) {
+                const float g = __fmul_rn(gdep, wn[j]);
+                gd[j] = has[j] ? __fadd_rn(gd[j], g) : g;
+                has[j] = true;
+            }
+        }
+        if (grad_direct != nullptr) grad_direct[o] = first == 0 && want_depth ? gd[0] : 0.f;
+        if (grad_lud != nullptr) grad_lud[o] = first == 0 ? __fmul_rn(gu[0], u[0]) : 0.f;
+        if (grad_luk != nullptr) {
+#pragma unroll
+            for (int j = 1; j < 4; ++j) grad_luk[o * 3 + j - 1] = __fmul_rn(gu[j], u[j]);
+        }
+    } else {
+        if (grad_direct != nullptr) grad_direct[o] = 0.f;
+        if (grad_lud != nullptr) grad_lud[o] = 0.f;
+        if (grad_luk != nullptr) grad_luk[o * 3] = grad_luk[o * 3 + 1] = grad_luk[o * 3 + 2] = 0.f;
+    }
+    if (grad_scores != nullptr) grad_scores[o] = g_sc;
+
+    // back through the clamps, the means of two, the divisions and the relus
+    float gq[5] = {0.f, 0.f, 0.f, 0.f, 0.f};
+    bool hq[5] = {false, false, false, false, false};
+#pragma unroll
+    for (int j = 1; j < 4; ++j) {
+        if (!has[j]) continue;
+        const float g = (draw[j] >= lo && draw[j] <= hi) ? gd[j] : 0.f;
+        if (j == 1) { gq[0] = g; hq[0] = true; }
+        else {
+            const float gh = __fdiv_rn(g, 2.f);
+            gq[2 * j - 3] = gh; gq[2 * j - 2] = gh; hq[2 * j - 3] = hq[2 * j - 2] = true;
+        }
+    }
+    float gfh[3] = {0.f, 0.f, 0.f}, gv[10];
+#pragma unroll
+    for (int t = 0; t < 10; ++t) gv[t] = 0.f;
+#pragma unroll
+    for (int e = 0; e < 5; ++e) {
+        if (!hq[e]) continue;
+        const float den = __fadd_rn(__fmul_rn(fmaxf(ht[e], 0.f), down_ratio), eps);
+        const float gf = __fdiv_rn(gq[e], den);
+        const int grp = e == 0 ? 0 : (e + 1) / 2;
+        gfh[grp] = __fadd_rn(gfh[grp], gf);
+        const float gden = __fmul_rn(-gq[e], __fdiv_rn(q[e], den));
+        const float gh = ht[e] > 0.f ? __fmul_rn(gden, down_ratio) : 0.f;
+        gv[PA[e]] = gh;
+        gv[PB[e]] = -gh;
+    }
+    if (grad_kp10 != nullptr) {
+        float* gk = grad_kp10 + o * 20;
+#pragma unroll
+        for (int t = 0; t < 10; ++t) { gk[2 * t] = 0.f; gk[2 * t + 1] = gv[t]; }
+    }
+    if (grad_dims != nullptr) {
+        float gh = 0.f;
+        bool any = false;
+#pragma unroll
+        for (int grp = 0; grp < 3; ++grp) {
+            if (!hq[grp == 0 ? 0 : 2 * grp - 1]) continue;
+            const float t = __fmul_rn(gfh[grp], f_u);
+            gh = any ? __fadd_rn(gh, t) : t;
+            any = true;
+        }
+        grad_dims[o * 3] = 0.f; grad_dims[o * 3 + 1] = gh; grad_dims[o * 3 + 2] = 0.f;
+    }
+}
+
 // GMW/main.py:542-547
 __global__ void __launch_bounds__(256)
 gmw_ray_rescale_kernel(const float* __restrict__ raw_location, const float* __restrict__ pred_depth, const float* __restrict__ dim,
@@ -306,6 +510,18 @@ int launch_dgde_depth_ensemble(const float* kp10, const float* dims, const float
                                cudaStream_t st) {
     dgde_depth_ensemble_kernel<<<(unsigned)((N + 255) / 256), 256, 0, st>>>(kp10, dims, K, direct, lud, luk, scores, N, down_ratio, eps,
                                                                              lo, hi, kp_depths, depth, depth_error, argmax, scores_out);
+    DCD_CHECK_LAUNCH();
+    return DCD_OK;
+}
+
+int launch_dgde_depth_ensemble_bwd(const float* kp10, const float* dims, const float* K, const float* direct, const float* lud,
+                                   const float* luk, const float* scores, int64_t N, float down_ratio, float eps, float lo, float hi,
+                                   const float* g_kd, const float* g_depth, const float* g_err, const float* g_so, float* grad_kp10,
+                                   float* grad_dims, float* grad_direct, float* grad_lud, float* grad_luk, float* grad_scores,
+                                   cudaStream_t st) {
+    dgde_depth_ensemble_bwd_kernel<<<(unsigned)((N + 255) / 256), 256, 0, st>>>(
+        kp10, dims, K, direct, lud, luk, scores, N, down_ratio, eps, lo, hi, g_kd, g_depth, g_err, g_so, grad_kp10, grad_dims,
+        grad_direct, grad_lud, grad_luk, grad_scores);
     DCD_CHECK_LAUNCH();
     return DCD_OK;
 }
@@ -337,7 +553,80 @@ poi_gather_kernel(const float* __restrict__ feat, const int64_t* __restrict__ in
     out[t] = (p >= 0 && p < HW) ? __ldg(feat + (b * C + c) * HW + p) : __int_as_float(0x7fc00000);   // out of range: NaN, no fault
 }
 
+// Backward, pass 1: the dense [B,C,H,W] gradient is zero except at <= B*K positions per channel, so it is filled at full store
+// bandwidth (16-byte stores, grid-stride) and pass 2 overwrites the selected positions.
+__global__ void __launch_bounds__(256)
+poi_fill_zero_kernel(float* __restrict__ out, int64_t total, bool vec) {
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    int64_t done = 0;
+    if (vec) {
+        float4* o4 = reinterpret_cast<float4*>(out);
+        const int64_t n4 = total / 4;
+        for (int64_t i = t; i < n4; i += stride) o4[i] = make_float4(0.f, 0.f, 0.f, 0.f);
+        done = n4 * 4;
+    }
+    for (int64_t i = done + t; i < total; i += stride) out[i] = 0.f;
+}
+
+// Backward, pass 2: one CTA per target slot (b, k).  The slot writes its position only if no earlier slot of the image holds
+// the same position; it then sums, per channel, grad_out over every slot k' >= k with that position in ascending k', so each
+// selected element is written once, deterministically, without atomics.  The duplicate scan is O(K) per slot
+// (K <= DCD_POI_BWD_MAX_K).  An index outside [0, HW) drops its gradient (the forward gave NaN there).
+__global__ void __launch_bounds__(128)
+poi_scatter_kernel(const float* __restrict__ grad_out, const int64_t* __restrict__ index, int64_t B, int Kp, int C, int64_t HW,
+                   float* __restrict__ grad_maps) {
+    __shared__ int list[DCD_POI_BWD_MAX_K];
+    __shared__ int count;
+    const int tid = threadIdx.x, lane = tid & 31;
+    for (int64_t slot = blockIdx.x; slot < B * Kp; slot += gridDim.x) {
+        const int64_t b = slot / Kp;
+        const int k = (int)(slot - b * Kp);
+        const int64_t* ib = index + b * Kp;
+        const int64_t p = ib[k];
+        if (p < 0 || p >= HW) continue;                                   // uniform over the CTA
+        bool earlier = false;
+        for (int j = tid; j < k; j += blockDim.x) earlier |= ib[j] == p;
+        if (__syncthreads_or(earlier)) continue;
+        if (tid < 32) {                                                   // warp 0: ascending list of the slots >= k at p
+            int cnt = 0;
+            for (int base = k; base < Kp; base += 32) {
+                const int j = base + lane;
+                const bool m = j < Kp && ib[j] == p;
+                const unsigned bal = __ballot_sync(0xffffffffu, m);
+                if (m) list[cnt + __popc(bal & ((1u << lane) - 1u))] = j;
+                cnt += __popc(bal);
+            }
+            if (lane == 0) count = cnt;
+        }
+        __syncthreads();
+        const int cnt = count;
+        const float* gb = grad_out + b * (int64_t)Kp * C;
+        for (int c = tid; c < C; c += blockDim.x) {
+            float acc = 0.f;
+            for (int i = 0; i < cnt; ++i) acc += __ldg(gb + (int64_t)list[i] * C + c);
+            grad_maps[(b * C + c) * HW + p] = acc;
+        }
+        __syncthreads();                                                  // list / count are rebuilt for the next slot
+    }
+}
+
 }  // namespace
+
+int launch_poi_gather_bwd(const float* grad_out, const int64_t* index, int64_t B, int64_t Kp, int C, int64_t HW, float* grad_maps,
+                          cudaStream_t st) {
+    const int64_t total = B * C * HW;
+    const int64_t cap = (int64_t)device_sm_count() * 8;
+    int64_t want = (total / 4 + 255) / 256;
+    poi_fill_zero_kernel<<<(unsigned)(want < cap ? (want > 0 ? want : 1) : cap), 256, 0, st>>>(
+        grad_maps, total, (reinterpret_cast<uintptr_t>(grad_maps) & 15) == 0);
+    DCD_CHECK_LAUNCH();
+    if (Kp == 0) return DCD_OK;
+    want = B * Kp;
+    poi_scatter_kernel<<<(unsigned)(want < cap * 4 ? want : cap * 4), 128, 0, st>>>(grad_out, index, B, (int)Kp, C, HW, grad_maps);
+    DCD_CHECK_LAUNCH();
+    return DCD_OK;
+}
 
 int launch_poi_gather(const float* feat, const int64_t* index, int64_t B, int64_t Kp, int C, int64_t HW, float* out, cudaStream_t st) {
     const int64_t total = B * Kp * C;

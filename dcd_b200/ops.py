@@ -39,11 +39,19 @@ def _num_edges(n: int) -> int:
 
 
 def _inference_only(name: str, *tensors) -> None:
-    """The frame-epilogue ops (SURVEY 8f rows N2/N4) have no backward: fail loudly instead of silently cutting the
-    autograd graph when the reference would differentiate through them (detector_loss.py:391)."""
+    """The inference-form frame-epilogue ops (compute_pairs_kpts_depth, frame_depths_from_map, ray_rescale) have no
+    backward: fail loudly instead of silently cutting the autograd graph."""
     if torch.is_grad_enabled() and any(t is not None and torch.is_tensor(t) and t.requires_grad for t in tensors):
         raise RuntimeError("dcd_b200.%s is inference-only (no backward is implemented): call it under torch.no_grad() "
                            "or detach its inputs" % name)
+
+
+def _constant_inputs(name: str, **inputs) -> None:
+    """Inputs that are constants in the reference (calibration, padding) get no gradient: fail loudly instead of silently
+    cutting the graph when one requires grad."""
+    for arg, t in inputs.items():
+        if torch.is_grad_enabled() and torch.is_tensor(t) and t.requires_grad:
+            raise RuntimeError("dcd_b200.%s: `%s` receives no gradient (a constant in the reference): detach it" % (name, arg))
 
 
 def _check_shapes(kps, kps_3d, rot, K=None):
@@ -303,30 +311,88 @@ def frame_depths_from_map(pred_regression, indexs, pred_rots, P, pad_size, dims=
     return (depth, loc, kimg, k3) if return_keypoints else (depth, loc)
 
 
+class _LocateFlatten(torch.autograd.Function):
+    """decode_location_flatten through dcd_dgde_locate_fwd (no solve); backward dcd_dgde_locate_bwd -> points (when floating
+    and requiring grad), offsets, depths."""
+
+    @staticmethod
+    def forward(ctx, pts, ofs, dep, K, pad):
+        N = pts.shape[0]
+        loc = torch.empty((N, 3), dtype=torch.float32, device=pts.device)
+        if N:
+            check(_lib.lib().dcd_dgde_locate_fwd(0, 0, 0, ptr(K), ptr(pts), ptr(ofs), ptr(pad), 0, ptr(dep), N, 2, 0.0, 0.0, 0,
+                                                 DOWN_RATIO, 0, ptr(loc), stream_ptr()), "dcd_dgde_locate_fwd")
+        ctx.save_for_backward(pts, ofs, dep, K, pad)
+        ctx.set_materialize_grads(False)
+        return loc
+
+    @staticmethod
+    def backward(ctx, g_loc):
+        pts, ofs, dep, K, pad = ctx.saved_tensors
+        need = ctx.needs_input_grad
+        if g_loc is None:
+            return None, None, None, None, None
+        N = pts.shape[0]
+        g_pts = torch.empty_like(pts) if need[0] else None
+        g_ofs = torch.empty_like(ofs) if need[1] else None
+        g_dep = torch.empty_like(dep) if need[2] else None
+        if N and (need[0] or need[1] or need[2]):
+            check(_lib.lib().dcd_dgde_locate_bwd(ptr(K), ptr(pts), ptr(ofs), ptr(pad), ptr(dep), ptr(f32c(g_loc)), N, DOWN_RATIO,
+                                                 ptr(g_ofs), ptr(g_pts), ptr(g_dep), stream_ptr()), "dcd_dgde_locate_bwd")
+        return g_pts, g_ofs, g_dep, None, None
+
+
 def decode_location_flatten(points, offsets, depths, P, pad_size, batch_idxs=None):
     """Anno_Encoder.decode_location_flatten (DGDE/model/anno_encoder.py:147-161) with the calibration given as the
     3x4 matrix of the image ([3,4]) or per object ([N,3,4]) instead of Calibration objects -> locations [N,3].
-    Inference-only (no backward; raises when an input requires grad)."""
+    Differentiable w.r.t. offsets, depths and (floating) points; P and pad_size are constants (raise when they require
+    grad).  float64 inputs get float64 gradients (the arithmetic is FP32)."""
     require_cuda(points, offsets, depths)
-    _inference_only("decode_location_flatten", points, offsets, depths)
+    _constant_inputs("decode_location_flatten", P=P, pad_size=pad_size)
     pts, ofs, dep = f32c(points), f32c(offsets), f32c(depths).reshape(-1)
     N, dev = pts.shape[0], pts.device
     K = _calib_per_object(P, N, dev)
     pad = _pad_per_object(pad_size, batch_idxs, N, dev)
-    loc = torch.empty((N, 3), dtype=torch.float32, device=dev)
-    if N:
-        check(_lib.lib().dcd_dgde_locate_fwd(0, 0, 0, ptr(K), ptr(pts), ptr(ofs), ptr(pad), 0, ptr(dep), N, 2, 0.0, 0.0, 0,
-                                             DOWN_RATIO, 0, ptr(loc), stream_ptr()), "dcd_dgde_locate_fwd")
-    return loc
+    return _LocateFlatten.apply(pts, ofs, dep, K, pad)
+
+
+class _PoiGather(torch.autograd.Function):
+    """select_point_of_interest through dcd_poi_gather_fwd; backward dcd_poi_gather_bwd (dense map gradient, duplicates summed
+    in ascending slot order, no atomics)."""
+
+    @staticmethod
+    def forward(ctx, fm, idx):
+        B, C, H, W = fm.shape
+        out = torch.empty((B, idx.shape[1], C), dtype=torch.float32, device=fm.device)
+        if out.numel():
+            check(_lib.lib().dcd_poi_gather_fwd(ptr(fm), ptr(idx), B, idx.shape[1], C, H * W, ptr(out), stream_ptr()),
+                  "dcd_poi_gather_fwd")
+        ctx.save_for_backward(idx)
+        ctx.shape = (B, C, H, W)
+        ctx.set_materialize_grads(False)
+        return out
+
+    @staticmethod
+    def backward(ctx, g_out):
+        if g_out is None:
+            return None, None
+        (idx,) = ctx.saved_tensors
+        B, C, H, W = ctx.shape
+        g_map = torch.empty((B, C, H, W), dtype=torch.float32, device=idx.device)
+        g = f32c(g_out)
+        check(_lib.lib().dcd_poi_gather_bwd(ptr(g), ptr(idx), B, idx.shape[1], C, H * W, ptr(g_map), stream_ptr()),
+              "dcd_poi_gather_bwd")
+        return g_map, None
 
 
 def select_point_of_interest(batch, index, feature_maps, validate: bool = False):
     """Drop-in for DGDE/model/layers/utils.py:120-145: feature_maps [B,C,H,W], index [B,K] flattened positions (or
     [B,K,2] (x, y) points) -> [B,K,C], reading only the selected values (no NHWC copy of the map).  An index outside the
     map yields NaN; `validate=True` checks the range first (a host synchronisation) and raises like torch.gather.
-    Inference-only (no backward; raises when feature_maps requires grad)."""
+    Differentiable w.r.t. feature_maps: the [B,C,H,W] gradient is written densely by the library (no NHWC copy, no
+    scatter_add), positions selected by several slots receive the sum of their gradients in ascending slot order, an index
+    outside the map passes none; at most DCD_POI_BWD_MAX_K (1024) slots per image."""
     require_cuda(feature_maps, index)
-    _inference_only("select_point_of_interest", feature_maps)
     fm = f32c(feature_maps)
     B, C, H, W = fm.shape
     if index.dim() == 3:
@@ -334,43 +400,90 @@ def select_point_of_interest(batch, index, feature_maps, validate: bool = False)
     idx = index.reshape(batch, -1).long().contiguous()
     if validate and idx.numel() and (int(idx.min()) < 0 or int(idx.max()) >= H * W):
         raise RuntimeError("index out of range")
-    out = torch.empty((B, idx.shape[1], C), dtype=torch.float32, device=fm.device)
-    if out.numel():
-        check(_lib.lib().dcd_poi_gather_fwd(ptr(fm), ptr(idx), B, idx.shape[1], C, H * W, ptr(out), stream_ptr()),
-              "dcd_poi_gather_fwd")
-    return out
+    return _PoiGather.apply(fm, idx)
 
 
 DEPTH_RANGE = (0.1, 100.0)   # MODEL.HEAD.DEPTH_RANGE (DGDE/config/defaults.py:196)
 KP_DEPTH_EPS = 1e-3          # Anno_Encoder.EPS (anno_encoder.py:17)
 
 
+class _DepthEnsemble(torch.autograd.Function):
+    """dcd_dgde_depth_ensemble_fwd: keypoint depths only (`ensemble` False, decode_depth_from_keypoints_batch) or the whole
+    ensemble (depth_ensemble).  Backward dcd_dgde_depth_ensemble_bwd: one launch for every output's gradient; an output the
+    loss does not use passes none, so the keypoint-depth gradient alone is the same launch for both functions."""
+
+    @staticmethod
+    def forward(ctx, kp, dm, K, luk, dd, lud, sc, ensemble):
+        N, dev = kp.shape[0], kp.device
+        kd = torch.empty((N, 3), dtype=torch.float32, device=dev)
+        depth = err = amax = so = None
+        if ensemble:
+            depth = torch.empty((N,), dtype=torch.float32, device=dev)
+            err = torch.empty((N,), dtype=torch.float32, device=dev)
+            amax = torch.empty((N,), dtype=torch.int64, device=dev)
+            so = torch.empty((N,), dtype=torch.float32, device=dev) if sc is not None else None
+        if N:
+            check(_lib.lib().dcd_dgde_depth_ensemble_fwd(ptr(kp), ptr(dm), ptr(K), ptr(dd), ptr(lud), ptr(luk), ptr(sc), N,
+                                                         DOWN_RATIO, KP_DEPTH_EPS, DEPTH_RANGE[0], DEPTH_RANGE[1], ptr(kd),
+                                                         ptr(depth), ptr(err), ptr(amax), ptr(so), stream_ptr()),
+                  "dcd_dgde_depth_ensemble_fwd")
+        ctx.save_for_backward(kp, dm, K, luk, dd, lud, sc)
+        ctx.set_materialize_grads(False)
+        if not ensemble:
+            return kd
+        if amax is not None:
+            ctx.mark_non_differentiable(amax)
+        if so is None:
+            so = torch.empty((0,), dtype=torch.float32, device=dev)
+            ctx.mark_non_differentiable(so)
+        return kd, depth, err, amax, so
+
+    @staticmethod
+    def backward(ctx, g_kd, g_depth=None, g_err=None, _g_amax=None, g_so=None):
+        kp, dm, K, luk, dd, lud, sc = ctx.saved_tensors
+        need = ctx.needs_input_grad
+        N = kp.shape[0]
+        if sc is None:
+            g_so = None
+        g_up = [f32c(g).reshape(-1) if g is not None else None for g in (g_kd, g_depth, g_err, g_so)]
+        outs = [torch.empty_like(t) if t is not None and need[i] else None
+                for i, t in ((0, kp), (1, dm), (4, dd), (5, lud), (3, luk), (6, sc))]
+        if N and any(g is not None for g in g_up) and any(o is not None for o in outs):
+            check(_lib.lib().dcd_dgde_depth_ensemble_bwd(ptr(kp), ptr(dm), ptr(K), ptr(dd), ptr(lud), ptr(luk), ptr(sc), N,
+                                                         DOWN_RATIO, KP_DEPTH_EPS, DEPTH_RANGE[0], DEPTH_RANGE[1],
+                                                         *(ptr(g) for g in g_up), *(ptr(o) for o in outs), stream_ptr()),
+                  "dcd_dgde_depth_ensemble_bwd")
+        else:
+            outs = [o.zero_() if o is not None else None for o in outs]
+        g_kp, g_dm, g_dd, g_lud, g_luk, g_sc = outs
+        return g_kp, g_dm, None, g_luk, g_dd, g_lud, g_sc, None
+
+
 def decode_depth_from_keypoints_batch(pred_keypoints, pred_dimensions, P, batch_idxs=None):
     """Anno_Encoder.decode_depth_from_keypoints_batch (DGDE/model/anno_encoder.py:193-224) with the calibration as the
-    image's 3x4 matrix ([3,4]; [B,3,4] with batch_idxs; or per object [N,3,4]) -> [N,3] (centre, corner_02, corner_13)."""
+    image's 3x4 matrix ([3,4]; [B,3,4] with batch_idxs; or per object [N,3,4]) -> [N,3] (centre, corner_02, corner_13).
+    Differentiable w.r.t. pred_keypoints (v column; the u column's gradient is exactly 0) and pred_dimensions (h column);
+    P is a constant (raises when it requires grad)."""
     require_cuda(pred_keypoints, pred_dimensions)
-    _inference_only("decode_depth_from_keypoints_batch", pred_keypoints, pred_dimensions)
+    _constant_inputs("decode_depth_from_keypoints_batch", P=P)
     kp, dm = f32c(pred_keypoints).reshape(-1, 10, 2), f32c(pred_dimensions)
     N, dev = kp.shape[0], kp.device
     P = torch.as_tensor(P)
     if P.dim() == 3 and batch_idxs is not None and P.shape[0] != N:
         P = P.to(dev)[batch_idxs.to(dev).long()]
     K = _calib_per_object(P, N, dev)
-    out = torch.empty((N, 3), dtype=torch.float32, device=dev)
-    if N:
-        check(_lib.lib().dcd_dgde_depth_ensemble_fwd(ptr(kp), ptr(dm), ptr(K), 0, 0, 0, 0, N, DOWN_RATIO, KP_DEPTH_EPS,
-                                                     DEPTH_RANGE[0], DEPTH_RANGE[1], ptr(out), 0, 0, 0, 0, stream_ptr()),
-              "dcd_dgde_depth_ensemble_fwd")
-    return out
+    return _DepthEnsemble.apply(kp, dm, K, None, None, None, None, False)
 
 
 def depth_ensemble(pred_keypoints, pred_dimensions, P, keypoint_log_uncertainty, direct_depths=None,
                    direct_log_uncertainty=None, scores=None):
     """Fused detector_infer.py:141-171,197-203: keypoint depths, uncertainties = exp(channels), inverse-uncertainty soft
-    ensemble -> dict(keypoint_depths [N,3], depth [N], depth_error [N], min_uncertainty [N] int64, scores [N,1] or None)."""
+    ensemble -> dict(keypoint_depths [N,3], depth [N], depth_error [N], min_uncertainty [N] int64, scores [N,1] or None).
+    Differentiable (like the reference's autograd) w.r.t. pred_keypoints (v column), pred_dimensions (h column), the log
+    uncertainties, direct_depths and scores; min_uncertainty is not differentiable and P is a constant (raises when it
+    requires grad)."""
     require_cuda(pred_keypoints, pred_dimensions, keypoint_log_uncertainty)
-    _inference_only("depth_ensemble", pred_keypoints, pred_dimensions, keypoint_log_uncertainty, direct_depths,
-                    direct_log_uncertainty, scores)
+    _constant_inputs("depth_ensemble", P=P)
     kp, dm = f32c(pred_keypoints).reshape(-1, 10, 2), f32c(pred_dimensions)
     N, dev = kp.shape[0], kp.device
     K = _calib_per_object(P, N, dev)
@@ -380,20 +493,9 @@ def depth_ensemble(pred_keypoints, pred_dimensions, P, keypoint_log_uncertainty,
     if (dd is None) != (lud is None):
         raise RuntimeError("direct depth and its uncertainty channel go together")
     sc = f32c(scores).reshape(-1) if scores is not None else None
-    kd = torch.empty((N, 3), dtype=torch.float32, device=dev)
-    depth = torch.empty((N,), dtype=torch.float32, device=dev)
-    err = torch.empty((N,), dtype=torch.float32, device=dev)
-    amax = torch.empty((N,), dtype=torch.int64, device=dev)
-    so = torch.empty((N,), dtype=torch.float32, device=dev) if sc is not None else None
-    if N:
-        check(_lib.lib().dcd_dgde_depth_ensemble_fwd(ptr(kp), ptr(dm), ptr(K), ptr(dd) if dd is not None else 0,
-                                                     ptr(lud) if lud is not None else 0, ptr(luk),
-                                                     ptr(sc) if sc is not None else 0, N, DOWN_RATIO, KP_DEPTH_EPS,
-                                                     DEPTH_RANGE[0], DEPTH_RANGE[1], ptr(kd), ptr(depth), ptr(err), ptr(amax),
-                                                     ptr(so) if so is not None else 0, stream_ptr()),
-              "dcd_dgde_depth_ensemble_fwd")
+    kd, depth, err, amax, so = _DepthEnsemble.apply(kp, dm, K, luk, dd, lud, sc, True)
     return {"keypoint_depths": kd, "depth": depth, "depth_error": err, "min_uncertainty": amax,
-            "scores": so.reshape(-1, 1) if so is not None else None}
+            "scores": so.reshape(-1, 1) if sc is not None else None}
 
 
 def ray_rescale(raw_location, pred_depth, dim):

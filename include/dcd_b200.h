@@ -129,6 +129,42 @@ int dcd_dgde_depth_ensemble_fwd(const float* kp10, const float* dims, const floa
 int dcd_poi_gather_fwd(const float* feature_maps, const int64_t* index, int64_t B, int64_t K, int C, int64_t HW,
                        float* out, void* stream);
 
+/* ------------------------------------------------------------------------------------------------
+ * Backward of the frame-epilogue functions around the edge solve (the autograd of the reference's DGDE loss,
+ * detector_loss.py:391).  Same conventions as the forwards: outputs OVERWRITTEN, N == 0 (B == 0) a no-op, deterministic, no
+ * atomics, arguments checked before any CUDA call.
+ *
+ * Backward of dcd_poi_gather_fwd.  grad_out [B,K,C] -> grad_maps [B,C,HW] (dense, every element written):
+ * grad_maps[b,c,p] = sum of grad_out[b,k,c] over the k with index[b,k] == p, summed in ascending k, +0.0 elsewhere.
+ * Duplicate positions (padded target slots) are the normal case.  An index outside [0, HW) drops its gradient.  Each slot
+ * scans the image's K indices for duplicates: K > DCD_POI_BWD_MAX_K returns DCD_E_UNSUPPORTED.  grad_out and index may be
+ * NULL when K == 0 (grad_maps is then filled with zeros). */
+#define DCD_POI_BWD_MAX_K 1024
+int dcd_poi_gather_bwd(const float* grad_out, const int64_t* index, int64_t B, int64_t K, int C, int64_t HW, float* grad_maps,
+                       void* stream);
+
+/* Backward of dcd_dgde_locate_fwd's no-solve form (decode_location_flatten, anno_encoder.py:147-161; kpts_off == NULL, dims
+ * == NULL): grad_loc [N,3] -> grad_offsets [N,2], grad_points [N,2] (the same values: both enter as points + offsets) and
+ * grad_depth [N].  K, points, offsets, pad, depth: the forward's inputs (depth = its depth_in).  Each output may be NULL, not
+ * all three.  No gradient flows to K or pad (the calibration and the padding are constants in the reference). */
+int dcd_dgde_locate_bwd(const float* K, const float* points, const float* offsets, const float* pad, const float* depth,
+                        const float* grad_loc, int64_t N, float down_ratio, float* grad_offsets, float* grad_points,
+                        float* grad_depth, void* stream);
+
+/* Backward of dcd_dgde_depth_ensemble_fwd, same inputs and scalars.  Upstream gradients grad_kp_depths [N,3], grad_depth [N],
+ * grad_depth_error [N], grad_scores_out [N]: each may be NULL (no gradient from that output), not all four; any of the last
+ * three needs log_unc_kp (and log_unc_direct when direct != NULL), grad_scores_out needs scores.  Outputs, each may be NULL,
+ * not all: grad_kp10 [N,10,2] (v column; the u column is exactly 0), grad_dims [N,3] (h column; l and w exactly 0),
+ * grad_direct [N], grad_log_unc_direct [N] (both need direct != NULL), grad_log_unc_kp [N,3], grad_scores [N].  argmax has no
+ * gradient, K none (calibration).  Masks as torch: relu passes where height > 0, clamps are inclusive; a NaN score product
+ * (zeroed by the forward) passes no gradient.  Height NaNs are outside the contract (the forward's relu maps them to 0). */
+int dcd_dgde_depth_ensemble_bwd(const float* kp10, const float* dims, const float* K, const float* direct,
+                                const float* log_unc_direct, const float* log_unc_kp, const float* scores, int64_t N,
+                                float down_ratio, float eps, float lo, float hi, const float* grad_kp_depths,
+                                const float* grad_depth, const float* grad_depth_error, const float* grad_scores_out,
+                                float* grad_kp10, float* grad_dims, float* grad_direct, float* grad_log_unc_direct,
+                                float* grad_log_unc_kp, float* grad_scores, void* stream);
+
 /* GMW validation (GMW/main.py:542-547): move a detector location [N,3] along its viewing ray through the box centre to
  * the GMW depth: scale = pred_depth / z; y -= h/2; loc *= scale; y += h/2  (dim [N,3] = (h,w,l) there). */
 int dcd_gmw_ray_rescale_fwd(const float* raw_location, const float* pred_depth, const float* dim, int64_t N,
