@@ -50,6 +50,9 @@ SIGNATURES = {
     "dcd_gmw_depth_workspace_bytes": (c_size_t, [c_int64, c_int, c_int, c_int64]),
     "dcd_gmw_depth_fwd": (c_int, [c_void_p] * 5 + [c_int64, c_int, c_int, c_int, c_float, c_float, c_int64]
                           + [c_void_p] * 4 + [c_size_t, c_void_p]),
+    "dcd_dgde_gmw_refine_workspace_bytes": (c_size_t, [c_int64, c_int, c_int, c_int64]),
+    "dcd_dgde_gmw_refine_fwd": (c_int, [c_void_p] * 3 + [c_int64] + [c_int] * 6 + [c_void_p] * 6 + [c_int64, c_int, c_int, c_int, c_int64]
+                                + [c_void_p] * 8 + [c_size_t, c_void_p]),
 }
 
 _lib = None

@@ -18,7 +18,10 @@ int launch_gmw_weights_fwd(const float*, const float*, const float*, const float
 int launch_dgde_locate(const float*, const float*, const float*, const float*, const float*, const float*, const float*,
                        const float*, const float*, int64_t, int, float, float, int, float, float*, float*, cudaStream_t);
 int launch_dgde_frame(const float*, const int64_t*, const int32_t*, int, int, int, int, int, int, const float*, const float*,
-                      const float*, const float*, int64_t, int, float, float, int, float, float*, float*, float*, float*, cudaStream_t);
+                      const float*, const float*, int64_t, int, float, float, int, float, float*, float*, float*, float*, float*, float*,
+                      cudaStream_t);
+int launch_gmw_aggregate_rescale_fwd(const float*, const float*, const int64_t*, int64_t, int64_t, int, int, float*, const float*,
+                                     const float*, float*, cudaStream_t);
 int launch_dgde_depth_ensemble(const float*, const float*, const float*, const float*, const float*, const float*, const float*,
                                int64_t, float, float, float, float, float*, float*, float*, int64_t*, float*, cudaStream_t);
 int launch_gmw_ray_rescale(const float*, const float*, const float*, int64_t, float*, cudaStream_t);
@@ -51,6 +54,45 @@ namespace {
 inline bool bad_n(int n) { return n < 2 || n > DCD_MAX_KPTS; }
 inline bool misaligned(const void* p, size_t a) { return (reinterpret_cast<uintptr_t>(p) & (a - 1)) != 0; }
 inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
+
+// The chunk loop of dcd_gmw_depth_fwd (workspace laid out by dcd_gmw_depth_workspace_bytes for `chunk` <= N objects): per
+// chunk the top-k edge selection, the edge MLP and the softmax aggregate.  raw_loc != NULL (with dims, loc_out; all [N,3]):
+// the aggregate also moves raw_loc along its viewing ray to the weighted depth (dcd_dgde_gmw_refine_fwd).
+int gmw_depth_chunks(const float* kpts2d, const float* kpts3d, const float* rot, const float* params4, const float* params6,
+                     int64_t N, int n, int depth, int k, float lo, float hi, int64_t chunk, float* depth_out, int64_t* idx_out,
+                     float* reg_weights, void* workspace, const float* raw_loc, const float* dims, float* loc_out,
+                     cudaStream_t st) {
+    const int64_t E = num_edges(n);
+    unsigned char* p = static_cast<unsigned char*>(workspace);
+    const size_t mlp_bytes = align_up(dcd_gmw_workspace_bytes(chunk, n, depth, 0), 256);
+    float* mlp_ws = reinterpret_cast<float*>(p);
+    p += mlp_bytes;
+    int64_t* idx_ws = reinterpret_cast<int64_t*>(p);
+    p += align_up((size_t)chunk * E * sizeof(int64_t), 256);
+    float* zsel_ws = reinterpret_cast<float*>(p);
+    p += align_up((size_t)chunk * E * sizeof(float), 256);
+    float* regw_ws = reinterpret_cast<float*>(p);
+    for (int64_t c0 = 0; c0 < N; c0 += chunk) {
+        const int64_t nc = (N - c0 < chunk) ? N - c0 : chunk;
+        const float* k2 = kpts2d + c0 * n * 2;
+        const float* k3 = kpts3d + c0 * n * 3;
+        int64_t* idx = idx_out ? idx_out + c0 * k : idx_ws;
+        float* rw = reg_weights ? reg_weights + c0 * E : regw_ws;
+        int rc = launch_edge_select(k2, k3, rot + c0, nullptr, nullptr, nc, n, k, lo, hi, 0, idx, zsel_ws, nullptr,
+                                    nullptr, st);
+        if (rc != DCD_OK) return rc;
+        rc = launch_gmw_weights_fwd(k2, k3, params4, params6, nc, n, depth, 0, rw, nullptr, nullptr, mlp_ws, st);
+        if (rc != DCD_OK) return rc;
+        rc = raw_loc ? launch_gmw_aggregate_rescale_fwd(rw, zsel_ws, idx, nc, E, k, 1, depth_out + c0, raw_loc + c0 * 3,
+                                                        dims + c0 * 3, loc_out + c0 * 3, st)
+                     : launch_gmw_aggregate_fwd(rw, zsel_ws, idx, nc, E, k, 1, depth_out + c0, nullptr, st);
+        if (rc != DCD_OK) return rc;
+    }
+    return DCD_OK;
+}
+
+// fixed scalars of the detector head's frame epilogue (frame_depths_from_map) and of compute_z inside the refine chain
+constexpr float kDgdeLo = 2.f, kDgdeHi = 80.f, kDownRatio = 4.f, kGmwLo = 0.1f, kGmwHi = 80.f;
 }  // namespace
 
 extern "C" {
@@ -133,7 +175,8 @@ int dcd_dgde_frame_fwd(const float* feature_maps, const int64_t* index, const in
     if (!feature_maps || !index || !rot || !K || !pad || (!depth_out && !locations)) return DCD_E_INVALID;
     if (B > 1 && !batch_idx) return DCD_E_INVALID;
     return launch_dgde_frame(feature_maps, index, batch_idx, C, H, W, ch_kpts2d, ch_kpts3d, ch_offset3d, rot, K, pad, dims, N, n, lo,
-                             hi, flags, down_ratio, depth_out, locations, kpts_img_out, kps3d_out, (cudaStream_t)stream);
+                             hi, flags, down_ratio, depth_out, locations, kpts_img_out, kps3d_out, nullptr, nullptr,
+                             (cudaStream_t)stream);
 }
 
 int dcd_dgde_depth_ensemble_fwd(const float* kp10, const float* dims, const float* K, const float* direct,
@@ -351,31 +394,51 @@ int dcd_gmw_depth_fwd(const float* kpts2d, const float* kpts3d, const float* rot
     if (chunk > N) chunk = N;
     if (misaligned(workspace, 256) || workspace_bytes < dcd_gmw_depth_workspace_bytes(N, n, depth, chunk))
         return DCD_E_WORKSPACE;
+    return gmw_depth_chunks(kpts2d, kpts3d, rot, params4, params6, N, n, depth, k, lo, hi, chunk, depth_out, idx_out, reg_weights,
+                            workspace, nullptr, nullptr, nullptr, (cudaStream_t)stream);
+}
+
+// workspace of the refine chain: [GMW 2D keypoints N*73*2][template points N*73*3][dcd_gmw_depth_fwd workspace for 73 keypoints]
+size_t dcd_dgde_gmw_refine_workspace_bytes(int64_t N, int n, int depth, int64_t chunk) {
+    if (N <= 0 || bad_n(n) || n < DCD_GMW_KPTS || depth < 1 || chunk < 1) return 0;
+    size_t b = align_up((size_t)N * DCD_GMW_KPTS * 2 * sizeof(float), 256);
+    b += align_up((size_t)N * DCD_GMW_KPTS * 3 * sizeof(float), 256);
+    return b + dcd_gmw_depth_workspace_bytes(N, DCD_GMW_KPTS, depth, chunk);
+}
+
+int dcd_dgde_gmw_refine_fwd(const float* feature_maps, const int64_t* index, const int32_t* batch_idx, int64_t B, int C, int H,
+                            int W, int ch_kpts2d, int ch_kpts3d, int ch_offset3d, const float* rot, const float* K, const float* pad,
+                            const float* dims, const float* params4, const float* params6, int64_t N, int n, int depth, int k,
+                            int64_t chunk, float* dgde_depth, float* dgde_location, float* gmw_depth, float* location,
+                            float* gmw_kpts, float* kps3d, int64_t* idx_out, void* workspace, size_t workspace_bytes,
+                            void* stream) {
+    if (N < 0 || B < 1 || C < 1 || H < 1 || W < 1 || bad_n(n) || n < DCD_GMW_KPTS || depth < 1 || chunk < 1)
+        return DCD_E_INVALID;
+    if (ch_kpts2d < 0 || ch_kpts2d + 2 * n > C || ch_kpts3d < 0 || ch_kpts3d + 3 * n > C || ch_offset3d < 0 || ch_offset3d + 2 > C)
+        return DCD_E_INVALID;
+    if (k < 1 || k > num_edges(DCD_GMW_KPTS)) return DCD_E_INVALID;
+    if (N == 0) return DCD_OK;
+    if (!feature_maps || !index || !rot || !K || !pad || !dims || !params4 || !params6) return DCD_E_INVALID;
+    if (!dgde_depth || !dgde_location || !gmw_depth || !location || !workspace) return DCD_E_INVALID;
+    if (B > 1 && !batch_idx) return DCD_E_INVALID;
+    if (misaligned(gmw_kpts, 8) || misaligned(params4, 16) || misaligned(params6, 16)) return DCD_E_INVALID;
+    if (chunk > N) chunk = N;
+    if (misaligned(workspace, 256) || workspace_bytes < dcd_dgde_gmw_refine_workspace_bytes(N, n, depth, chunk))
+        return DCD_E_WORKSPACE;
     cudaStream_t st = (cudaStream_t)stream;
     unsigned char* p = static_cast<unsigned char*>(workspace);
-    const size_t mlp_bytes = align_up(dcd_gmw_workspace_bytes(chunk, n, depth, 0), 256);
-    float* mlp_ws = reinterpret_cast<float*>(p);
-    p += mlp_bytes;
-    int64_t* idx_ws = reinterpret_cast<int64_t*>(p);
-    p += align_up((size_t)chunk * E * sizeof(int64_t), 256);
-    float* zsel_ws = reinterpret_cast<float*>(p);
-    p += align_up((size_t)chunk * E * sizeof(float), 256);
-    float* regw_ws = reinterpret_cast<float*>(p);
-    for (int64_t c0 = 0; c0 < N; c0 += chunk) {
-        const int64_t nc = (N - c0 < chunk) ? N - c0 : chunk;
-        const float* k2 = kpts2d + c0 * n * 2;
-        const float* k3 = kpts3d + c0 * n * 3;
-        int64_t* idx = idx_out ? idx_out + c0 * k : idx_ws;
-        float* rw = reg_weights ? reg_weights + c0 * E : regw_ws;
-        int rc = launch_edge_select(k2, k3, rot + c0, nullptr, nullptr, nc, n, k, lo, hi, 0, idx, zsel_ws, nullptr,
-                                    nullptr, st);
-        if (rc != DCD_OK) return rc;
-        rc = launch_gmw_weights_fwd(k2, k3, params4, params6, nc, n, depth, 0, rw, nullptr, nullptr, mlp_ws, st);
-        if (rc != DCD_OK) return rc;
-        rc = launch_gmw_aggregate_fwd(rw, zsel_ws, idx, nc, E, k, 1, depth_out + c0, nullptr, st);
-        if (rc != DCD_OK) return rc;
-    }
-    return DCD_OK;
+    float* k2 = reinterpret_cast<float*>(p);
+    p += align_up((size_t)N * DCD_GMW_KPTS * 2 * sizeof(float), 256);
+    float* k3 = reinterpret_cast<float*>(p);
+    p += align_up((size_t)N * DCD_GMW_KPTS * 3 * sizeof(float), 256);
+    if (gmw_kpts) k2 = gmw_kpts;
+    if (kps3d) k3 = kps3d;
+    int rc = launch_dgde_frame(feature_maps, index, batch_idx, C, H, W, ch_kpts2d, ch_kpts3d, ch_offset3d, rot, K, pad, dims, N, n,
+                               kDgdeLo, kDgdeHi, DCD_NORMALISE_2D | DCD_SUB_B3, kDownRatio, dgde_depth, dgde_location, nullptr,
+                               nullptr, k2, k3, st);
+    if (rc != DCD_OK) return rc;
+    return gmw_depth_chunks(k2, k3, rot, params4, params6, N, DCD_GMW_KPTS, depth, k, kGmwLo, kGmwHi, chunk, gmw_depth, idx_out,
+                            nullptr, p, dgde_location, dims, location, st);
 }
 
 }  // extern "C"

@@ -92,14 +92,17 @@ dgde_locate_warp_kernel(const float* __restrict__ kpts_off, const float* __restr
 // the values of their channel groups at that position of the [B,C,H,W] map (select_point_of_interest,
 // DGDE/model/layers/utils.py:120-145, + the key2channel slices of detector_infer.py:133,216,219), so POI gather ->
 // image keypoints -> edge solve -> mean -> location is ONE launch and the [B,K,C] gather never exists in memory.
-template <int THREADS>
+// GMW = true (dcd_dgde_gmw_refine_fwd) also writes GMW's inputs for keypoints 0 .. DCD_GMW_KPTS-1: the normalised 2D keypoints
+// ((u - K[0][2]) / K[0][0], (v - K[1][2]) / K[1][1]; the two FP32 roundings of wire.from_detector) and the template points,
+// both with a row stride of DCD_GMW_KPTS.  GMW = false is the kernel of dcd_dgde_frame_fwd, unchanged.
+template <int THREADS, bool GMW>
 __global__ void __launch_bounds__(THREADS)
 dgde_frame_warp_kernel(const float* __restrict__ fmap, const int64_t* __restrict__ index, const int32_t* __restrict__ batch_idx,
                        int C, int H, int W, int ch_k2, int ch_k3, int ch_off,
                        const float* __restrict__ rot, const float* __restrict__ K, const float* __restrict__ pad,
                        const float* __restrict__ dims, int64_t N, int n, float lo, float hi, int flags, float down_ratio,
                        float* __restrict__ depth_out, float* __restrict__ loc_out, float* __restrict__ kimg_out,
-                       float* __restrict__ k3_out) {
+                       float* __restrict__ k3_out, float* __restrict__ gmw_k2_out, float* __restrict__ gmw_k3_out) {
     constexpr int NWARP = THREADS / 32;
     const int E = n * (n - 1) / 2;
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -144,6 +147,16 @@ dgde_frame_warp_kernel(const float* __restrict__ fmap, const int64_t* __restrict
                 float* o = k3_out + (obj * n + t) * 3;
                 o[0] = X; o[1] = Y; o[2] = Z;
             }
+            if constexpr (GMW) {
+                if (t < DCD_GMW_KPTS) {
+                    const float u_img = __fsub_rn(__fmul_rn(__fadd_rn(chan(ch_k2 + 2 * t), cx), down_ratio), pad_u);
+                    float* g2 = gmw_k2_out + (obj * DCD_GMW_KPTS + t) * 2;
+                    g2[0] = __fdiv_rn(__fsub_rn(u_img, c_u), f_u);
+                    g2[1] = __fdiv_rn(__fsub_rn(v_img, c_v), f_v);
+                    float* g3 = gmw_k3_out + (obj * DCD_GMW_KPTS + t) * 3;
+                    g3[0] = X; g3[1] = Y; g3[2] = Z;
+                }
+            }
         }
         __syncwarp();
         float acc = 0.f;
@@ -175,21 +188,23 @@ dgde_frame_warp_kernel(const float* __restrict__ fmap, const int64_t* __restrict
 
 }  // namespace
 
+// gmw_k2_out == NULL: the dcd_dgde_frame_fwd kernel; otherwise (with gmw_k3_out, both [N,DCD_GMW_KPTS,.], n >= DCD_GMW_KPTS) the
+// GMW = true instantiation that also writes GMW's inputs.
 int launch_dgde_frame(const float* fmap, const int64_t* index, const int32_t* batch_idx, int C, int H, int W, int ch_k2, int ch_k3,
                       int ch_off, const float* rot, const float* K, const float* pad, const float* dims, int64_t N, int n, float lo,
                       float hi, int flags, float down_ratio, float* depth_out, float* loc_out, float* kimg_out, float* k3_out,
-                      cudaStream_t st) {
+                      float* gmw_k2_out, float* gmw_k3_out, cudaStream_t st) {
     constexpr int T = 128;                                  // a frame has <= 50 detections: more, smaller CTAs
     const int E = n * (n - 1) / 2;
     const size_t smem = (size_t)(T / 32) * n * sizeof(float4) + (size_t)E * sizeof(uint32_t);
     if (smem > 227 * 1024) return DCD_E_UNSUPPORTED;
-    if (smem > 48 * 1024)
-        cudaFuncSetAttribute(dgde_frame_warp_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    auto kernel = gmw_k2_out != nullptr ? dgde_frame_warp_kernel<T, true> : dgde_frame_warp_kernel<T, false>;
+    if (smem > 48 * 1024) cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     const int64_t want = (N + T / 32 - 1) / (T / 32);
     const int64_t cap = (int64_t)device_sm_count() * 8;
     const int grid = (int)(want < cap ? want : cap);
-    dgde_frame_warp_kernel<T><<<grid, T, smem, st>>>(fmap, index, batch_idx, C, H, W, ch_k2, ch_k3, ch_off, rot, K, pad, dims, N, n,
-                                                     lo, hi, flags, down_ratio, depth_out, loc_out, kimg_out, k3_out);
+    kernel<<<grid, T, smem, st>>>(fmap, index, batch_idx, C, H, W, ch_k2, ch_k3, ch_off, rot, K, pad, dims, N, n, lo, hi, flags,
+                                  down_ratio, depth_out, loc_out, kimg_out, k3_out, gmw_k2_out, gmw_k3_out);
     DCD_CHECK_LAUNCH();
     return DCD_OK;
 }
@@ -494,12 +509,8 @@ gmw_ray_rescale_kernel(const float* __restrict__ raw_location, const float* __re
                        int64_t N, float* __restrict__ out) {
     const int64_t o = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (o >= N) return;
-    const float x = __ldg(raw_location + o * 3), y = __ldg(raw_location + o * 3 + 1), z = __ldg(raw_location + o * 3 + 2);
-    const float scale = __fdiv_rn(__ldg(pred_depth + o), z);
-    const float hh = __fmul_rn(__ldg(dim + o * 3), 0.5f);
-    out[o * 3 + 0] = __fmul_rn(scale, x);
-    out[o * 3 + 1] = __fadd_rn(__fmul_rn(scale, __fsub_rn(y, hh)), hh);
-    out[o * 3 + 2] = __fmul_rn(scale, z);
+    ray_rescale_one(__ldg(raw_location + o * 3), __ldg(raw_location + o * 3 + 1), __ldg(raw_location + o * 3 + 2),
+                    __ldg(pred_depth + o), __ldg(dim + o * 3), out + o * 3);
 }
 
 }  // namespace

@@ -31,10 +31,14 @@ __device__ __forceinline__ Softmax warp_softmax_stats(const float* __restrict__ 
     return {mx, s};
 }
 
+// RESCALE (dcd_dgde_gmw_refine_fwd): lane 0 also moves the detector location raw_loc [N,3] to the weighted depth it just
+// wrote (ray_rescale_one with h = dims[:, 1], dims (l,h,w)) -> loc_out [N,3]: the values of gmw_ray_rescale_kernel on depth_out.
+template <bool RESCALE>
 __global__ void __launch_bounds__(AGG_THREADS)
 gmw_aggregate_fwd_kernel(const float* __restrict__ reg_w, const float* __restrict__ depths,
                          const int64_t* __restrict__ idx, int64_t N, int64_t E, int k, int sel,
-                         float* __restrict__ depth_out, float* __restrict__ probs) {
+                         float* __restrict__ depth_out, float* __restrict__ probs, const float* __restrict__ raw_loc,
+                         const float* __restrict__ dims, float* __restrict__ loc_out) {
     const int lane = threadIdx.x & 31;
     const int64_t obj = (int64_t)blockIdx.x * (AGG_THREADS / 32) + (threadIdx.x >> 5);
     if (obj >= N) return;
@@ -51,7 +55,12 @@ gmw_aggregate_fwd_kernel(const float* __restrict__ reg_w, const float* __restric
         acc += z * p;
     }
     acc = warp_sum(acc);
-    if (lane == 0) depth_out[obj] = acc;
+    if (lane == 0) {
+        depth_out[obj] = acc;
+        if constexpr (RESCALE)
+            ray_rescale_one(__ldg(raw_loc + obj * 3), __ldg(raw_loc + obj * 3 + 1), __ldg(raw_loc + obj * 3 + 2), acc,
+                            __ldg(dims + obj * 3 + 1), loc_out + obj * 3);
+    }
 }
 
 __global__ void __launch_bounds__(AGG_THREADS)
@@ -98,7 +107,19 @@ int launch_gmw_aggregate_fwd(const float* reg_w, const float* depths, const int6
                              int k, int sel, float* depth_out, float* probs, cudaStream_t st) {
     const int64_t per = AGG_THREADS / 32;
     const unsigned grid = (unsigned)((N + per - 1) / per);
-    gmw_aggregate_fwd_kernel<<<grid, AGG_THREADS, 0, st>>>(reg_w, depths, idx, N, E, k, sel, depth_out, probs);
+    gmw_aggregate_fwd_kernel<false><<<grid, AGG_THREADS, 0, st>>>(reg_w, depths, idx, N, E, k, sel, depth_out, probs, nullptr,
+                                                                  nullptr, nullptr);
+    DCD_CHECK_LAUNCH();
+    return DCD_OK;
+}
+
+int launch_gmw_aggregate_rescale_fwd(const float* reg_w, const float* depths, const int64_t* idx, int64_t N, int64_t E, int k,
+                                     int sel, float* depth_out, const float* raw_loc, const float* dims, float* loc_out,
+                                     cudaStream_t st) {
+    const int64_t per = AGG_THREADS / 32;
+    const unsigned grid = (unsigned)((N + per - 1) / per);
+    gmw_aggregate_fwd_kernel<true><<<grid, AGG_THREADS, 0, st>>>(reg_w, depths, idx, N, E, k, sel, depth_out, nullptr, raw_loc,
+                                                                 dims, loc_out);
     DCD_CHECK_LAUNCH();
     return DCD_OK;
 }

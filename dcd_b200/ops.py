@@ -269,18 +269,11 @@ def compute_pairs_kpts_depth(pred_extra_kpts_2d, pred_bbox_points, pred_offset_3
 DGDE_CHANNELS = {"3d_offset": 4, "extra_kpts_2d": 50, "extra_kpts_3d": 196}
 
 
-def frame_depths_from_map(pred_regression, indexs, pred_rots, P, pad_size, dims=None, batch_idxs=None, n: int = 73,
-                          channels=None, return_keypoints: bool = False):
-    """POI gather + image keypoints + edge solve + mean + 3D location in ONE launch, reading the regression map itself
-    (detector_infer.py:107 select_point_of_interest, :133 / :216-219 channel slices, :215-227 compute_pairs_kpts_depth,
-    :186-188 decode_location_flatten): pred_regression [B,C,H,W], indexs [N] int64 heat-map positions y * W + x of the kept
-    detections (select_topk), pred_rots [N] decoded yaw, P the 3x4 calibration ([3,4], per image [B,3,4] with batch_idxs, or
-    per object), pad_size [2] / [B,2], dims [N,3] or None -> (depth [N], locations [N,3]) and, with return_keypoints, the
-    image-space 2D keypoints [N,n,2] and template points [N,n,3] that generate_infer_data dumps (:228-236).  Inference-only."""
-    require_cuda(pred_regression, indexs, pred_rots)
-    _inference_only("frame_depths_from_map", pred_regression, pred_rots, dims)
+def _frame_inputs(pred_regression, indexs, pred_rots, P, pad_size, batch_idxs, channels):
+    """Arguments of the regression-map entry points -> (map [B,C,H,W], index [N] int64, batch index [N] int32 or None,
+    yaw [N], calibration [N,3,4], pad [N,2] (all FP32 contiguous), channel table)."""
     fm = f32c(pred_regression)
-    B, C, H, W = fm.shape
+    B = fm.shape[0]
     ch = dict(DGDE_CHANNELS)
     if channels:
         ch.update(channels)
@@ -297,6 +290,22 @@ def frame_depths_from_map(pred_regression, indexs, pred_rots, P, pad_size, dims=
         Pt = Pt.to(dev)[batch_idxs.to(dev).long()]
     K = _calib_per_object(Pt, N, dev)
     pad = _pad_per_object(pad_size, batch_idxs, N, dev)
+    return fm, idx, bi, rot, K, pad, ch
+
+
+def frame_depths_from_map(pred_regression, indexs, pred_rots, P, pad_size, dims=None, batch_idxs=None, n: int = 73,
+                          channels=None, return_keypoints: bool = False):
+    """POI gather + image keypoints + edge solve + mean + 3D location in ONE launch, reading the regression map itself
+    (detector_infer.py:107 select_point_of_interest, :133 / :216-219 channel slices, :215-227 compute_pairs_kpts_depth,
+    :186-188 decode_location_flatten): pred_regression [B,C,H,W], indexs [N] int64 heat-map positions y * W + x of the kept
+    detections (select_topk), pred_rots [N] decoded yaw, P the 3x4 calibration ([3,4], per image [B,3,4] with batch_idxs, or
+    per object), pad_size [2] / [B,2], dims [N,3] or None -> (depth [N], locations [N,3]) and, with return_keypoints, the
+    image-space 2D keypoints [N,n,2] and template points [N,n,3] that generate_infer_data dumps (:228-236).  Inference-only."""
+    require_cuda(pred_regression, indexs, pred_rots)
+    _inference_only("frame_depths_from_map", pred_regression, pred_rots, dims)
+    fm, idx, bi, rot, K, pad, ch = _frame_inputs(pred_regression, indexs, pred_rots, P, pad_size, batch_idxs, channels)
+    B, C, H, W = fm.shape
+    N, dev = idx.shape[0], fm.device
     d3 = f32c(dims) if dims is not None else None
     depth = torch.empty((N,), dtype=torch.float32, device=dev)
     loc = torch.empty((N, 3), dtype=torch.float32, device=dev)
@@ -816,3 +825,62 @@ def gmw_weighted_depth(kpts_2d, kpts_3d, pred_rot, model: GMW, chunk: int = 1024
                                       model.depth, num_k, lo, hi, chunk, ptr(out), ptr(idx), 0, ptr(ws),
                                       ws.numel() * 4, stream_ptr()), "dcd_gmw_depth_fwd")
     return (out, idx) if return_idx else out
+
+
+GMW_KPTS = 73                # GMW reads the first 73 keypoints of every object (DCD_GMW_KPTS, wire.NUM_KPTS)
+
+
+def refine_detections(pred_regression, indexs, pred_rots, P, pad_size, dims, gmw: GMW, batch_idxs=None, n: int = 73,
+                      channels=None, chunk: int = 1024, params=None, return_inputs: bool = False) -> Dict[str, torch.Tensor]:
+    """DGDE detections refined by GMW in one stream-ordered library call (dcd_dgde_gmw_refine_fwd): the regression map to
+    the GMW-rescaled 3D locations with no host round trip (the reference writes gen_data_infer.json in
+    DGDE/engine/inference.py:59-84 and reads it back in GMW/main.py:524-547).
+
+    pred_regression, indexs, pred_rots, P, pad_size, batch_idxs, n, channels: as frame_depths_from_map (P [3,4], per image
+    [B,3,4] with batch_idxs, or per object [N,3,4]).  dims [N,3]: the head's pred_dimensions in ITS order (l, h, w); h =
+    dims[:, 1] is the `+ h/2` of the DGDE location and the h of the GMW ray rescale (GMW itself orders dim (h, w, l)).
+    GMW's compute_z gets the same decoded yaw `pred_rots` as the DGDE solve (what wire.from_detector(pred_rot=...) records
+    too).  gmw: a dcd_b200.GMW (its depth, and its parameter blobs unless `params` = (params4, params6) is given, e.g.
+    `model._dcd_b200_blobs.get()` of a reference module patched by dcd_b200.patch.install, with gmw=`model._dcd_b200`).
+    chunk: objects per GMW launch sequence (bounds the workspace, as gmw_weighted_depth's).
+
+    Returns a dict: dgde_depth [N], dgde_location [N,3] (== frame_depths_from_map(..., dims)), gmw_depth [N] and location
+    [N,3] (the GMW-rescaled location); with return_inputs also kpts_2d [N,73,2] (the normalised keypoints
+    ((u - c_u) / f_u, (v - c_v) / f_v) of wire.from_detector, bit for bit), kpts_3d [N,73,3] and good_idx [N,1500] int64.
+    Every output equals frame_depths_from_map -> normalisation -> gmw_weighted_depth (same chunk) -> ray_rescale(loc, z,
+    dims[:, [1, 2, 0]]) bit for bit.  Inference-only (raises when an input requires grad; no gradient reaches the GMW
+    parameters); a detection index outside the map gives NaN outputs for that object only."""
+    if dims is None:
+        raise ValueError("refine_detections needs dims [N,3] (l, h, w): h places the box centre for the ray rescale")
+    if n < GMW_KPTS:
+        raise ValueError("refine_detections needs n >= %d keypoints per object (GMW reads keypoints 0..%d), got %d"
+                         % (GMW_KPTS, GMW_KPTS - 1, n))
+    _inference_only("refine_detections", pred_regression, pred_rots, dims)
+    p4, p6 = params if params is not None else (gmw.params4, gmw.params6)
+    require_cuda(pred_regression, indexs, pred_rots, dims, p4, p6)
+    fm, idx, bi, rot, K, pad, ch = _frame_inputs(pred_regression, indexs, pred_rots, P, pad_size, batch_idxs, channels)
+    B, C, H, W = fm.shape
+    N, dev = idx.shape[0], fm.device
+    d3 = f32c(dims)
+    if tuple(d3.shape) != (N, 3):
+        raise ValueError("dims must be [N,3] (l, h, w), got %s" % (tuple(d3.shape),))
+    p4, p6 = f32c(p4.detach()), f32c(p6.detach())
+    f32 = dict(dtype=torch.float32, device=dev)
+    out = {"dgde_depth": torch.empty((N,), **f32), "dgde_location": torch.empty((N, 3), **f32),
+           "gmw_depth": torch.empty((N,), **f32), "location": torch.empty((N, 3), **f32)}
+    k2 = k3 = gidx = None
+    if return_inputs:
+        k2 = torch.empty((N, GMW_KPTS, 2), **f32)
+        k3 = torch.empty((N, GMW_KPTS, 3), **f32)
+        gidx = torch.empty((N, K_SEL), dtype=torch.int64, device=dev)
+        out.update(kpts_2d=k2, kpts_3d=k3, good_idx=gidx)
+    if N:
+        L = _lib.lib()
+        chunk = max(1, min(chunk, N))
+        ws = _alloc_bytes(L.dcd_dgde_gmw_refine_workspace_bytes(N, n, gmw.depth, chunk), dev)
+        check(L.dcd_dgde_gmw_refine_fwd(ptr(fm), ptr(idx), ptr(bi), B, C, H, W, ch["extra_kpts_2d"], ch["extra_kpts_3d"],
+                                        ch["3d_offset"], ptr(rot), ptr(K), ptr(pad), ptr(d3), ptr(p4), ptr(p6), N, n, gmw.depth,
+                                        K_SEL, chunk, ptr(out["dgde_depth"]), ptr(out["dgde_location"]), ptr(out["gmw_depth"]),
+                                        ptr(out["location"]), ptr(k2), ptr(k3), ptr(gidx), ptr(ws), ws.numel() * 4,
+                                        stream_ptr()), "dcd_dgde_gmw_refine_fwd")
+    return out

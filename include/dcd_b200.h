@@ -12,6 +12,7 @@
  * Notation: N objects, n keypoints per object, E = n(n-1)/2 edges in row-major strict-upper-triangle
  * order (edge e <-> (i,j), i<j; identical to torch.triu_indices(n,n,1)), k selected edges (1500 in
  * the reference).  Reference citations are relative to the BraveGroup/DCD repository.
+ * 31 exported functions.
  */
 #ifndef DCD_B200_H_
 #define DCD_B200_H_
@@ -45,6 +46,7 @@ extern "C" {
 
 #define DCD_MAX_KPTS      256   /* pair ids are packed in 16 bits */
 #define DCD_NET_CH        128   /* channels of the edge MLP (yi2018cvpr/config.py:72) */
+#define DCD_GMW_KPTS       73   /* GMW reads the first 73 keypoints of every object (GMW/utilities/dataset_utilities.py:45-46) */
 
 int         dcd_version(void);
 const char* dcd_strerror(int rc);
@@ -298,6 +300,29 @@ int dcd_gmw_depth_fwd(const float* kpts2d, const float* kpts3d, const float* rot
                       int64_t N, int n, int depth, int k, float lo, float hi, int64_t chunk,
                       float* depth_out, int64_t* idx_out, float* reg_weights,
                       void* workspace, size_t workspace_bytes, void* stream);
+
+/* ------------------------------------------------------------------------------------------------
+ * DGDE detections refined by GMW in one stream-ordered chain (SURVEY 8f row N3, on-GPU half): the regression map to the
+ * GMW-rescaled 3D locations, replacing the gen_data_infer.json hand-off (DGDE/engine/inference.py:59-84 -> GMW/main.py:
+ * 524-547).  Launches, no host synchronisation, no allocation:
+ *   1. the dcd_dgde_frame_fwd kernel over all N objects with its fixed scalars (lo, hi = 2, 80; DCD_NORMALISE_2D |
+ *      DCD_SUB_B3; down_ratio 4) -> dgde_depth [N], dgde_location [N,3] (with + h/2), and GMW's inputs for keypoints
+ *      0 .. 72: gmw_kpts [N,73,2] = ((u - K[0][2]) / K[0][0], (v - K[1][2]) / K[1][1]) (FP32, one rounding each) and
+ *      kps3d [N,73,3];
+ *   2. per chunk of <= `chunk` objects, dcd_gmw_depth_fwd's sequence on those inputs with lo, hi = 0.1, 80, no flags and
+ *      the DGDE yaw `rot` -> gmw_depth [N]; its aggregate also writes location [N,3] = the GMW ray rescale
+ *      (dcd_gmw_ray_rescale_fwd's operations) of dgde_location to gmw_depth with h = dims[:, 1].
+ * Every output is bit-identical to dcd_dgde_frame_fwd -> normalisation -> dcd_gmw_depth_fwd (same chunk) ->
+ * dcd_gmw_ray_rescale_fwd(dim = dims[:, (1,2,0)]).  Arguments as dcd_dgde_frame_fwd and dcd_gmw_depth_fwd; dims [N,3] (l,h,w)
+ * is required; n >= DCD_GMW_KPTS; 1 <= k <= 2628.  gmw_kpts, kps3d, idx_out [N,k] int64 (the selected edges) may be NULL
+ * (the workspace holds them then).  A position outside the map yields NaN outputs for that object only. */
+size_t dcd_dgde_gmw_refine_workspace_bytes(int64_t N, int n, int depth, int64_t chunk);
+int dcd_dgde_gmw_refine_fwd(const float* feature_maps, const int64_t* index, const int32_t* batch_idx, int64_t B, int C, int H,
+                            int W, int ch_kpts2d, int ch_kpts3d, int ch_offset3d, const float* rot, const float* K, const float* pad,
+                            const float* dims, const float* params4, const float* params6, int64_t N, int n, int depth, int k,
+                            int64_t chunk, float* dgde_depth, float* dgde_location, float* gmw_depth, float* location,
+                            float* gmw_kpts, float* kps3d, int64_t* idx_out, void* workspace, size_t workspace_bytes,
+                            void* stream);
 
 #if defined(__GNUC__)
 #pragma GCC visibility pop
