@@ -364,6 +364,7 @@ int dcd_gmw_aggregate_bwd(const float* reg_weights, const float* depths, const i
                           int k, int depths_are_selected, const float* grad_depth_out, float* grad_reg_weights,
                           float* grad_depths, void* stream) {
     if (N < 0 || E < 1 || k < 1 || k > E) return DCD_E_INVALID;
+    if (k > DCD_AGG_BWD_MAX_K) return DCD_E_UNSUPPORTED;
     if (N == 0) return DCD_OK;
     if (!reg_weights || !depths || !idx || !grad_depth_out || !grad_reg_weights) return DCD_E_INVALID;
     return launch_gmw_aggregate_bwd(reg_weights, depths, idx, N, E, k, depths_are_selected, grad_depth_out,

@@ -63,6 +63,17 @@ gmw_aggregate_fwd_kernel(const float* __restrict__ reg_w, const float* __restric
     }
 }
 
+// Claim of slot r on its edge, stored in the grad_w row as the bits of a positive NaN whose payload k - r is largest for the
+// first slot.  A computed gradient is never such a NaN: the GPU's float arithmetic returns the canonical NaN 0x7fffffff, and
+// k - r <= k <= DCD_AGG_BWD_MAX_K = 2^22 stays below that payload.
+__device__ __forceinline__ int slot_claim(int r, int k) { return 0x7f800000 | (k - r); }
+
+// The backward of the gather is torch's scatter_add: a repeated index receives the SUM of its slots' gradients.  Every slot
+// claims its edge with an integer atomicMax (the first slot wins); if no slot lost its claim (all indices distinct, the case of
+// compute_z's top-k) each slot writes its value as a plain store.  Otherwise the warp walks the slots in ascending chunks of
+// 32: the lanes of a chunk that share an edge are summed by the lowest of them in lane order, onto the edge's running sum
+// from earlier chunks (the first slot starts it), so repeated edges are summed in ascending slot order, deterministically,
+// without floating-point atomics.
 __global__ void __launch_bounds__(AGG_THREADS)
 gmw_aggregate_bwd_kernel(const float* __restrict__ reg_w, const float* __restrict__ depths,
                          const int64_t* __restrict__ idx, int64_t N, int64_t E, int k, int sel,
@@ -75,9 +86,11 @@ gmw_aggregate_bwd_kernel(const float* __restrict__ reg_w, const float* __restric
     const int64_t* id_row = idx + obj * k;
     const float* z_row = depths + obj * (sel ? (int64_t)k : E);
     float* gw_row = grad_w + obj * E;
+    int* claim_row = reinterpret_cast<int*>(gw_row);
+    float* gz_dense = grad_z != nullptr && !sel ? grad_z + obj * E : nullptr;
     for (int64_t e = lane; e < E; e += 32) gw_row[e] = 0.f;
-    if (grad_z != nullptr && !sel)
-        for (int64_t e = lane; e < E; e += 32) grad_z[obj * E + e] = 0.f;
+    if (gz_dense != nullptr)
+        for (int64_t e = lane; e < E; e += 32) gz_dense[e] = 0.f;
     const Softmax sm = warp_softmax_stats(w_row, id_row, k, E, lane);
     float acc = 0.f;
     for (int r = lane; r < k; r += 32) {
@@ -88,16 +101,63 @@ gmw_aggregate_bwd_kernel(const float* __restrict__ reg_w, const float* __restric
     }
     const float Zbar = warp_sum(acc);
     const float g = __ldg(grad_out + obj);
-    __syncwarp();   // orders the zero fill before the scatter
-    for (int r = lane; r < k; r += 32) {
-        const int64_t id = edge_id(id_row, r, E);
-        const float p = __fdiv_rn(expf(__ldg(w_row + id) - sm.mx), sm.sum);
-        const float z = sel ? __ldg(z_row + r) : __ldg(z_row + id);
-        gw_row[id] = g * p * (z - Zbar);
-        if (grad_z != nullptr) {
-            if (sel) grad_z[obj * k + r] = g * p;
-            else grad_z[obj * E + id] = g * p;
+    __syncwarp();   // orders the zero fill before the claims
+    for (int r = lane; r < k; r += 32) atomicMax(claim_row + edge_id(id_row, r, E), slot_claim(r, k));
+    __syncwarp();
+    bool lost = false;
+    for (int r = lane; r < k; r += 32) lost |= __ldcg(claim_row + edge_id(id_row, r, E)) != slot_claim(r, k);
+    const bool repeated = __any_sync(0xffffffffu, lost);
+    __syncwarp();   // every claim is read before a value overwrites one
+    if (!repeated) {
+        for (int r = lane; r < k; r += 32) {
+            const int64_t id = edge_id(id_row, r, E);
+            const float p = __fdiv_rn(expf(__ldg(w_row + id) - sm.mx), sm.sum);
+            const float z = sel ? __ldg(z_row + r) : __ldg(z_row + id);
+            gw_row[id] = g * p * (z - Zbar);
+            if (grad_z != nullptr) {
+                if (sel) grad_z[obj * k + r] = g * p;
+                else gz_dense[id] = g * p;
+            }
         }
+        return;
+    }
+    for (int base = 0; base < k; base += 32) {
+        const int r = base + lane;
+        int64_t id = -1;
+        float vw = 0.f, vz = 0.f;
+        if (r < k) {
+            id = edge_id(id_row, r, E);
+            const float p = __fdiv_rn(expf(__ldg(w_row + id) - sm.mx), sm.sum);
+            const float z = sel ? __ldg(z_row + r) : __ldg(z_row + id);
+            vw = g * p * (z - Zbar);
+            vz = g * p;
+            if (grad_z != nullptr && sel) grad_z[obj * k + r] = vz;
+        }
+        const unsigned grp = __match_any_sync(0xffffffffu, (unsigned long long)id);
+        if (r < k) {
+            const bool lead = lane == __ffs(grp) - 1;
+            float sw = vw, sz = vz;
+            if (lead) {
+                const int cur = __ldcg(claim_row + id);
+                if (cur != slot_claim(r, k)) {                       // not the edge's first slot: continue its sum
+                    sw = __fadd_rn(__int_as_float(cur), vw);
+                    if (gz_dense != nullptr) sz = __fadd_rn(__ldcg(gz_dense + id), vz);
+                }
+            }
+            for (unsigned m = grp & (grp - 1u); m != 0u; m &= m - 1u) {   // the group's other lanes, ascending
+                const int j = __ffs(m) - 1;
+                const float aw = __shfl_sync(grp, vw, j), az = __shfl_sync(grp, vz, j);
+                if (lead) {
+                    sw = __fadd_rn(sw, aw);
+                    sz = __fadd_rn(sz, az);
+                }
+            }
+            if (lead) {
+                gw_row[id] = sw;
+                if (gz_dense != nullptr) gz_dense[id] = sz;
+            }
+        }
+        __syncwarp();   // this chunk's sums are stored before the next chunk reads them
     }
 }
 

@@ -787,7 +787,9 @@ class GMW(nn.Module):
 
 def compute_reg_loss(pre_depths, edge_weight, gt_depth, good_idx=None, validate: bool = False):
     """Drop-in for GMW/main.py:364-371 -> (reg_loss, Z_select_weighted).  Shapes are checked; `validate=True` also checks
-    the index range (a host synchronisation; the kernels clamp an out-of-range index instead of faulting)."""
+    the index range (a host synchronisation; the kernels clamp an out-of-range index to 0 or E - 1 instead of faulting).
+    good_idx may repeat an edge: as with torch.gather, every slot counts in the softmax and the edge's gradients are the sum
+    over its slots (in ascending slot order, deterministic)."""
     if good_idx is None:
         raise UnboundLocalError("compute_reg_loss needs good_idx (the reference fails without it too)")
     require_cuda(pre_depths, edge_weight, good_idx)

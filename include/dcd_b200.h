@@ -282,8 +282,12 @@ int dcd_gmw_aggregate_fwd(const float* reg_weights, const float* depths, const i
                           float* depth_out, float* probs, void* stream);
 
 /* Backward: grad_reg_weights [N,E] (dense, zero outside idx; OVERWRITTEN) = g * p_r * (z_r - depth_out),
- * grad_depths (may be NULL; [N,E] dense or [N,k] as in the forward) = g * p_r.
+ * grad_depths (may be NULL; [N,E] dense or [N,k] as in the forward) = g * p_r.  An edge that idx selects at several slots
+ * receives the sum over those slots (torch.gather's scatter_add backward), summed in ascending slot order: deterministic, no
+ * floating-point atomics; with distinct indices each edge's value is its one slot's.  An index outside [0, E) is clamped to
+ * 0 or E - 1 like the forward (and adds to that edge).  k > DCD_AGG_BWD_MAX_K returns DCD_E_UNSUPPORTED.
  */
+#define DCD_AGG_BWD_MAX_K (1 << 22)
 int dcd_gmw_aggregate_bwd(const float* reg_weights, const float* depths, const int64_t* idx,
                           int64_t N, int64_t E, int k, int depths_are_selected,
                           const float* grad_depth_out, float* grad_reg_weights, float* grad_depths,
