@@ -1,4 +1,4 @@
-"""ctypes binding of libdcd_b200.so (the C ABI declared in include/dcd_b200.h).
+"""ctypes binding of libdcd_b200.so (the C ABI declared in include/dcd_b200.h and include/dcd_b200_grad.h).
 
 There is no CPU fallback: if the library is missing or a tensor is not on a CUDA device the
 call raises.  The library is built in-tree by `python -m dcd_b200.build` (or
@@ -55,6 +55,14 @@ SIGNATURES = {
                                 + [c_void_p] * 8 + [c_size_t, c_void_p]),
 }
 
+# name -> (restype, argtypes); mirrors include/dcd_b200_grad.h (backward of the fused frame-epilogue entry points)
+GRAD_SIGNATURES = {
+    "dcd_dgde_frame_bwd": (c_int, [c_void_p] * 3 + [c_int64] + [c_int] * 6 + [c_void_p] * 4 + [c_int64, c_int, c_float, c_float, c_int, c_float]
+                           + [c_void_p] * 7),
+    "dcd_dgde_locate_solve_bwd": (c_int, [c_void_p] * 8 + [c_int64, c_int, c_float, c_float, c_int, c_float] + [c_void_p] * 8),
+    "dcd_gmw_ray_rescale_bwd": (c_int, [c_void_p] * 4 + [c_int64] + [c_void_p] * 4),
+}
+
 _lib = None
 
 
@@ -65,7 +73,7 @@ def load_library(path: str = LIB_PATH) -> ctypes.CDLL:
             "libdcd_b200.so is not built (%s missing): run `python -m dcd_b200.build`; "
             "dcd_b200 has no CPU or PyTorch fallback" % path)
     lib = ctypes.CDLL(path)
-    for name, (res, args) in SIGNATURES.items():
+    for name, (res, args) in list(SIGNATURES.items()) + list(GRAD_SIGNATURES.items()):
         fn = getattr(lib, name)          # AttributeError if the symbol is not exported
         fn.restype = res
         fn.argtypes = args

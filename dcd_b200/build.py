@@ -27,7 +27,8 @@ def _stale() -> bool:
     if not os.path.exists(LIB):
         return True
     t = os.path.getmtime(LIB)
-    deps = [os.path.join(CSRC, f) for f in os.listdir(CSRC)] + [os.path.join(HERE, "..", "include", "dcd_b200.h")]
+    inc = os.path.join(HERE, "..", "include")
+    deps = [os.path.join(CSRC, f) for f in os.listdir(CSRC)] + [os.path.join(inc, f) for f in os.listdir(inc)]
     return any(os.path.getmtime(d) > t for d in deps)
 
 

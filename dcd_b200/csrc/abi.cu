@@ -1,6 +1,7 @@
 // extern "C" entry points of libdcd_b200.so: argument validation, workspace carving, kernel launches.
-// See include/dcd_b200.h for the contract of every function.
+// See include/dcd_b200.h and include/dcd_b200_grad.h for the contract of every function.
 #include "gmw_mlp.cuh"
+#include "../../include/dcd_b200_grad.h"
 
 namespace dcd {
 int launch_edge_solve_fwd(const float*, const float*, const float*, const float*, int64_t, int, float, float, int,
@@ -32,6 +33,13 @@ int launch_dgde_locate_bwd(const float*, const float*, const float*, const float
 int launch_dgde_depth_ensemble_bwd(const float*, const float*, const float*, const float*, const float*, const float*, const float*,
                                    int64_t, float, float, float, float, const float*, const float*, const float*, const float*, float*,
                                    float*, float*, float*, float*, float*, cudaStream_t);
+int launch_dgde_frame_bwd(const float*, const int64_t*, const int32_t*, int64_t, int, int, int, int, int, int, const float*, const float*,
+                          const float*, int64_t, int, float, float, int, float, const float*, const float*, const float*, const float*,
+                          float*, float*, cudaStream_t);
+int launch_dgde_locate_solve_bwd(const float*, const float*, const float*, const float*, const float*, const float*, const float*, int64_t,
+                                 int, float, float, int, float, const float*, const float*, float*, float*, float*, float*, float*,
+                                 cudaStream_t);
+int launch_gmw_ray_rescale_bwd(const float*, const float*, const float*, const float*, int64_t, float*, float*, float*, cudaStream_t);
 size_t gmw_transport_workspace_bytes(int64_t N, int E);
 int launch_gmw_transport_fwd(const float*, const float*, int64_t, int, float, float, int, float*, float*, float*, float*, void*,
                              cudaStream_t);
@@ -248,6 +256,53 @@ int dcd_gmw_ray_rescale_fwd(const float* raw_location, const float* pred_depth, 
     if (N == 0) return DCD_OK;
     if (!raw_location || !pred_depth || !dim || !pred_location) return DCD_E_INVALID;
     return launch_gmw_ray_rescale(raw_location, pred_depth, dim, N, pred_location, (cudaStream_t)stream);
+}
+
+int dcd_dgde_frame_bwd(const float* feature_maps, const int64_t* index, const int32_t* batch_idx, int64_t B, int C, int H, int W,
+                       int ch_kpts2d, int ch_kpts3d, int ch_offset3d, const float* rot, const float* K, const float* pad,
+                       const float* dims, int64_t N, int n, float lo, float hi, int flags, float down_ratio, const float* grad_depth,
+                       const float* grad_locations, const float* grad_kpts_img, const float* grad_kps3d, float* grad_maps,
+                       float* grad_dims, void* stream) {
+    if (N < 0 || B < 1 || C < 1 || H < 1 || W < 1 || bad_n(n)) return DCD_E_INVALID;
+    if (ch_kpts2d < 0 || ch_kpts2d + 2 * n > C || ch_kpts3d < 0 || ch_kpts3d + 3 * n > C || ch_offset3d < 0 || ch_offset3d + 2 > C)
+        return DCD_E_INVALID;
+    const int lo_[3] = {ch_kpts2d, ch_kpts3d, ch_offset3d}, hi_[3] = {ch_kpts2d + 2 * n, ch_kpts3d + 3 * n, ch_offset3d + 2};
+    for (int a = 0; a < 3; ++a)                              // each channel's gradient is written by one group
+        for (int b = a + 1; b < 3; ++b)
+            if (lo_[a] < hi_[b] && lo_[b] < hi_[a]) return DCD_E_INVALID;
+    if (N == 0) return DCD_OK;
+    if (!grad_depth && !grad_locations && !grad_kpts_img && !grad_kps3d) return DCD_E_INVALID;
+    if (!feature_maps || !index || !rot || !K || !pad || !grad_maps) return DCD_E_INVALID;
+    if (grad_dims && !dims) return DCD_E_INVALID;
+    if (B > 1 && !batch_idx) return DCD_E_INVALID;
+    return launch_dgde_frame_bwd(feature_maps, index, batch_idx, B, C, H, W, ch_kpts2d, ch_kpts3d, ch_offset3d, rot, K, pad, N, n, lo, hi,
+                                 flags, down_ratio, grad_depth, grad_locations, grad_kpts_img, grad_kps3d, grad_maps, grad_dims,
+                                 (cudaStream_t)stream);
+}
+
+int dcd_dgde_locate_solve_bwd(const float* kpts_off, const float* kps3d, const float* rot, const float* K, const float* points,
+                              const float* offsets, const float* pad, const float* dims, int64_t N, int n, float lo, float hi, int flags,
+                              float down_ratio, const float* grad_depth, const float* grad_locations, float* grad_kpts_off,
+                              float* grad_kps3d, float* grad_offsets, float* grad_points, float* grad_dims, void* stream) {
+    if (N < 0 || bad_n(n)) return DCD_E_INVALID;
+    if (N == 0) return DCD_OK;
+    if (!grad_depth && !grad_locations) return DCD_E_INVALID;
+    if (!grad_kpts_off && !grad_kps3d && !grad_offsets && !grad_points && !grad_dims) return DCD_E_INVALID;
+    if (!kpts_off || !kps3d || !rot || !K || !points || !offsets || !pad) return DCD_E_INVALID;
+    if (grad_dims && !dims) return DCD_E_INVALID;
+    return launch_dgde_locate_solve_bwd(kpts_off, kps3d, rot, K, points, offsets, pad, N, n, lo, hi, flags, down_ratio, grad_depth,
+                                        grad_locations, grad_kpts_off, grad_kps3d, grad_offsets, grad_points, grad_dims,
+                                        (cudaStream_t)stream);
+}
+
+int dcd_gmw_ray_rescale_bwd(const float* raw_location, const float* pred_depth, const float* dim, const float* grad_pred_location,
+                            int64_t N, float* grad_raw_location, float* grad_pred_depth, float* grad_dim, void* stream) {
+    if (N < 0) return DCD_E_INVALID;
+    if (N == 0) return DCD_OK;
+    if (!raw_location || !pred_depth || !dim || !grad_pred_location) return DCD_E_INVALID;
+    if (!grad_raw_location && !grad_pred_depth && !grad_dim) return DCD_E_INVALID;
+    return launch_gmw_ray_rescale_bwd(raw_location, pred_depth, dim, grad_pred_location, N, grad_raw_location, grad_pred_depth, grad_dim,
+                                      (cudaStream_t)stream);
 }
 
 size_t dcd_gmw_transport_workspace_bytes(int64_t N, int n) {

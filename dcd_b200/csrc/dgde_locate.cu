@@ -624,16 +624,22 @@ poi_scatter_kernel(const float* __restrict__ grad_out, const int64_t* __restrict
 
 }  // namespace
 
+// pass 1 of a dense map gradient: poi_fill_zero_kernel over `total` floats
+int fill_zero(float* out, int64_t total, cudaStream_t st) {
+    const int64_t cap = (int64_t)device_sm_count() * 8;
+    const int64_t want = (total / 4 + 255) / 256;
+    poi_fill_zero_kernel<<<(unsigned)(want < cap ? (want > 0 ? want : 1) : cap), 256, 0, st>>>(
+        out, total, (reinterpret_cast<uintptr_t>(out) & 15) == 0);
+    DCD_CHECK_LAUNCH();
+    return DCD_OK;
+}
+
 int launch_poi_gather_bwd(const float* grad_out, const int64_t* index, int64_t B, int64_t Kp, int C, int64_t HW, float* grad_maps,
                           cudaStream_t st) {
-    const int64_t total = B * C * HW;
+    const int rc = fill_zero(grad_maps, B * C * HW, st);
+    if (rc != DCD_OK || Kp == 0) return rc;
     const int64_t cap = (int64_t)device_sm_count() * 8;
-    int64_t want = (total / 4 + 255) / 256;
-    poi_fill_zero_kernel<<<(unsigned)(want < cap ? (want > 0 ? want : 1) : cap), 256, 0, st>>>(
-        grad_maps, total, (reinterpret_cast<uintptr_t>(grad_maps) & 15) == 0);
-    DCD_CHECK_LAUNCH();
-    if (Kp == 0) return DCD_OK;
-    want = B * Kp;
+    const int64_t want = B * Kp;
     poi_scatter_kernel<<<(unsigned)(want < cap * 4 ? want : cap * 4), 128, 0, st>>>(grad_out, index, B, (int)Kp, C, HW, grad_maps);
     DCD_CHECK_LAUNCH();
     return DCD_OK;
@@ -642,6 +648,309 @@ int launch_poi_gather_bwd(const float* grad_out, const int64_t* index, int64_t B
 int launch_poi_gather(const float* feat, const int64_t* index, int64_t B, int64_t Kp, int C, int64_t HW, float* out, cudaStream_t st) {
     const int64_t total = B * Kp * C;
     poi_gather_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(feat, index, B, Kp, C, HW, out);
+    DCD_CHECK_LAUNCH();
+    return DCD_OK;
+}
+
+}  // namespace dcd
+
+// ---------------------------------------------------------------------------------------------
+// Backward of the fused frame epilogue: dgde_frame_warp_kernel (from the regression map) and the solve form of
+// dgde_locate_warp_kernel (from gathered channels), sharing one per-object routine; and of the GMW ray rescale.
+// ---------------------------------------------------------------------------------------------
+namespace dcd {
+namespace {
+
+constexpr int FB_THREADS = 128;
+
+// What the forward read for one object: keypoint offsets (t, u/v), template points (t, X/Y/Z), the sub-pixel offset and
+// the heat-map peak, either from the map column at the object's position ...
+struct MapObject {
+    const float* base;
+    int64_t HW;
+    int ch_k2, ch_k3, ch_off;
+    float px, py;
+    __device__ float off(int t, int c) const { return __ldg(base + (int64_t)(ch_k2 + 2 * t + c) * HW); }
+    __device__ float k3(int t, int c) const { return __ldg(base + (int64_t)(ch_k3 + 3 * t + c) * HW); }
+    __device__ float ofs(int c) const { return __ldg(base + (int64_t)(ch_off + c) * HW); }
+    __device__ float pt(int c) const { return c == 0 ? px : py; }
+};
+
+// ... or from the gathered [N,n,2] / [N,n,3] / [N,2] arrays of dcd_dgde_locate_fwd.
+struct ArrayObject {
+    const float *kpts_off, *kps3d, *points, *offsets;
+    int64_t obj;
+    int n;
+    __device__ float off(int t, int c) const { return __ldg(kpts_off + (obj * n + t) * 2 + c); }
+    __device__ float k3(int t, int c) const { return __ldg(kps3d + (obj * n + t) * 3 + c); }
+    __device__ float ofs(int c) const { return __ldg(offsets + obj * 2 + c); }
+    __device__ float pt(int c) const { return __ldg(points + obj * 2 + c); }
+};
+
+struct FrameGrads {            // upstream gradients, each NULL when that output passes none
+    const float *depth, *loc, *kimg, *k3;
+};
+
+// One object's gradient w.r.t. what the forward read, CTA-wide, into col_s [5n + 2] in channel order: keypoint offsets
+// [2n] (u, v per keypoint), template points [3n], sub-pixel offset [2].  Sum of
+//   the location (dgde_locate_bwd_kernel's operations, on the depth recomputed bit for bit like the forward's lane-strided
+//   sum): d/d(centre) and d/d(depth);
+//   the mean over all E edges: dL/d(depth) / E on every edge, through keypoint_edge_grad (edge_solve_bwd_kernel's gather)
+//   -> d/d(v_img), d/d(X, Y, Z); the u column of the solve is exactly 0;
+//   the upstream gradients of the image keypoints and template points;
+// then through (kpts_off + centre) * down_ratio - pad: the keypoint channels get down_ratio x d/d(kimg), the sub-pixel
+// offset the sum of those over the keypoints (ascending) plus the location's term.  No gradient to rot, K or pad.
+// Ends with a barrier: col_s is complete, kp_s / sc_s may be reused.
+template <class Src>
+__device__ void frame_object_bwd(const Src& src, int64_t obj, int n, float lo, float hi, int flags, float down_ratio,
+                                 const float* __restrict__ rot, const float* __restrict__ K, const float* __restrict__ pad,
+                                 const FrameGrads& up, float4* kp_s, float* col_s, float* sc_s) {
+    constexpr int NWARP = FB_THREADS / 32;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int E = n * (n - 1) / 2;
+    const float* Ko = K + obj * 12;
+    const float f_u = __ldg(Ko + 0), c_u = __ldg(Ko + 2), f_v = __ldg(Ko + 5), c_v = __ldg(Ko + 6);
+    const float cx = __fadd_rn(src.pt(0), src.ofs(0)), cyy = __fadd_rn(src.pt(1), src.ofs(1));
+    const float pad_u = __ldg(pad + obj * 2), pad_v = __ldg(pad + obj * 2 + 1);
+    const bool normalise = (flags & DCD_NORMALISE_2D) != 0;
+    const bool solve = up.depth != nullptr || up.loc != nullptr;
+    const float r = __ldg(rot + obj);
+    const float sn = sinf(r), cs = cosf(r);
+    if (solve) {
+        for (int t = tid; t < n; t += FB_THREADS) {
+            const float v_img = __fsub_rn(__fmul_rn(__fadd_rn(src.off(t, 1), cyy), down_ratio), pad_v);
+            kp_s[t] = keypoint_terms(v_img, src.k3(t, 0), src.k3(t, 1), src.k3(t, 2), sn, cs, normalise, c_v, f_v);
+        }
+        __syncthreads();
+        if (warp == 0) {
+            float g_u = 0.f, g_v = 0.f, g = up.depth != nullptr ? __ldg(up.depth + obj) : 0.f;
+            if (up.loc != nullptr) {
+                const float b3 = (flags & DCD_SUB_B3) ? __ldg(Ko + 11) : 0.f;
+                float acc = 0.f;
+                for (int e = lane; e < E; e += 32) {
+                    int i, j;
+                    decode_edge(e, n, i, j);
+                    acc += edge_depth(kp_s[i], kp_s[j], lo, hi, b3);
+                }
+                acc = warp_sum(acc);
+                const float depth = __fdiv_rn(acc, (float)E);
+                const float gx = __ldg(up.loc + obj * 3), gy = __ldg(up.loc + obj * 3 + 1), gz = __ldg(up.loc + obj * 3 + 2);
+                const float ax = __fdiv_rn(gx, f_u), ay = __fdiv_rn(gy, f_v);
+                g_u = __fmul_rn(__fmul_rn(ax, depth), down_ratio);
+                g_v = __fmul_rn(__fmul_rn(ay, depth), down_ratio);
+                const float u = __fsub_rn(__fmul_rn(cx, down_ratio), pad_u), v = __fsub_rn(__fmul_rn(cyy, down_ratio), pad_v);
+                const float gd = __fadd_rn(__fadd_rn(__fmul_rn(ax, __fsub_rn(u, c_u)), __fmul_rn(ay, __fsub_rn(v, c_v))), gz);
+                g = up.depth != nullptr ? __fadd_rn(g, gd) : gd;
+            }
+            if (lane == 0) {
+                sc_s[0] = g_u;
+                sc_s[1] = g_v;
+                sc_s[2] = __fdiv_rn(g, (float)E);
+            }
+        }
+        __syncthreads();
+    }
+    const float gm = solve ? sc_s[2] : 0.f;
+    float* col_k2 = col_s;
+    float* col_k3 = col_s + 2 * n;
+    for (int t = warp; t < n; t += NWARP) {
+        float g_vi = 0.f, gX = 0.f, gY = 0.f, gZ = 0.f;
+        if (solve) {
+            const float4 me = kp_s[t];
+            float gH, gV;
+            keypoint_edge_grad(kp_s, me, t, n, lane, lo, hi, [&](int) { return gm; }, gH, gV);
+            const float gv = gV + gH * me.w;          // d/dv: V and the v*C term of H
+            const float gC = gH * me.x;               // d/dC
+            g_vi = normalise ? __fdiv_rn(gv, f_v) : gv;
+            gX = gC * sn;
+            gY = gH;
+            gZ = -gC * cs;
+        }
+        if (lane == 0) {
+            const int64_t kt = obj * n + t;
+            float g_ui = 0.f;
+            if (up.kimg != nullptr) {
+                g_ui = __ldg(up.kimg + kt * 2);
+                g_vi = __fadd_rn(g_vi, __ldg(up.kimg + kt * 2 + 1));
+            }
+            if (up.k3 != nullptr) {
+                gX = __fadd_rn(gX, __ldg(up.k3 + kt * 3));
+                gY = __fadd_rn(gY, __ldg(up.k3 + kt * 3 + 1));
+                gZ = __fadd_rn(gZ, __ldg(up.k3 + kt * 3 + 2));
+            }
+            col_k2[2 * t] = __fmul_rn(g_ui, down_ratio);
+            col_k2[2 * t + 1] = __fmul_rn(g_vi, down_ratio);
+            col_k3[3 * t] = gX;
+            col_k3[3 * t + 1] = gY;
+            col_k3[3 * t + 2] = gZ;
+        }
+    }
+    __syncthreads();
+    if (tid < 2) {
+        float s = 0.f;
+        for (int t = 0; t < n; ++t) s = __fadd_rn(s, col_k2[2 * t + tid]);
+        col_s[5 * n + tid] = solve ? __fadd_rn(s, sc_s[tid]) : s;
+    }
+    __syncthreads();
+}
+
+// dL/d(dims) of the `+ h / 2` on the location's y: only the h column is non-zero.
+__device__ __forceinline__ void dims_grad(const float* __restrict__ grad_loc, int64_t obj, float* __restrict__ grad_dims) {
+    grad_dims[obj * 3] = 0.f;
+    grad_dims[obj * 3 + 1] = grad_loc != nullptr ? __fmul_rn(__ldg(grad_loc + obj * 3 + 1), 0.5f) : 0.f;
+    grad_dims[obj * 3 + 2] = 0.f;
+}
+
+// Backward of dgde_frame_warp_kernel<GMW = false>, pass 2 (pass 1 is poi_fill_zero_kernel over the map gradient): one CTA per
+// detection slot, with the conventions of poi_scatter_kernel.  A slot writes its map column only if no earlier slot of the
+// same image holds the same position; it then runs frame_object_bwd for every slot >= its own at that position, in
+// ascending slot order (found 32 slots at a time by a ballot, so the number of duplicates is not bounded), sums the columns
+// in that order and writes each of the 5n + 2 channels once: deterministic, no atomics.  A position outside [0, HW)
+// passes no gradient to the map; grad_dims is written for every slot.
+__global__ void __launch_bounds__(FB_THREADS)
+dgde_frame_bwd_kernel(const float* __restrict__ fmap, const int64_t* __restrict__ index, const int32_t* __restrict__ batch_idx,
+                      int C, int H, int W, int ch_k2, int ch_k3, int ch_off, const float* __restrict__ rot, const float* __restrict__ K,
+                      const float* __restrict__ pad, int64_t N, int n, float lo, float hi, int flags, float down_ratio, FrameGrads up,
+                      float* __restrict__ grad_maps, float* __restrict__ grad_dims) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    float4* kp_s = reinterpret_cast<float4*>(smem_raw);                       // [n]
+    float* col_s = reinterpret_cast<float*>(kp_s + n);                        // [5n + 2]
+    float* acc_s = col_s + 5 * n + 2;                                         // [5n + 2]
+    __shared__ float sc_s[4];
+    __shared__ int64_t list_s[32];
+    __shared__ int count_s;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int G = 5 * n + 2;
+    const int64_t HW = (int64_t)H * W;
+    for (int64_t slot = blockIdx.x; slot < N; slot += gridDim.x) {
+        if (grad_dims != nullptr && tid == 0) dims_grad(up.loc, slot, grad_dims);
+        const int64_t p = index[slot];
+        if (p < 0 || p >= HW) continue;                                   // uniform over the CTA
+        const int b = batch_idx != nullptr ? batch_idx[slot] : 0;
+        bool earlier = false;
+        for (int64_t j = tid; j < slot; j += FB_THREADS) earlier |= index[j] == p && (batch_idx == nullptr || batch_idx[j] == b);
+        if (__syncthreads_or(earlier)) continue;
+        const MapObject src{fmap + (int64_t)b * C * HW + p, HW, ch_k2, ch_k3, ch_off, (float)(p % W), (float)(p / W)};
+        for (int c = tid; c < G; c += FB_THREADS) acc_s[c] = 0.f;          // each thread owns the same channels throughout
+        for (int64_t j0 = slot; j0 < N; j0 += 32) {
+            if (warp == 0) {                                              // ascending list of this chunk's slots at (b, p)
+                const int64_t j = j0 + lane;
+                const bool m = j < N && index[j] == p && (batch_idx == nullptr || batch_idx[j] == b);
+                const unsigned bal = __ballot_sync(0xffffffffu, m);
+                if (m) list_s[__popc(bal & ((1u << lane) - 1u))] = j;
+                if (lane == 0) count_s = __popc(bal);
+            }
+            __syncthreads();
+            const int cnt = count_s;
+            for (int i = 0; i < cnt; ++i) {
+                frame_object_bwd(src, list_s[i], n, lo, hi, flags, down_ratio, rot, K, pad, up, kp_s, col_s, sc_s);
+                for (int c = tid; c < G; c += FB_THREADS) acc_s[c] += col_s[c];
+                __syncthreads();                                          // col_s is rewritten by the next slot
+            }
+            __syncthreads();                                              // list_s / count_s are rebuilt for the next chunk
+        }
+        float* gb = grad_maps + (int64_t)b * C * HW + p;
+        for (int c = tid; c < G; c += FB_THREADS) {
+            const int ch = c < 2 * n ? ch_k2 + c : (c < 5 * n ? ch_k3 + c - 2 * n : ch_off + c - 5 * n);
+            gb[(int64_t)ch * HW] = acc_s[c];
+        }
+    }
+}
+
+// Backward of the solve form of dgde_locate_warp_kernel: one CTA per object, frame_object_bwd on the gathered arrays.
+__global__ void __launch_bounds__(FB_THREADS)
+dgde_locate_solve_bwd_kernel(const float* __restrict__ kpts_off, const float* __restrict__ kps3d, const float* __restrict__ rot,
+                             const float* __restrict__ K, const float* __restrict__ points, const float* __restrict__ offsets,
+                             const float* __restrict__ pad, int64_t N, int n, float lo, float hi, int flags, float down_ratio,
+                             FrameGrads up, float* __restrict__ grad_kpts_off, float* __restrict__ grad_kps3d,
+                             float* __restrict__ grad_offsets, float* __restrict__ grad_points, float* __restrict__ grad_dims) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    float4* kp_s = reinterpret_cast<float4*>(smem_raw);                       // [n]
+    float* col_s = reinterpret_cast<float*>(kp_s + n);                        // [5n + 2]
+    __shared__ float sc_s[4];
+    const int tid = threadIdx.x;
+    for (int64_t obj = blockIdx.x; obj < N; obj += gridDim.x) {
+        frame_object_bwd(ArrayObject{kpts_off, kps3d, points, offsets, obj, n}, obj, n, lo, hi, flags, down_ratio, rot, K, pad, up,
+                         kp_s, col_s, sc_s);
+        if (grad_kpts_off != nullptr)
+            for (int c = tid; c < 2 * n; c += FB_THREADS) grad_kpts_off[obj * 2 * n + c] = col_s[c];
+        if (grad_kps3d != nullptr)
+            for (int c = tid; c < 3 * n; c += FB_THREADS) grad_kps3d[obj * 3 * n + c] = col_s[2 * n + c];
+        if (tid < 2) {
+            if (grad_offsets != nullptr) grad_offsets[obj * 2 + tid] = col_s[5 * n + tid];
+            if (grad_points != nullptr) grad_points[obj * 2 + tid] = col_s[5 * n + tid];
+        }
+        if (grad_dims != nullptr && tid == 0) dims_grad(up.loc, obj, grad_dims);
+        __syncthreads();                                                  // col_s is rewritten by the next object
+    }
+}
+
+// Backward of gmw_ray_rescale_kernel in the order torch's autograd forms it for GMW/main.py:542-547:
+//   scale = z_gmw / z;  out = scale * (x, y - h/2, z) + (0, h/2, 0)
+//   d/dscale = g0 x + g1 (y - h/2) + g2 z;  d/dz = scale g2 - d/dscale ((z_gmw / z) / z);  d/dz_gmw = d/dscale / z;
+//   d/dh = (g1 - scale g1) / 2 (the h of dim[:, 0]; the other columns exactly 0).
+__global__ void __launch_bounds__(256)
+gmw_ray_rescale_bwd_kernel(const float* __restrict__ raw_location, const float* __restrict__ pred_depth, const float* __restrict__ dim,
+                           const float* __restrict__ grad_out, int64_t N, float* __restrict__ grad_raw, float* __restrict__ grad_depth,
+                           float* __restrict__ grad_dim) {
+    const int64_t o = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (o >= N) return;
+    const float x = __ldg(raw_location + o * 3), y = __ldg(raw_location + o * 3 + 1), z = __ldg(raw_location + o * 3 + 2);
+    const float zg = __ldg(pred_depth + o), h = __ldg(dim + o * 3);
+    const float g0 = __ldg(grad_out + o * 3), g1 = __ldg(grad_out + o * 3 + 1), g2 = __ldg(grad_out + o * 3 + 2);
+    const float scale = __fdiv_rn(zg, z);
+    const float hh = __fmul_rn(h, 0.5f);
+    const float gs = __fadd_rn(__fadd_rn(__fmul_rn(g0, x), __fmul_rn(g1, __fsub_rn(y, hh))), __fmul_rn(g2, z));
+    if (grad_raw != nullptr) {
+        grad_raw[o * 3] = __fmul_rn(scale, g0);
+        grad_raw[o * 3 + 1] = __fmul_rn(scale, g1);
+        grad_raw[o * 3 + 2] = __fsub_rn(__fmul_rn(scale, g2), __fmul_rn(gs, __fdiv_rn(scale, z)));
+    }
+    if (grad_depth != nullptr) grad_depth[o] = __fdiv_rn(gs, z);
+    if (grad_dim != nullptr) {
+        grad_dim[o * 3] = __fmul_rn(__fsub_rn(g1, __fmul_rn(scale, g1)), 0.5f);
+        grad_dim[o * 3 + 1] = 0.f;
+        grad_dim[o * 3 + 2] = 0.f;
+    }
+}
+
+int frame_bwd_grid(int64_t N) {
+    const int64_t cap = (int64_t)device_sm_count() * 16;
+    return (int)(N < cap ? N : cap);
+}
+
+}  // namespace
+
+int launch_dgde_frame_bwd(const float* fmap, const int64_t* index, const int32_t* batch_idx, int64_t B, int C, int H, int W, int ch_k2,
+                          int ch_k3, int ch_off, const float* rot, const float* K, const float* pad, int64_t N, int n, float lo, float hi,
+                          int flags, float down_ratio, const float* g_depth, const float* g_loc, const float* g_kimg, const float* g_k3,
+                          float* grad_maps, float* grad_dims, cudaStream_t st) {
+    const size_t smem = (size_t)n * sizeof(float4) + (size_t)2 * (5 * n + 2) * sizeof(float);
+    const int rc = fill_zero(grad_maps, B * C * (int64_t)H * W, st);
+    if (rc != DCD_OK) return rc;
+    dgde_frame_bwd_kernel<<<frame_bwd_grid(N), FB_THREADS, smem, st>>>(fmap, index, batch_idx, C, H, W, ch_k2, ch_k3, ch_off, rot, K, pad,
+                                                                        N, n, lo, hi, flags, down_ratio,
+                                                                        FrameGrads{g_depth, g_loc, g_kimg, g_k3}, grad_maps, grad_dims);
+    DCD_CHECK_LAUNCH();
+    return DCD_OK;
+}
+
+int launch_dgde_locate_solve_bwd(const float* kpts_off, const float* kps3d, const float* rot, const float* K, const float* points,
+                                 const float* offsets, const float* pad, int64_t N, int n, float lo, float hi, int flags,
+                                 float down_ratio, const float* g_depth, const float* g_loc, float* grad_kpts_off, float* grad_kps3d,
+                                 float* grad_offsets, float* grad_points, float* grad_dims, cudaStream_t st) {
+    const size_t smem = (size_t)n * sizeof(float4) + (size_t)(5 * n + 2) * sizeof(float);
+    dgde_locate_solve_bwd_kernel<<<frame_bwd_grid(N), FB_THREADS, smem, st>>>(
+        kpts_off, kps3d, rot, K, points, offsets, pad, N, n, lo, hi, flags, down_ratio, FrameGrads{g_depth, g_loc, nullptr, nullptr},
+        grad_kpts_off, grad_kps3d, grad_offsets, grad_points, grad_dims);
+    DCD_CHECK_LAUNCH();
+    return DCD_OK;
+}
+
+int launch_gmw_ray_rescale_bwd(const float* raw_location, const float* pred_depth, const float* dim, const float* grad_out, int64_t N,
+                               float* grad_raw, float* grad_depth, float* grad_dim, cudaStream_t st) {
+    gmw_ray_rescale_bwd_kernel<<<(unsigned)((N + 255) / 256), 256, 0, st>>>(raw_location, pred_depth, dim, grad_out, N, grad_raw,
+                                                                             grad_depth, grad_dim);
     DCD_CHECK_LAUNCH();
     return DCD_OK;
 }

@@ -771,34 +771,11 @@ edge_solve_bwd_kernel(const float* __restrict__ kps, const float* __restrict__ k
         const float* gd = (idx == nullptr && grad_depth != nullptr) ? grad_depth + obj * (int64_t)E : nullptr;
         for (int kk = warp; kk < n; kk += NWARP) {
             const float4 me = kp_s[kk];
-            float gH = 0.f, gV = 0.f;
-            for (int m = lane; m < n; m += 32) {
-                if (m == kk) continue;
-                const int i = min(kk, m), j = max(kk, m);
-                const int e = row_offset(i, n) + j - i - 1;
-                float g;
-                if (idx != nullptr) g = g_s[e];
-                else g = (gd != nullptr ? __ldg(gd + e) : 0.f) + gm;
-                if (g == 0.f) continue;
-                const float4 a = (kk == i) ? me : kp_s[m];
-                const float4 b = (kk == i) ? kp_s[m] : me;
-                const float H = __fadd_rn(__fsub_rn(a.y, b.y), __fsub_rn(a.z, b.z));
-                const float V = __fsub_rn(a.x, b.x);
-                const float aV = fabsf(V);
-                const float Vc = fmaxf(aV, 1e-10f);
-                const float x = __fdiv_rn(fabsf(H), Vc);
-                const bool pass = (x >= lo) && (fmaxf(x, lo) <= hi);
-                if (!pass) continue;
-                const float sH = (H > 0.f) ? 1.f : ((H < 0.f) ? -1.f : 0.f);
-                const float sV = (V > 0.f) ? 1.f : ((V < 0.f) ? -1.f : 0.f);
-                const float dH = g * sH / Vc;
-                const float dV = (aV >= 1e-10f) ? -g * (x / Vc) * sV : 0.f;
-                const float sgn = (kk == i) ? 1.f : -1.f;
-                gH += sgn * dH;
-                gV += sgn * dV;
-            }
-            gH = warp_sum(gH);
-            gV = warp_sum(gV);
+            float gH, gV;
+            keypoint_edge_grad(kp_s, me, kk, n, lane, lo, hi, [&](int e) {
+                if (idx != nullptr) return g_s[e];
+                return (gd != nullptr ? __ldg(gd + e) : 0.f) + gm;
+            }, gH, gV);
             if (lane == 0) {
                 const float gv = gV + gH * me.w;          // d/dv: V and the v*C term of H
                 const float gC = gH * me.x;               // d/dC

@@ -39,8 +39,7 @@ def _num_edges(n: int) -> int:
 
 
 def _inference_only(name: str, *tensors) -> None:
-    """The inference-form frame-epilogue ops (compute_pairs_kpts_depth, frame_depths_from_map, ray_rescale) have no
-    backward: fail loudly instead of silently cutting the autograd graph."""
+    """Inference-only ops (refine_detections) have no backward: fail loudly instead of silently cutting the autograd graph."""
     if torch.is_grad_enabled() and any(t is not None and torch.is_tensor(t) and t.requires_grad for t in tensors):
         raise RuntimeError("dcd_b200.%s is inference-only (no backward is implemented): call it under torch.no_grad() "
                            "or detach its inputs" % name)
@@ -233,6 +232,52 @@ def _pad_per_object(pad_size, batch_idxs, N, dev):
     return f32c(pad)
 
 
+class _LocateSolve(torch.autograd.Function):
+    """compute_pairs_kpts_depth through dcd_dgde_locate_fwd (solve form); backward dcd_dgde_locate_solve_bwd -> keypoint offsets,
+    template points, points (when floating), sub-pixel offsets, dims (h column)."""
+
+    @staticmethod
+    def forward(ctx, off, k3, pts, ofs, d3, rot, K, pad, want_loc):
+        depth, loc = _locate_solve_fwd(off, k3, pts, ofs, d3, rot, K, pad, want_loc)
+        ctx.save_for_backward(off, k3, pts, ofs, d3, rot, K, pad)
+        ctx.set_materialize_grads(False)
+        return (depth, loc) if want_loc else depth
+
+    @staticmethod
+    def backward(ctx, g_depth, g_loc=None):
+        off, k3, pts, ofs, d3, rot, K, pad = ctx.saved_tensors
+        need = ctx.needs_input_grad
+        outs = [torch.empty_like(t) if t is not None and need[i] else None for i, t in ((0, off), (1, k3), (3, ofs), (2, pts), (4, d3))]
+        N, n = off.shape[0], off.shape[1]
+        if g_depth is None and g_loc is None or all(o is None for o in outs):
+            return (None,) * 9
+        if N:
+            lo, hi = DGDE_CLAMP
+            gd, gl = (f32c(g) if g is not None else None for g in (g_depth, g_loc))
+            check(_lib.lib().dcd_dgde_locate_solve_bwd(ptr(off), ptr(k3), ptr(rot), ptr(K), ptr(pts), ptr(ofs), ptr(pad), ptr(d3), N, n,
+                                                       lo, hi, FLAG_NORMALISE_2D | FLAG_SUB_B3, DOWN_RATIO, ptr(gd), ptr(gl),
+                                                       *(ptr(o) for o in outs), stream_ptr()), "dcd_dgde_locate_solve_bwd")
+        g_off, g_k3, g_ofs, g_pts, g_d3 = outs
+        return g_off, g_k3, g_pts, g_ofs, g_d3, None, None, None, None
+
+
+def _locate_solve_fwd(off, k3, pts, ofs, d3, rot, K, pad, want_loc):
+    N, n = off.shape[0], off.shape[1]
+    depth = torch.empty((N,), dtype=torch.float32, device=off.device)
+    loc = torch.empty((N, 3), dtype=torch.float32, device=off.device) if want_loc else None
+    lo, hi = DGDE_CLAMP
+    if N:
+        check(_lib.lib().dcd_dgde_locate_fwd(ptr(off), ptr(k3), ptr(rot), ptr(K), ptr(pts), ptr(ofs), ptr(pad),
+                                             ptr(d3) if d3 is not None else 0, 0, N, n, lo, hi,
+                                             FLAG_NORMALISE_2D | FLAG_SUB_B3, DOWN_RATIO, ptr(depth),
+                                             ptr(loc) if loc is not None else 0, stream_ptr()), "dcd_dgde_locate_fwd")
+    return depth, loc
+
+
+def _needs_grad(*tensors) -> bool:
+    return torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in tensors)
+
+
 def compute_pairs_kpts_depth(pred_extra_kpts_2d, pred_bbox_points, pred_offset_3D, pad_size, pred_extra_kpts_3d, pred_rots, P,
                              batch_idxs=None, dims=None, return_locations: bool = False):
     """Fused form of PostProcessor.compute_pairs_kpts_depth (DGDE/model/head/detector_infer.py:215-227): the image-space
@@ -240,10 +285,11 @@ def compute_pairs_kpts_depth(pred_extra_kpts_2d, pred_bbox_points, pred_offset_3
     averaged -> depth [N].  With `return_locations` also the object's 3D location (decode_location_flatten,
     anno_encoder.py:147-161, and `+ h / 2` on y when `dims` [N,3] is given, detector_infer.py:186-188) from the same launch.
     P: the image's 3x4 projection matrix (or one per object), pad_size: [2], [1,2], or [B,2] with batch_idxs.
-    Inference-only (no backward; raises when an input requires grad)."""
+    Differentiable (dcd_dgde_locate_solve_bwd) w.r.t. pred_extra_kpts_2d (the u column's gradient is exactly 0),
+    pred_extra_kpts_3d, pred_offset_3D, pred_bbox_points when floating, and dims (h column); pred_rots, P and pad_size
+    receive none (raise when they require grad).  float64 inputs get float64 gradients (the arithmetic is FP32)."""
+    _constant_inputs("compute_pairs_kpts_depth", pred_rots=pred_rots, P=P, pad_size=pad_size)
     require_cuda(pred_extra_kpts_2d, pred_extra_kpts_3d, pred_rots, pred_bbox_points, pred_offset_3D)
-    _inference_only("compute_pairs_kpts_depth", pred_extra_kpts_2d, pred_extra_kpts_3d, pred_rots, pred_bbox_points,
-                    pred_offset_3D, dims)
     off, k3 = f32c(pred_extra_kpts_2d), f32c(pred_extra_kpts_3d)
     rot = f32c(pred_rots).reshape(-1)
     N, n = off.shape[0], off.shape[1]
@@ -253,14 +299,9 @@ def compute_pairs_kpts_depth(pred_extra_kpts_2d, pred_bbox_points, pred_offset_3
     pts, ofs = f32c(pred_bbox_points), f32c(pred_offset_3D)
     pad = _pad_per_object(pad_size, batch_idxs, N, dev)
     d3 = f32c(dims) if dims is not None else None
-    depth = torch.empty((N,), dtype=torch.float32, device=dev)
-    loc = torch.empty((N, 3), dtype=torch.float32, device=dev) if return_locations else None
-    lo, hi = DGDE_CLAMP
-    if N:
-        check(_lib.lib().dcd_dgde_locate_fwd(ptr(off), ptr(k3), ptr(rot), ptr(K), ptr(pts), ptr(ofs), ptr(pad),
-                                             ptr(d3) if d3 is not None else 0, 0, N, n, lo, hi,
-                                             FLAG_NORMALISE_2D | FLAG_SUB_B3, DOWN_RATIO, ptr(depth),
-                                             ptr(loc) if loc is not None else 0, stream_ptr()), "dcd_dgde_locate_fwd")
+    if _needs_grad(off, k3, pts, ofs, d3):
+        return _LocateSolve.apply(off, k3, pts, ofs, d3, rot, K, pad, return_locations)
+    depth, loc = _locate_solve_fwd(off, k3, pts, ofs, d3, rot, K, pad, return_locations)
     return (depth, loc) if return_locations else depth
 
 
@@ -293,20 +334,9 @@ def _frame_inputs(pred_regression, indexs, pred_rots, P, pad_size, batch_idxs, c
     return fm, idx, bi, rot, K, pad, ch
 
 
-def frame_depths_from_map(pred_regression, indexs, pred_rots, P, pad_size, dims=None, batch_idxs=None, n: int = 73,
-                          channels=None, return_keypoints: bool = False):
-    """POI gather + image keypoints + edge solve + mean + 3D location in ONE launch, reading the regression map itself
-    (detector_infer.py:107 select_point_of_interest, :133 / :216-219 channel slices, :215-227 compute_pairs_kpts_depth,
-    :186-188 decode_location_flatten): pred_regression [B,C,H,W], indexs [N] int64 heat-map positions y * W + x of the kept
-    detections (select_topk), pred_rots [N] decoded yaw, P the 3x4 calibration ([3,4], per image [B,3,4] with batch_idxs, or
-    per object), pad_size [2] / [B,2], dims [N,3] or None -> (depth [N], locations [N,3]) and, with return_keypoints, the
-    image-space 2D keypoints [N,n,2] and template points [N,n,3] that generate_infer_data dumps (:228-236).  Inference-only."""
-    require_cuda(pred_regression, indexs, pred_rots)
-    _inference_only("frame_depths_from_map", pred_regression, pred_rots, dims)
-    fm, idx, bi, rot, K, pad, ch = _frame_inputs(pred_regression, indexs, pred_rots, P, pad_size, batch_idxs, channels)
+def _frame_fwd(fm, idx, bi, rot, K, pad, d3, ch, n, return_keypoints):
     B, C, H, W = fm.shape
     N, dev = idx.shape[0], fm.device
-    d3 = f32c(dims) if dims is not None else None
     depth = torch.empty((N,), dtype=torch.float32, device=dev)
     loc = torch.empty((N, 3), dtype=torch.float32, device=dev)
     kimg = torch.empty((N, n, 2), dtype=torch.float32, device=dev) if return_keypoints else None
@@ -318,6 +348,59 @@ def frame_depths_from_map(pred_regression, indexs, pred_rots, P, pad_size, dims=
                                             FLAG_NORMALISE_2D | FLAG_SUB_B3, DOWN_RATIO, ptr(depth), ptr(loc), ptr(kimg), ptr(k3),
                                             stream_ptr()), "dcd_dgde_frame_fwd")
     return (depth, loc, kimg, k3) if return_keypoints else (depth, loc)
+
+
+class _FrameDepths(torch.autograd.Function):
+    """frame_depths_from_map through dcd_dgde_frame_fwd; backward dcd_dgde_frame_bwd -> the dense map gradient and dims (h
+    column).  An output the loss does not use passes no gradient."""
+
+    @staticmethod
+    def forward(ctx, fm, d3, idx, bi, rot, K, pad, ch, n, return_keypoints):
+        out = _frame_fwd(fm, idx, bi, rot, K, pad, d3, ch, n, return_keypoints)
+        ctx.save_for_backward(fm, d3, idx, bi, rot, K, pad)
+        ctx.cfg = (ch, n)
+        ctx.set_materialize_grads(False)
+        return out
+
+    @staticmethod
+    def backward(ctx, g_depth, g_loc, g_kimg=None, g_k3=None):
+        fm, d3, idx, bi, rot, K, pad = ctx.saved_tensors
+        ch, n = ctx.cfg
+        up = [f32c(g) if g is not None else None for g in (g_depth, g_loc, g_kimg, g_k3)]
+        if all(g is None for g in up):
+            return (None,) * 10
+        B, C, H, W = fm.shape
+        N = idx.shape[0]
+        g_map = torch.empty_like(fm) if N else torch.zeros_like(fm)
+        g_d3 = torch.empty_like(d3) if d3 is not None and ctx.needs_input_grad[1] else None
+        if N:
+            lo, hi = DGDE_CLAMP
+            check(_lib.lib().dcd_dgde_frame_bwd(ptr(fm), ptr(idx), ptr(bi), B, C, H, W, ch["extra_kpts_2d"], ch["extra_kpts_3d"],
+                                                ch["3d_offset"], ptr(rot), ptr(K), ptr(pad), ptr(d3), N, n, lo, hi,
+                                                FLAG_NORMALISE_2D | FLAG_SUB_B3, DOWN_RATIO, *(ptr(g) for g in up), ptr(g_map),
+                                                ptr(g_d3), stream_ptr()), "dcd_dgde_frame_bwd")
+        return (g_map if ctx.needs_input_grad[0] else None), g_d3, None, None, None, None, None, None, None, None
+
+
+def frame_depths_from_map(pred_regression, indexs, pred_rots, P, pad_size, dims=None, batch_idxs=None, n: int = 73,
+                          channels=None, return_keypoints: bool = False):
+    """POI gather + image keypoints + edge solve + mean + 3D location in ONE launch, reading the regression map itself
+    (detector_infer.py:107 select_point_of_interest, :133 / :216-219 channel slices, :215-227 compute_pairs_kpts_depth,
+    :186-188 decode_location_flatten): pred_regression [B,C,H,W], indexs [N] int64 heat-map positions y * W + x of the kept
+    detections (select_topk), pred_rots [N] decoded yaw, P the 3x4 calibration ([3,4], per image [B,3,4] with batch_idxs, or
+    per object), pad_size [2] / [B,2], dims [N,3] or None -> (depth [N], locations [N,3]) and, with return_keypoints, the
+    image-space 2D keypoints [N,n,2] and template points [N,n,3] that generate_infer_data dumps (:228-236).
+    Every output is differentiable w.r.t. pred_regression and dims (h column) (dcd_dgde_frame_bwd: one dense map gradient,
+    non-zero only in the three channel groups at the detections' positions; detections on one position summed in ascending
+    order; a position outside the map passes none).  pred_rots, P and pad_size receive no gradient (raise when they require
+    grad); float64 inputs get float64 gradients (the arithmetic is FP32).  The channel groups must not overlap."""
+    _constant_inputs("frame_depths_from_map", pred_rots=pred_rots, P=P, pad_size=pad_size)
+    require_cuda(pred_regression, indexs, pred_rots)
+    fm, idx, bi, rot, K, pad, ch = _frame_inputs(pred_regression, indexs, pred_rots, P, pad_size, batch_idxs, channels)
+    d3 = f32c(dims) if dims is not None else None
+    if _needs_grad(fm, d3):
+        return _FrameDepths.apply(fm, d3, idx, bi, rot, K, pad, ch, n, return_keypoints)
+    return _frame_fwd(fm, idx, bi, rot, K, pad, d3, ch, n, return_keypoints)
 
 
 class _LocateFlatten(torch.autograd.Function):
@@ -507,16 +590,44 @@ def depth_ensemble(pred_keypoints, pred_dimensions, P, keypoint_log_uncertainty,
             "scores": so.reshape(-1, 1) if sc is not None else None}
 
 
-def ray_rescale(raw_location, pred_depth, dim):
-    """GMW/main.py:542-547: detector location [N,3] moved along its viewing ray to the GMW depth (dim [N,3] = (h,w,l))."""
-    require_cuda(raw_location, pred_depth, dim)
-    _inference_only("ray_rescale", raw_location, pred_depth, dim)
-    rl, pd, dm = f32c(raw_location), f32c(pred_depth).reshape(-1), f32c(dim)
+class _RayRescale(torch.autograd.Function):
+    """dcd_gmw_ray_rescale_fwd; backward dcd_gmw_ray_rescale_bwd -> raw location, GMW depth, dim (h column)."""
+
+    @staticmethod
+    def forward(ctx, rl, pd, dm):
+        out = _ray_rescale_fwd(rl, pd, dm)
+        ctx.save_for_backward(rl, pd, dm)
+        ctx.set_materialize_grads(False)
+        return out
+
+    @staticmethod
+    def backward(ctx, g_out):
+        if g_out is None:
+            return None, None, None
+        rl, pd, dm = ctx.saved_tensors
+        outs = [torch.empty_like(t) if ctx.needs_input_grad[i] else None for i, t in enumerate((rl, pd, dm))]
+        if rl.shape[0]:
+            check(_lib.lib().dcd_gmw_ray_rescale_bwd(ptr(rl), ptr(pd), ptr(dm), ptr(f32c(g_out)), rl.shape[0],
+                                                     *(ptr(o) for o in outs), stream_ptr()), "dcd_gmw_ray_rescale_bwd")
+        return tuple(outs)
+
+
+def _ray_rescale_fwd(rl, pd, dm):
     out = torch.empty_like(rl)
     if rl.shape[0]:
         check(_lib.lib().dcd_gmw_ray_rescale_fwd(ptr(rl), ptr(pd), ptr(dm), rl.shape[0], ptr(out), stream_ptr()),
               "dcd_gmw_ray_rescale_fwd")
     return out
+
+
+def ray_rescale(raw_location, pred_depth, dim):
+    """GMW/main.py:542-547: detector location [N,3] moved along its viewing ray to the GMW depth (dim [N,3] = (h,w,l)).
+    Differentiable w.r.t. all three inputs (dim: h column only); float64 inputs get float64 gradients."""
+    require_cuda(raw_location, pred_depth, dim)
+    rl, pd, dm = f32c(raw_location), f32c(pred_depth).reshape(-1), f32c(dim)
+    if _needs_grad(rl, pd, dm):
+        return _RayRescale.apply(rl, pd, dm)
+    return _ray_rescale_fwd(rl, pd, dm)
 
 
 def compute_z(kpts_2d, kpts_3d, pred_rot, num_k: int = K_SEL) -> Tuple[torch.Tensor, torch.Tensor]:
