@@ -49,6 +49,12 @@
 #ifndef DCD_FUSED_DONE_SLEEP
 #define DCD_FUSED_DONE_SLEEP 20      // converters waiting for an operand buffer
 #endif
+#ifndef DCD_FUSED_STAT_NBAR
+#define DCD_FUSED_STAT_NBAR 0        // 1: converters wait for a layer's statistics on a hardware named barrier, 0: on an mbarrier
+#endif
+#ifndef DCD_FUSED_STEP_UNROLL
+#define DCD_FUSED_STEP_UNROLL 2      // unroll depth of the converters' step loop (1: 0.5 % slower, DESIGN.md §5)
+#endif
 
 namespace dcd {
 // Optional in-kernel timeline (build with -DDCD_FUSED_TRACE, see profiles/trace_fused.py): lane 0 of converter warp 0
@@ -84,6 +90,7 @@ __device__ int g_trace_n[3];
 #endif
 namespace {
 
+constexpr int kStepUnroll = DCD_FUSED_STEP_UNROLL;
 constexpr int FCS = 24;             // CTAs per group = edge slices per object
 constexpr int FOBJ = 3;             // a group works on THREE objects at a time (same net, same layer weights)
 constexpr int FCONV_WARPS = 12;     // converter warps: 4 TMEM lane quarters x 3 units (16 edges) of a 48-edge sub-tile
@@ -108,8 +115,9 @@ static_assert(FOBJ * FES_MAX <= FCONV_THREADS, "one converter thread per staged 
 enum { BAR_FULL0 = 0, BAR_FULL1 = 1, BAR_DONE0 = 2, BAR_DONE1 = 3, BAR_PDONE = 4, BAR_WREADY = 5, BAR_STAT0 = 6, BAR_COUNT = 9 };
 // hardware named barriers (a blocked warp takes no issue slots): 0 = CTA, 1 = converters, 2..4 = the units of the epilogue,
 // 5..7 = partial statistics of object 0..2 posted: the converters (12 warps) arrive, the statistics warps (3 warps) wait;
-// 8 = the statistics warps among themselves
-enum { NB_PART0 = 5, NB_STATW = 8 };
+// 8 = the statistics warps among themselves; 9..11 = (mean, rstd) of object 0..2 handed back: the statistics warps arrive,
+// the converters wait (DCD_FUSED_STAT_NBAR)
+enum { NB_PART0 = 5, NB_STATW = 8, NB_STAT0 = 9 };
 constexpr int FSTAT_THREADS = 96;
 constexpr int NB_THREADS = FCONV_THREADS + FSTAT_THREADS;
 
@@ -186,22 +194,10 @@ __device__ __forceinline__ void tmem_ld16_wait(uint32_t (&r)[16]) {
                  : "memory");
 }
 
-// packed FP32 pair arithmetic (sm_100 FFMA2 / FADD2): one issue slot for two elements
-__device__ __forceinline__ void ffma2_bc(float& d0, float& d1, float a0, float a1, float b, float c) {   // d = a * b + c
-    asm("{\n\t.reg .b64 a, b, c, d;\n\tmov.b64 a, {%2, %3};\n\tmov.b64 b, {%4, %4};\n\tmov.b64 c, {%5, %5};\n\t"
-        "fma.rn.f32x2 d, a, b, c;\n\tmov.b64 {%0, %1}, d;\n\t}"
-        : "=f"(d0), "=f"(d1) : "f"(a0), "f"(a1), "f"(b), "f"(c));
-}
-__device__ __forceinline__ void fsq2_acc(float& s0, float& s1, float d0, float d1) {                      // s += d * d
-    asm("{\n\t.reg .b64 d, s;\n\tmov.b64 d, {%2, %3};\n\tmov.b64 s, {%0, %1};\n\t"
-        "fma.rn.f32x2 s, d, d, s;\n\tmov.b64 {%0, %1}, s;\n\t}"
-        : "+f"(s0), "+f"(s1) : "f"(d0), "f"(d1));
-}
-__device__ __forceinline__ void fadd2_acc(float& s0, float& s1, float d0, float d1) {                     // s += d
-    asm("{\n\t.reg .b64 d, s;\n\tmov.b64 d, {%2, %3};\n\tmov.b64 s, {%0, %1};\n\t"
-        "add.rn.f32x2 s, s, d;\n\tmov.b64 {%0, %1}, s;\n\t}"
-        : "+f"(s0), "+f"(s1) : "f"(d0), "f"(d1));
-}
+// packed FP32 pair arithmetic (sm_100 FFMA2 / FADD2, crt/sm_100_rt.hpp): one issue slot for two elements.  The operands are
+// float2 values that ptxas places in register pairs itself; the broadcast pairs are built once per layer or object.
+__device__ __forceinline__ float2 f2_of(uint32_t a, uint32_t b) { return make_float2(__uint_as_float(a), __uint_as_float(b)); }
+__device__ __forceinline__ float2 bcast2(float a) { return make_float2(a, a); }
 
 // no-swizzle (interleaved) shared-memory matrix descriptor
 __device__ __forceinline__ uint64_t smem_desc_ns(uint32_t addr, uint32_t lbo, uint32_t sbo) {
@@ -221,16 +217,19 @@ __device__ __forceinline__ void split2_neg(float v0, float v1, uint32_t& hp, uin
         : "f"(v0), "f"(v1));
 }
 
-// 16 edges (edge blocks 2u, 2u+1 of the sub-tile) of input channel ch -> FP16 hi / -lo, two 16-byte stores each
-__device__ __forceinline__ void store_unit(unsigned char* b_hi, unsigned char* b_lo, int ch, int u, const float (&v)[16]) {
+// byte offset of a converter thread's 16 edges (edge blocks 2u, 2u+1 of the sub-tile) of input channel ch in an operand part
+__device__ __forceinline__ uint32_t unit_offset(int ch, int u) {
+    return (uint32_t)(2 * u) * FB_SBO + (uint32_t)(ch >> 3) * FB_LBO + (uint32_t)(ch & 7) * 16u;
+}
+// 16 edges of one input channel -> FP16 hi / -lo, two 16-byte stores each (b_hi: the unit's place in the hi part)
+__device__ __forceinline__ void store_unit(unsigned char* b_hi, const float2 (&v)[8]) {
     uint32_t hp[8], lp[8];
 #pragma unroll
-    for (int q = 0; q < 8; ++q) split2_neg(v[2 * q], v[2 * q + 1], hp[q], lp[q]);
-    const uint32_t off = (uint32_t)(2 * u) * FB_SBO + (uint32_t)(ch >> 3) * FB_LBO + (uint32_t)(ch & 7) * 16u;
-    *reinterpret_cast<uint4*>(b_hi + off) = make_uint4(hp[0], hp[1], hp[2], hp[3]);
-    *reinterpret_cast<uint4*>(b_hi + off + FB_SBO) = make_uint4(hp[4], hp[5], hp[6], hp[7]);
-    *reinterpret_cast<uint4*>(b_lo + off) = make_uint4(lp[0], lp[1], lp[2], lp[3]);
-    *reinterpret_cast<uint4*>(b_lo + off + FB_SBO) = make_uint4(lp[4], lp[5], lp[6], lp[7]);
+    for (int q = 0; q < 8; ++q) split2_neg(v[q].x, v[q].y, hp[q], lp[q]);
+    *reinterpret_cast<uint4*>(b_hi) = make_uint4(hp[0], hp[1], hp[2], hp[3]);
+    *reinterpret_cast<uint4*>(b_hi + FB_SBO) = make_uint4(hp[4], hp[5], hp[6], hp[7]);
+    *reinterpret_cast<uint4*>(b_hi + FB_PART) = make_uint4(lp[0], lp[1], lp[2], lp[3]);
+    *reinterpret_cast<uint4*>(b_hi + FB_PART + FB_SBO) = make_uint4(lp[4], lp[5], lp[6], lp[7]);
 }
 
 // one sub-tile GEMM D[128 x N] = W[128 x 128] . B[128 x N] as 3 x 8 MMAs: Wh.(-(-Bl)), Wl.Bh, Wh.Bh
@@ -312,9 +311,15 @@ __global__ void __launch_bounds__(1024) fused_prep_kernel(const float* __restric
 
 namespace {
 
+template <int V> struct IntC { static constexpr int value = V; };   // compile-time step variant (converters' generic lambdas)
+
+// UPO = 16-edge units per object in a CTA = 48-column tiles per layer (FOBJ * ES == 48 * UPO): the slice geometry is a
+// compile-time constant, so the converters' object boundaries, unit streams and operand offsets are too.
+template <int UPO>
 __global__ void __launch_bounds__(FTHREADS, 1)
 mlp_fused_kernel(MlpArgs a, const float2* __restrict__ scales, const float* __restrict__ bias2, const uint32_t* __restrict__ wimg,
                  float2* xg, float* __restrict__ reg_w, float4* park) {
+    static_assert(UPO >= 3 && 16 * UPO <= FES_MAX, "slice geometry");
     const WsLayout& L = a.L;
     const int tid = threadIdx.x, lane = tid & 31;
     const int warp = __shfl_sync(0xffffffffu, tid >> 5, 0);  // warp-uniform for the compiler (uniform datapath)
@@ -323,13 +328,13 @@ mlp_fused_kernel(MlpArgs a, const float2* __restrict__ scales, const float* __re
     const int ch = 32 * quarter + lane;                      // this thread's channel = TMEM lane = weight row
     const uint32_t rank = blockIdx.x % FCS, group = blockIdx.x / FCS;   // 24 consecutive CTAs form a group (co-resident: cooperative launch)
     const int E = L.E, EP = L.EP, depth = L.depth;
-    const int upo = (E + 16 * FCS - 1) / (16 * FCS);         // 16-edge units per object in this CTA
-    const int ES = 16 * upo;                                 // edges per CTA and object
-    const int ntile = upo;                                   // 48-column tiles of the CTA: FOBJ * ES == 48 * upo
+    constexpr int upo = UPO;                                 // 16-edge units per object in this CTA
+    constexpr int ES = 16 * upo;                             // edges per CTA and object
+    constexpr int ntile = upo;                               // 48-column tiles of the CTA
     const int nphase = 2 * depth;                            // per block: folded preconv.conv1, conv2
 #if DCD_FUSED_CONV_FINAL
     // (slices of 4 units: a converter warp's next post could overtake another warp's read of the shared partial slots)
-    const bool conv_final = upo != 4;
+    constexpr bool conv_final = upo != 4;
 #endif
 
     extern __shared__ __align__(1024) unsigned char smem[];
@@ -475,6 +480,15 @@ mlp_fused_kernel(MlpArgs a, const float2* __restrict__ scales, const float* __re
             nbar_sync(NB_STATW, FSTAT_THREADS);
             TR(2, 720 + o);
         };
+        // (mean, rstd) or the rank-subset results of object o are in the partial slots: release the converters waiting for them
+        auto stat_handback = [&](int o) {
+#if DCD_FUSED_STAT_NBAR
+            nbar_arrive(NB_STAT0 + o, NB_THREADS);     // (a hardware barrier: the waiting converter warps take no issue slots)
+#else
+            __syncwarp();
+            if (lane == 0) mbar_arrive(bar + BAR_STAT0 + o);
+#endif
+        };
         // Collect the 24 slices (the own one included) and hand (mean, rstd) to the converters.  Each statistics warp takes 8
         // ranks for all 128 channels (a lane: 4 channels x 8 flagged words in flight at once, re-read until every word carries
         // this exchange's flag) and merges them; the three subset results meet in the object's partial slots, then every channel
@@ -513,8 +527,7 @@ mlp_fused_kernel(MlpArgs a, const float2* __restrict__ scales, const float* __re
             }
 #if DCD_FUSED_CONV_FINAL
             if (conv_final) {                                 // the converter threads finish their channel themselves (see `collect`)
-                __syncwarp();
-                if (lane == 0) mbar_arrive(bar + BAR_STAT0 + o);
+                stat_handback(o);
                 TR(2, 730 + o);
                 sxc = (sxc & ~(3u << (2 * o))) | (((((sxc >> (2 * o)) & 3u) + 1u) & 3u) << (2 * o));
                 return;
@@ -539,8 +552,7 @@ mlp_fused_kernel(MlpArgs a, const float2* __restrict__ scales, const float* __re
 #pragma unroll
                 for (int k = 0; k < 3; ++k) pbuf[(o * 3 + k) * CH + c] = st;
             }
-            __syncwarp();
-            if (lane == 0) mbar_arrive(bar + BAR_STAT0 + o);
+            stat_handback(o);
             TR(2, 730 + o);
             sxc = (sxc & ~(3u << (2 * o))) | (((((sxc >> (2 * o)) & 3u) + 1u) & 3u) << (2 * o));
         };
@@ -637,7 +649,9 @@ mlp_fused_kernel(MlpArgs a, const float2* __restrict__ scales, const float* __re
             }
         };
         auto obj_of = [&](int u) { return (u >= upo ? 1 : 0) + (u >= 2 * upo ? 1 : 0); };
+#if !DCD_FUSED_STAT_NBAR
         uint32_t spar = 0;                                    // wait parities of the three statistics barriers (this warp's view)
+#endif
 #if DCD_FUSED_CONV_FINAL
         const float inv_em1_c = 1.0f / (float)(E - 1);
 #endif
@@ -719,40 +733,41 @@ mlp_fused_kernel(MlpArgs a, const float2* __restrict__ scales, const float* __re
             //      consecutive, so the object and the offset inside its slice are running values (firstmask / lastmask: the tiles
             //      where this warp's unit is its first / last of an object).
             float un_out = 0.f, b_out = 0.f, un_prev = 0.f, b_prev = 0.f;   // scale / bias of the matrices of this and the previous layer
+            float2 un2_out = make_float2(0.f, 0.f), un2_prev = un2_out;     // (the scales as broadcast pairs)
             float un_next = __ldg(scales + mat_base).y, b_next = __ldg(bias2 + mat_base * CH + ch);       // (fetched one layer ahead)
-            // the tile whose statistics are due next (two steps behind the conversion): tile, object, object's first column, parity of its layer
-            int npend = 0, t_e = 0, o_e = 0, ob_e = 0, p_e = 0;
-            float K = 0.f, s1 = 0.f, s2 = 0.f, bK = 0.f;      // shifted sums of the layer output being accumulated (one object at a time)
+            // the tile whose statistics are due next (two steps behind the conversion): tile, object, object's first column
+            int npend = 0, t_e = 0, o_e = 0, ob_e = 0;
+            float K = 0.f, s1 = 0.f, s2 = 0.f;                // shifted sums of the layer output being accumulated (one object at a time)
+            float2 bK2 = make_float2(0.f, 0.f);               // bias - K of that object, both halves
             bool have_K = false;
             uint32_t cv[16], sv[16];
 
-            // statistics of one unit from its raw accumulators (un, bb: scale and bias of the producing matrix), as sums shifted
+            // statistics of one unit from its raw accumulators (un2, bb: scale and bias of the producing matrix), as sums shifted
             // by K = the object's first value seen by this thread
-            auto stats_math = [&](const uint32_t (&raw)[16], int nv, float un, float bb) {
+            auto stats_math = [&](const uint32_t (&raw)[16], int nv, float2 un2, float bb) {
                 if (!have_K) {
-                    K = fmaf(__uint_as_float(raw[0]), un, bb);
-                    bK = bb - K;
+                    K = fmaf(__uint_as_float(raw[0]), un2.x, bb);
+                    bK2 = bcast2(bb - K);
                     have_K = true;
                 }
                 if (nv >= 16) {
-                    float t1[4] = {0.f, 0.f, 0.f, 0.f}, t2[4] = {0.f, 0.f, 0.f, 0.f};
+                    float2 t1a = make_float2(0.f, 0.f), t1b = t1a, t2a = t1a, t2b = t1a;
 #pragma unroll
                     for (int i = 0; i < 16; i += 4) {
-                        float d0, d1, d2, d3;
-                        ffma2_bc(d0, d1, __uint_as_float(raw[i]), __uint_as_float(raw[i + 1]), un, bK);
-                        ffma2_bc(d2, d3, __uint_as_float(raw[i + 2]), __uint_as_float(raw[i + 3]), un, bK);
-                        fadd2_acc(t1[0], t1[1], d0, d1);
-                        fadd2_acc(t1[2], t1[3], d2, d3);
-                        fsq2_acc(t2[0], t2[1], d0, d1);
-                        fsq2_acc(t2[2], t2[3], d2, d3);
+                        const float2 d01 = __ffma2_rn(f2_of(raw[i], raw[i + 1]), un2, bK2);
+                        const float2 d23 = __ffma2_rn(f2_of(raw[i + 2], raw[i + 3]), un2, bK2);
+                        t1a = __fadd2_rn(t1a, d01);
+                        t1b = __fadd2_rn(t1b, d23);
+                        t2a = __ffma2_rn(d01, d01, t2a);
+                        t2b = __ffma2_rn(d23, d23, t2b);
                     }
-                    s1 += (t1[0] + t1[1]) + (t1[2] + t1[3]);
-                    s2 += (t2[0] + t2[1]) + (t2[2] + t2[3]);
+                    s1 += (t1a.x + t1a.y) + (t1b.x + t1b.y);
+                    s2 += (t2a.x + t2a.y) + (t2b.x + t2b.y);
                 } else {
 #pragma unroll
                     for (int i = 0; i < 16; ++i)
                         if (i < nv) {
-                            const float dd = fmaf(__uint_as_float(raw[i]), un, bK);
+                            const float dd = fmaf(__uint_as_float(raw[i]), un2.x, bK2.x);
                             s1 += dd;
                             s2 = fmaf(dd, dd, s2);
                         }
@@ -767,14 +782,18 @@ mlp_fused_kernel(MlpArgs a, const float2* __restrict__ scales, const float* __re
                 pbuf[(o * 3 + k) * CH + ch] = make_float2(m, M2);
                 nbar_arrive(NB_PART0 + o, NB_THREADS);
                 TR(0, 603);
-                K = 0.f; s1 = 0.f; s2 = 0.f; bK = 0.f;
+                K = 0.f; s1 = 0.f; s2 = 0.f; bK2 = make_float2(0.f, 0.f);
                 have_K = false;
             };
             // (mean, rstd) of object o's latest layer, handed back by the statistics warps in this warp's partial slot
             auto collect = [&](int o) {
                 TR(0, 606);
+#if DCD_FUSED_STAT_NBAR
+                nbar_sync(NB_STAT0 + o, NB_THREADS);
+#else
                 mbar_wait_backoff(bar + BAR_STAT0 + o, (spar >> o) & 1u, DCD_FUSED_STAT_SLEEP);
                 spar ^= 1u << o;
+#endif
                 TR(0, 608);
 #if DCD_FUSED_CONV_FINAL
                 if (conv_final) {
@@ -796,114 +815,124 @@ mlp_fused_kernel(MlpArgs a, const float2* __restrict__ scales, const float* __re
 #endif
                 return pbuf[(o * 3 + stream_of(o)) * CH + ch];
             };
-            // statistics of the due tile (its MMA is complete; `loaded`: its accumulators are already in sv)
-            auto process_due = [&](bool loaded, int ph) {
+            // statistics of the due tile (its MMA is complete; `loaded`: its accumulators are already in sv; `cur`: it belongs to
+            // the layer being converted, else to the previous one).  FULL: every edge of the slice is valid.
+            auto process_due = [&](auto full_c, bool loaded, bool cur) {
+                constexpr bool FULL = decltype(full_c)::value != 0;
                 const int cb = FSUB * t_e + 16 * wg;          // first column of the unit
-                const int nv = valid - (cb - ob_e);           // valid edges from the unit's first on
+                const int nv = FULL ? 16 : valid - (cb - ob_e);   // valid edges from the unit's first on
                 if (nv > 0) {
                     if (!loaded) {
                         tmem_ld16_issue(t_lane + cb, sv);
                         tmem_ld16_wait(sv);
                     }
-                    const bool cur = p_e == (ph & 1);
-                    stats_math(sv, nv, cur ? un_out : un_prev, cur ? b_out : b_prev);
+                    stats_math(sv, nv, cur ? un2_out : un2_prev, cur ? b_out : b_prev);
                 }
                 if ((lastmask >> t_e) & 1u) post(o_e);
                 if (++t_e == ntile) {
-                    t_e = 0; o_e = 0; ob_e = 0; p_e ^= 1;
+                    t_e = 0; o_e = 0; ob_e = 0;
                 } else if ((firstmask >> t_e) & 1u) {
                     ++o_e; ob_e += ES;
                 }
             };
 
-            float a_in = 0.f, c_in = 0.f;
-            for (int ph = 0; ph < nphase; ++ph) {
-                const int kind = (ph & 1) ? 2 : 0;            // 0: (residual update ->) folded preconv.conv1, 2: conv2
-                un_prev = un_out;
-                b_prev = b_out;
-                un_out = un_next;
-                b_out = b_next;
-                if (ph + 1 < nphase) {
-                    un_next = __ldg(scales + mat_base + ph + 1).y;
-                    b_next = __ldg(bias2 + (mat_base + ph + 1) * CH + ch);
-                }
-                const bool reads_d = ph > 0;
-                // Software pipeline over the steps: the accumulators of the NEXT unit to convert (cv, issued at the end of the
-                // previous step) and of the unit whose statistics are due (sv, two steps behind: its MMA is known complete when
-                // its operand buffer comes free) are in flight from tensor memory while the current unit is being processed.
+            // input transform of the current object as one FMA on the raw accumulator, both halves: the context norm of the
+            // producing layer folded in ((d*un + b - mean) * rstd)
+            float2 a_in2 = make_float2(0.f, 0.f), c_in2 = a_in2;
+            auto take_stats = [&](int o) {
+                const float2 st = collect(o);
+                a_in2 = bcast2(un_prev * st.y);
+                c_in2 = bcast2((b_prev - st.x) * st.y);
+            };
+            const bool full = valid == ES;                    // no edge of the slice masked (all CTAs of a group but the last ones)
+            const uint32_t uoff = unit_offset(ch, wg);        // this thread's place in an operand part
+
+            // One layer, specialised by kind — 0: residual update, then the folded preconv.conv1; 1: the same for the net's first
+            // layer (no accumulators to read, X is the input); 2: conv2 — and by FULL (no tail masks).  Software pipeline over the
+            // steps: the accumulators of the NEXT unit to convert (cv, issued at the end of the previous step) and of the unit whose
+            // statistics are due (sv, two steps behind: its MMA is known complete when its operand buffer comes free) are in flight
+            // from tensor memory while the current unit is being processed.
+            auto layer = [&](auto kind_c, auto full_c, int ph) {
+                constexpr int KIND = decltype(kind_c)::value;
+                constexpr bool FULL = decltype(full_c)::value != 0;
+                constexpr bool reads_d = KIND != 1;
+                constexpr int KTAG = KIND == 2 ? 2 : 0;       // (trace tags: the kind of the layer's matrix)
+                (void)KTAG;
                 int o = 0, ob = 0;
+                if (reads_d) take_stats(0);
+#pragma unroll (UPO == 4 ? 1 : kStepUnroll)        // (UPO = 4 spills when unrolled)
                 for (int t = 0; t < ntile; ++t, ++g) {
                     const int cb = FSUB * t + 16 * wg;        // this warp's unit: columns [cb, cb + 16) of the CTA
-                    if ((firstmask >> t) & 1u) {
-                        if (t > 0) { ++o; ob += ES; }
-                        if (reads_d) {
-                            // input transform of this layer as one FMA on the raw accumulator: the context norm of the producing
-                            // layer folded in ((d*un + b - mean) * rstd)
-                            const float2 st = collect(o);
-                            a_in = un_prev * st.y;
-                            c_in = (b_prev - st.x) * st.y;
-                        }
+                    if (t > 0 && ((firstmask >> t) & 1u)) {
+                        ++o; ob += ES;
+                        if (reads_d) take_stats(o);
                     }
                     const int lc = cb - ob;                   // first edge of the unit inside the object's slice
+                    (void)lc;
                     const uint32_t b = g & 1u;
-                    TR(0, 1000 * kind + 100 + t);
-                    wait_buf(b);
-                    TRF(0, 1000 * kind + 200 + t);
-                    unsigned char* b_hi = Bbuf + (size_t)b * 2 * FB_PART;
-                    // the tile of two steps ago (same operand buffer: its MMA is complete) is due for its statistics
-                    const bool due = npend == 2;
+                    TR(0, 1000 * KTAG + 100 + t);
+                    if (reads_d) {                            // (both buffers are in use from the round's third step on)
+                        mbar_wait_backoff(bar + BAR_DONE0 + b, (par >> b) & 1u, DCD_FUSED_DONE_SLEEP);
+                        par ^= 1u << b;
+                        tc_fence_after();
+                    } else {
+                        wait_buf(b);
+                    }
+                    TRF(0, 1000 * KTAG + 200 + t);
+                    // the tile of two steps ago (same operand buffer: its MMA is complete) is due for its statistics (the first two
+                    // steps of a round have none)
+                    const bool due = KIND != 1 || t >= 2;
                     const int cb_e = FSUB * t_e + 16 * wg;
-                    const bool st_load = due && valid > cb_e - ob_e;
-                    float v[16];
+                    const bool st_load = due && (FULL || valid > cb_e - ob_e);
+                    float2 v[8];
                     float4* Xp = Xs + (cb >> 2) * CH + ch;
                     float4 x4[4];
-                    if (kind == 0) {
+                    if (KIND != 2) {
 #pragma unroll
                         for (int q4 = 0; q4 < 4; ++q4) x4[q4] = Xp[q4 * CH];
                     }
                     if (reads_d) tmem_ld16_wait(cv);
-                    TRF(0, 1000 * kind + 300 + t);
+                    TRF(0, 1000 * KTAG + 300 + t);
                     if (st_load) tmem_ld16_issue(t_lane + cb_e, sv);
-                    if (kind == 0) {
-                        if (reads_d) {
+                    if (KIND == 0) {
 #pragma unroll
-                            for (int i = 0; i < 16; i += 2) {
-                                ffma2_bc(v[i], v[i + 1], __uint_as_float(cv[i]), __uint_as_float(cv[i + 1]), a_in, c_in);
-                                v[i] = fmaxf(v[i], 0.f);
-                                v[i + 1] = fmaxf(v[i + 1], 0.f);
+                        for (int i = 0; i < 8; ++i) {
+                            v[i] = __ffma2_rn(f2_of(cv[2 * i], cv[2 * i + 1]), a_in2, c_in2);
+                            v[i].x = fmaxf(v[i].x, 0.f);
+                            v[i].y = fmaxf(v[i].y, 0.f);
+                        }
+#pragma unroll
+                        for (int q4 = 0; q4 < 4; ++q4) {
+                            v[2 * q4] = __fadd2_rn(v[2 * q4], make_float2(x4[q4].x, x4[q4].y));
+                            v[2 * q4 + 1] = __fadd2_rn(v[2 * q4 + 1], make_float2(x4[q4].z, x4[q4].w));
+                        }
+                        if (!FULL && lc + 16 > valid) {
+#pragma unroll
+                            for (int i = 0; i < 8; ++i) {
+                                if (lc + 2 * i >= valid) v[i].x = 0.f;
+                                if (lc + 2 * i + 1 >= valid) v[i].y = 0.f;
                             }
+                        }
 #pragma unroll
-                            for (int q4 = 0; q4 < 4; ++q4) {
-                                fadd2_acc(v[4 * q4], v[4 * q4 + 1], x4[q4].x, x4[q4].y);
-                                fadd2_acc(v[4 * q4 + 2], v[4 * q4 + 3], x4[q4].z, x4[q4].w);
-                            }
-                            if (lc + 16 > valid) {
+                        for (int q4 = 0; q4 < 4; ++q4) Xp[q4 * CH] = make_float4(v[2 * q4].x, v[2 * q4].y, v[2 * q4 + 1].x, v[2 * q4 + 1].y);
+                    } else if (KIND == 1) {
 #pragma unroll
-                                for (int i = 0; i < 16; ++i)
-                                    if (lc + i >= valid) v[i] = 0.f;
-                            }
-#pragma unroll
-                            for (int q4 = 0; q4 < 4; ++q4)
-                                Xp[q4 * CH] = make_float4(v[4 * q4], v[4 * q4 + 1], v[4 * q4 + 2], v[4 * q4 + 3]);
-                        } else {
-#pragma unroll
-                            for (int q4 = 0; q4 < 4; ++q4) {
-                                v[4 * q4] = x4[q4].x; v[4 * q4 + 1] = x4[q4].y; v[4 * q4 + 2] = x4[q4].z; v[4 * q4 + 3] = x4[q4].w;
-                            }
+                        for (int q4 = 0; q4 < 4; ++q4) {
+                            v[2 * q4] = make_float2(x4[q4].x, x4[q4].y);
+                            v[2 * q4 + 1] = make_float2(x4[q4].z, x4[q4].w);
                         }
                     } else {
 #pragma unroll
-                        for (int i = 0; i < 16; i += 2)
-                            ffma2_bc(v[i], v[i + 1], __uint_as_float(cv[i]), __uint_as_float(cv[i + 1]), a_in, c_in);
+                        for (int i = 0; i < 8; ++i) v[i] = __ffma2_rn(f2_of(cv[2 * i], cv[2 * i + 1]), a_in2, c_in2);
                     }
-                    store_unit(b_hi, b_hi + FB_PART, ch, wg, v);
-                    TRF(0, 1000 * kind + 400 + t);
+                    store_unit(Bbuf + (size_t)b * 2 * FB_PART + uoff, v);
+                    TRF(0, 1000 * KTAG + 400 + t);
                     fence_async_smem();
                     tc_fence_before();
                     __syncwarp();
                     if (lane == 0) mbar_arrive(bar + BAR_FULL0 + b);
                     pend |= 1u << b;
-                    TRF(0, 1000 * kind + 500 + t);
+                    TRF(0, 1000 * KTAG + 500 + t);
                     if (st_load) tmem_ld16_wait(sv);              // (before the next load is issued: the wait covers all loads in flight)
                     // the next unit to convert: the next tile's, else the next layer's first (whose producing MMA is long complete)
                     if (t + 1 < ntile) {
@@ -911,7 +940,29 @@ mlp_fused_kernel(MlpArgs a, const float2* __restrict__ scales, const float* __re
                     } else if (ph + 1 < nphase) {
                         tmem_ld16_issue(t_lane + 16 * wg, cv);
                     }
-                    if (due) process_due(true, ph); else ++npend;
+                    if (due) process_due(full_c, true, t >= 2); else ++npend;
+                }
+            };
+
+            for (int ph = 0; ph < nphase; ++ph) {
+                un_prev = un_out;
+                b_prev = b_out;
+                un_out = un_next;
+                b_out = b_next;
+                un2_prev = un2_out;
+                un2_out = bcast2(un_out);
+                if (ph + 1 < nphase) {
+                    un_next = __ldg(scales + mat_base + ph + 1).y;
+                    b_next = __ldg(bias2 + (mat_base + ph + 1) * CH + ch);
+                }
+                if (full) {
+                    if (ph & 1) layer(IntC<2>(), IntC<1>(), ph);
+                    else if (ph > 0) layer(IntC<0>(), IntC<1>(), ph);
+                    else layer(IntC<1>(), IntC<1>(), ph);
+                } else {
+                    if (ph & 1) layer(IntC<2>(), IntC<0>(), ph);
+                    else if (ph > 0) layer(IntC<0>(), IntC<0>(), ph);
+                    else layer(IntC<1>(), IntC<0>(), ph);
                 }
             }
             TR(0, 600);
@@ -922,8 +973,9 @@ mlp_fused_kernel(MlpArgs a, const float2* __restrict__ scales, const float* __re
             wait_buf(1);
             un_prev = un_out;
             b_prev = b_out;
+            un2_prev = un2_out;
             while (npend > 0) {
-                process_due(false, nphase);
+                process_due(IntC<0>(), false, false);
                 --npend;
             }
             TR(0, 601);
@@ -1088,11 +1140,18 @@ int launch_gmw_fused_fwd(const MlpArgs& a, const float* params4, const float* pa
     // (queried on every call: the library keeps no state between calls; these are host-side lookups, no device work)
     int dev = 0;
     if (cudaGetDevice(&dev) != cudaSuccess) return DCD_E_DEVICE;
-    cudaFuncSetAttribute(mlp_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFusedSmem);
+    // one instantiation per slice geometry (16-edge units per object and CTA, the range gmw_fused_supported accepts)
+    using FusedKernel = void (*)(MlpArgs, const float2*, const float*, const uint32_t*, float2*, float*, float4*);
+    static const FusedKernel kernels[] = {mlp_fused_kernel<3>, mlp_fused_kernel<4>, mlp_fused_kernel<5>, mlp_fused_kernel<6>,
+                                          mlp_fused_kernel<7>};
+    const int upo = (a.L.E + 16 * FCS - 1) / (16 * FCS);
+    if (upo < 3 || upo > 7) return DCD_E_UNSUPPORTED;
+    const FusedKernel kernel = kernels[upo - 3];
+    cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFusedSmem);
     cudaFuncSetAttribute(fused_prep_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(CH * CH * sizeof(float)));
     int coop = 0, per_sm = 0;
     cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, dev);
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, mlp_fused_kernel, FTHREADS, kFusedSmem);
+    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, FTHREADS, kFusedSmem);
     if (!coop || per_sm < 1) return DCD_E_UNSUPPORTED;
     int max_groups = device_sm_count() * per_sm / FCS;
     if (max_groups > FMAX_GROUPS) max_groups = FMAX_GROUPS;
@@ -1101,7 +1160,7 @@ int launch_gmw_fused_fwd(const MlpArgs& a, const float* params4, const float* pa
     cudaMemsetAsync(xg, 0x80, kExchangeBytes, st);            // every word starts with the flag its first use does not expect
     // work is dealt to the groups as object triples (paired schedule: both nets of a triple back to back; the first net's
     // features are parked in one activation slot, FOBJ * FCS * ES columns per group) or as (triple, net) rounds
-    const int64_t es = 16 * ((a.L.E + 16 * FCS - 1) / (16 * FCS));
+    const int64_t es = 16 * upo;
     const bool paired = reg_w != nullptr && a.L.N >= FOBJ * (int64_t)max_groups &&
                         a.L.N * (int64_t)a.L.EP >= (int64_t)max_groups * FOBJ * FCS * es;
     const int64_t npairs = (a.L.N + FOBJ - 1) / FOBJ;
@@ -1114,7 +1173,7 @@ int launch_gmw_fused_fwd(const MlpArgs& a, const float* params4, const float* pa
     float* regw_arg = paired ? reg_w : nullptr;
     float4* park_arg = reinterpret_cast<float4*>(act_ptr(a.ws, a.L, 0, 0, SLOT_Y1));
     void* kargs[] = {&args, &scales_arg, &bias_arg, &wimg_arg, &xg, &regw_arg, &park_arg};
-    if (cudaLaunchCooperativeKernel(reinterpret_cast<void*>(mlp_fused_kernel), dim3(FCS * ngroups), dim3(FTHREADS), kargs, kFusedSmem,
+    if (cudaLaunchCooperativeKernel(reinterpret_cast<void*>(kernel), dim3(FCS * ngroups), dim3(FTHREADS), kargs, kFusedSmem,
                                     st) != cudaSuccess) {
         cudaGetLastError();
         return DCD_E_LAUNCH;
